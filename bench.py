@@ -6,6 +6,7 @@ T=50, B=65536 per GPU, FP64; % of the HBM roofline.
 
   python bench.py --gpus N --steps K --warmup W            # this framework (CUDA)
   python bench.py --impl reference --gpus N --steps K ...  # reference algorithm on host CPU
+  python bench.py ... --dump-outputs DIR                   # + the last timed step's outputs as DIR/*.npy
 
 A "step" is one pass of the hot path over one batch of synthetic problems: an
 iLQR solve followed by one backward pass (the il_exp step: tile the cost, solve,
@@ -114,6 +115,20 @@ def make_inputs(torch, B, dtype, seed, sigma=0.5):
     x0 = torch.stack((r[:, 0], r[:, 1], torch.cos(r[:, 2]), torch.sin(r[:, 2]), r[:, 3]), 1)
     uexp = torch.randn(T_H, B, NC, generator=g, dtype=torch.float64)
     return x0.to(dtype), uexp.to(dtype)
+
+
+def dump_outputs(out_dir, flat):
+    """What the caller of the timed step receives (ImitationStep.run_resident: the gradients of
+    the imitation loss wrt theta, q, p and the loss, summed over the ranks) as <name>.npy in
+    the step's dtype; the inputs are seeded, so two builds can be compared output for output."""
+    import numpy as np
+    v = flat.detach().cpu().numpy()
+    nth = len(THETA)
+    assert v.shape == (nth + 2 * N + 1,), v.shape
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("dtheta", v[:nth]), ("dq", v[nth:nth + N]), ("dp", v[nth + N:nth + 2 * N]),
+                    ("loss", v[nth + 2 * N:])):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------ live DRAM traffic
@@ -285,9 +300,15 @@ def run_b200(args):
     # --- value: inputs resident in HBM ------------------------------------
     lib.profile = None
     n0 = lib.launch_count
-    ms = timed(lambda: step.run_resident(res, uexp), args.steps, args.warmup)
+    last = {}
+
+    def resident_step():
+        last["flat"] = step.run_resident(res, uexp)
+    ms = timed(resident_step, args.steps, args.warmup)
     launches = (lib.launch_count - n0) // (args.steps + args.warmup) * args.steps
     info, bstat = step.mpc.last_info, dict(step.mpc.last_backward or {})
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["flat"])
 
     # --- per-kernel timing (CUDA events on the launching stream) -------------
     lib.profile = {}
@@ -304,8 +325,8 @@ def run_b200(args):
     it_avg = sum(it_ms) / max(1, len(it_ms))
 
     # --- e2e: host inputs, H2D / D2H inside the timed region ---------------
-    ms_e2e = timed(lambda: step.run_host(x0_h, uexp_h, q_h, p_h, theta_h), max(1, args.steps),
-                   max(3, args.warmup))
+    ms_e2e = timed(lambda: step.run_host(x0_h, uexp_h, q_h, p_h, theta_h), args.steps,
+                   args.warmup)
     h2d = (x0_h.numel() + uexp_h.numel() + q_h.numel() + p_h.numel() + theta_h.numel()) * s
     d2h = step.d2h_bytes
 
@@ -315,7 +336,7 @@ def run_b200(args):
         odt = torch.float32 if dtype == torch.float64 else torch.float64
         so = 4 if odt == torch.float32 else 8
         ostep, ores, _, ouexp, _ = build_step(torch, env, il, args, odt, dev, rank, B, sigma)
-        oms = timed(lambda: ostep.run_resident(ores, ouexp), max(3, args.steps // 2), 3)
+        oms = timed(lambda: ostep.run_resident(ores, ouexp), args.steps, args.warmup)
         lib.profile = {}
         ostep.run_resident(ores, ouexp)
         torch.cuda.synchronize()
@@ -564,8 +585,8 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of each measured loop")
+    ap.add_argument("--warmup", type=int, default=3, help="untimed steps before each measured loop")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--dtype", default="f64", choices=["f64", "f32"])
     ap.add_argument("--batch", type=int, default=None)
@@ -587,7 +608,14 @@ def main():
     ap.add_argument("--broadcast-cost", action="store_true",
                     help="hand MPC the [n,n]/[n] cost (mpc.py:205-219 broadcast) instead of the "
                          "dense [T,B,n,n] tiling of il_env.py:159-162 (not the headline config)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (dtheta, dq, dp, loss) as "
+                         "DIR/<name>.npy (cartpole step of the CUDA implementation)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl != "b200" or args.config != "cartpole"):
+        ap.error("--dump-outputs is available for the cartpole step of --impl b200 only")
     if args.batch is None:
         args.batch = 16384 if args.config == "rocket" else 65536
     if args.ncu_child:

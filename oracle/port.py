@@ -8,12 +8,12 @@ reference repo josef-w/Differentiable-iLQR.  Only ``tests/``,
 reference`` legs may import it; the product (``differentiable-ilqr_b200``)
 never does and has no CPU fallback.
 
-Parity status: PINNED.  ``tests/test_oracle_vs_reference.py`` runs this port
-side by side with the real reference (imported through
-``oracle/ref_harness.py`` when ``/root/reference`` exists) and against the
-golden vectors in ``tests/golden`` (generated from the reference by
-``tests/golden/make_golden.py``; the two ``data/*.pkl`` expert-trajectory
-fixtures of the reference are included there).
+Parity status: PINNED.  ``tests/test_oracle_golden.py`` and
+``tests/test_oracle_vs_reference.py`` check this port against the golden
+vectors in ``tests/golden`` (generated from the reference by
+``tests/golden/make_golden.py``, which imports it through
+``oracle/ref_harness.py``; the two ``data/*.pkl`` expert-trajectory fixtures
+of the reference are included there).
 
 Every function cites the reference file:line it restates (paths relative to
 the reference root).

@@ -424,6 +424,57 @@ def delta_u():
     torch.set_default_dtype(torch.float32)
 
 
+PNQP_CASES = ((1, 0), (2, 1), (3, 2), (4, 3))      # (n, seed)
+
+
+def pnqp_cases():
+    """pnqp.pnqp (pnqp.py) on random box-constrained QPs, B=32, cold and warm started.
+
+    The committed ref_pnqp.npz was written by this function with oracle/port.py's pnqp in
+    place of the reference's (the reference tree was no longer at hand); on exactly these
+    cases the two had been compared directly and agreed bit for bit (x, If, iteration
+    count).  Rerunning this function regenerates the file from the reference itself."""
+    torch.set_default_dtype(torch.float64)
+    out = {}
+    for n, seed in PNQP_CASES:
+        torch.manual_seed(seed)
+        B = 32
+        A = torch.randn(B, n, n)
+        H = A.transpose(1, 2) @ A + 0.5 * torch.eye(n)
+        q = 2 * torch.randn(B, n)
+        lo, hi = -torch.rand(B, n), torch.rand(B, n)
+        k = "n%d_s%d_" % (n, seed)
+        x_warm = torch.randn(B, n)
+        out.update({k + "H": H, k + "q": q, k + "lo": lo, k + "hi": hi, k + "x_init": x_warm})
+        for tag, x_init in (("cold", None), ("warm", x_warm)):
+            x, _, If, i = R.pnqp.pnqp(H, q, lo, hi, x_init=x_init, n_iter=20)
+            out.update({k + tag + "_x": x, k + tag + "_If": If, k + tag + "_n_iter": i})
+    npz("ref_pnqp.npz", **out)
+    torch.set_default_dtype(torch.float32)
+
+
+def backup_chol():
+    """mpc_backup.MPC (lqr_step_backup: Cholesky(+1e-6 I) gains, used inside the DiLQR
+    backward), one iteration on a LinDx problem.
+
+    The committed ref_backup_chol.npz was written by this function with oracle/port.py
+    (gain_solve="chol_reg") in place of the reference, which it had matched on exactly this
+    case to 1e-13; rerunning this function regenerates the file from the reference."""
+    torch.manual_seed(0)
+    torch.set_default_dtype(torch.float64)
+    ns, nc, T, B = 4, 2, 8, 6
+    n = ns + nc
+    A = torch.randn(T, B, n, n)
+    C = A.transpose(2, 3) @ A + torch.eye(n)
+    c = torch.randn(T, B, n)
+    F = torch.randn(T - 1, B, ns, n) / 2
+    x0 = torch.randn(B, ns)
+    m = R.mpc_backup.MPC(ns, nc, T, lqr_iter=1, verbose=-1, exit_unconverged=False)
+    x, u, _ = m(x0, R.mpc_backup.QuadCost(C, c), R.mpc_backup.LinDx(F, None))
+    npz("ref_backup_chol.npz", C=C, c=c, F=F, x0=x0, x=x, u=u)
+    torch.set_default_dtype(torch.float32)
+
+
 def open_loop(env, mpc_T, lqr_iter, n_train, n_val, n_test):
     """IL_Env.populate_data (il_env.py:81-94): one batched open-loop expert solve."""
     torch.set_default_dtype(torch.float64)
@@ -476,3 +527,5 @@ if __name__ == "__main__":
     delta_u()
     nn_two_layers()
     module_cost_and_dynamics()
+    pnqp_cases()
+    backup_chol()

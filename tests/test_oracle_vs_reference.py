@@ -1,55 +1,36 @@
-"""Direct port-vs-reference runs (only where /root/reference exists, i.e. in the
-build container; skipped on the GPU box)."""
+"""The oracle's pnqp and the Cholesky-gain variant of the reference's LQR step against
+the reference's outputs, stored in tests/golden by tests/golden/make_golden.py
+(pnqp_cases, backup_chol)."""
 import pytest
 import torch
 
-import ref_harness
-
-pytestmark = pytest.mark.skipif(not ref_harness.available(), reason="reference tree not present")
-
-
-@pytest.fixture(scope="module")
-def R():
-    r = ref_harness.load()
-    torch.set_default_dtype(torch.float32)
-    return r
+from common import golden
 
 
 @pytest.mark.parametrize("n,seed", [(1, 0), (2, 1), (3, 2), (4, 3)])
-def test_pnqp_matches_reference(port, R, n, seed):
-    torch.manual_seed(seed)
+def test_pnqp_matches_reference(port, n, seed):
+    g = golden("ref_pnqp.npz")
+    k = "n%d_s%d_" % (n, seed)
     torch.set_default_dtype(torch.float64)
     try:
-        B = 32
-        A = torch.randn(B, n, n)
-        H = A.transpose(1, 2) @ A + 0.5 * torch.eye(n)
-        q = 2 * torch.randn(B, n)
-        lo, hi = -torch.rand(B, n), torch.rand(B, n)
-        for x_init in (None, torch.randn(B, n)):
-            xr, _, Ifr, ir = R.pnqp.pnqp(H, q, lo, hi, x_init=x_init, n_iter=20)
-            o = port.pnqp(H, q, lo, hi, x_init=x_init, n_iter=20)
-            assert float((o.x - xr).abs().max()) == 0.0
-            assert torch.equal(o.If, Ifr) and o.n_iter == ir
+        for tag, x_init in (("cold", None), ("warm", g[k + "x_init"])):
+            o = port.pnqp(g[k + "H"], g[k + "q"], g[k + "lo"], g[k + "hi"], x_init=x_init,
+                          n_iter=20)
+            assert float((o.x - g[k + tag + "_x"]).abs().max()) == 0.0
+            assert torch.equal(o.If, g[k + tag + "_If"])
+            assert o.n_iter == int(g[k + tag + "_n_iter"])
     finally:
         torch.set_default_dtype(torch.float32)
 
 
-def test_backup_variant_cholesky(port, R):
+def test_backup_variant_cholesky(port):
     """lqr_step_backup's Cholesky(+1e-6 I) gains (used inside the DiLQR backward)."""
-    torch.manual_seed(0)
+    g = golden("ref_backup_chol.npz")
     torch.set_default_dtype(torch.float64)
     try:
-        ns, nc, T, B = 4, 2, 8, 6
-        n = ns + nc
-        A = torch.randn(T, B, n, n)
-        C = A.transpose(2, 3) @ A + torch.eye(n)
-        c = torch.randn(T, B, n)
-        F = torch.randn(T - 1, B, ns, n) / 2
-        x0 = torch.randn(B, ns)
-        m = R.mpc_backup.MPC(ns, nc, T, lqr_iter=1, verbose=-1, exit_unconverged=False)
-        xr, ur, _ = m(x0, R.mpc_backup.QuadCost(C, c), R.mpc_backup.LinDx(F, None))
-        o = port.mpc_forward(x0, port.QuadCost(C, c), port.LinDx(F, None), ns, nc, T, lqr_iter=1,
-                             gain_solve="chol_reg", final_pass=False)
-        assert float((o.u - ur).abs().max()) < 1e-13
+        ns, nc, T = 4, 2, 8
+        o = port.mpc_forward(g["x0"], port.QuadCost(g["C"], g["c"]), port.LinDx(g["F"], None), ns,
+                             nc, T, lqr_iter=1, gain_solve="chol_reg", final_pass=False)
+        assert float((o.u - g["u"]).abs().max()) < 1e-13
     finally:
         torch.set_default_dtype(torch.float32)
