@@ -20,7 +20,7 @@ PNQP_MAX_ITER = 20
 
 ERRORS = {0: "ok", -1: "invalid argument", -2: "unsupported (dtype, n_state, n_ctrl, dynamics)",
           -3: "pointer not 16-byte aligned", -4: "workspace too small",
-          -5: "CUDA launch failure", -6: "lockstep launch: batch not co-resident"}
+          -5: "CUDA launch failure", -6: "group sweep launch: batch does not fit the device"}
 
 
 class DilqrLibraryError(RuntimeError):
@@ -57,7 +57,7 @@ class DilqrSolve(C.Structure):
         ("bounds_kind", C.c_int32), ("solo", C.c_int32),
         ("max_linesearch_iter", C.c_int32), ("iteration", C.c_int32),
         ("has_f", C.c_int32), ("gains_only", C.c_int32), ("C_bcast", C.c_int32),
-        ("c_bcast", C.c_int32), ("lockstep", C.c_int32),
+        ("c_bcast", C.c_int32),
         ("linesearch_decay", C.c_double),
         ("u_lower", C.c_double), ("u_upper", C.c_double),
         ("best_cost_eps", C.c_double),
@@ -117,9 +117,7 @@ class DilqrWsView(C.Structure):
 SYMBOLS = {
     "dilqr_version": (C.c_char_p, []),
     "dilqr_supported": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int]),
-    "dilqr_lockstep_capacity": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int]),
-    "dilqr_group_sweep_capacity": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int]),
-    "dilqr_shape_staged": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int]),
+    "dilqr_mpc_plan": (C.c_int, [C.POINTER(DilqrSolve)]),
     "dilqr_workspace_bytes": (C.c_size_t, [C.POINTER(DilqrSolve)]),
     "dilqr_mpc_begin": (C.c_int, [C.POINTER(DilqrSolve), C.c_void_p]),
     "dilqr_mpc_iterate": (C.c_int, [C.POINTER(DilqrSolve), C.c_void_p]),
@@ -129,8 +127,6 @@ SYMBOLS = {
     "dilqr_workspace_view": (C.c_int, [C.POINTER(DilqrSolve), C.POINTER(DilqrWsView)]),
     "dilqr_lam_tables": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_double), C.c_int, C.c_int]
                          + [C.c_void_p] * 5),
-    "dilqr_sens_theta_blocked": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_double), C.c_int,
-                                           C.c_int] + [C.c_void_p] * 8),
     "dilqr_sens_theta_adjoint": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_double), C.c_int,
                                            C.c_int] + [C.c_void_p] * 9),
     "dilqr_last_iterate_launches": (C.c_int, []),
@@ -204,7 +200,7 @@ def check(code, what):
 KERNELS_PER_CALL = {
     "dilqr_mpc_begin": 1, "dilqr_mpc_iterate": 1, "dilqr_mpc_commit": 1,
     "dilqr_mpc_finish": 1, "dilqr_mpc_gains": 3, "dilqr_lam_tables": 1,
-    "dilqr_sens_theta_blocked": 1, "dilqr_sens_theta_adjoint": 1, "dilqr_kkt_grads": 1, "dilqr_linearize": 1, "dilqr_rollout": 1,
+    "dilqr_sens_theta_adjoint": 1, "dilqr_kkt_grads": 1, "dilqr_linearize": 1, "dilqr_rollout": 1,
     "dilqr_costate_tables": 1, "dilqr_richardson_update": 1, "dilqr_sens_theta": 1,
     "dilqr_adjoint_factor": 1, "dilqr_adjoint_pass": 1, "dilqr_adjoint_final": 1,
     "dilqr_pnqp": 2, "dilqr_env_tables": 1, "dilqr_tile_cost": 2, "dilqr_tile_cost_grad": 2,

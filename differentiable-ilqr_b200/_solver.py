@@ -6,15 +6,12 @@ Nothing here computes on the CPU; torch is used for device memory, streams and
 autograd plumbing only.
 """
 import ctypes as C
-import os
 
 import torch
 
 from . import _lib
 
 _DT = {torch.float32: _lib.F32, torch.float64: _lib.F64}
-# A/B knob: dtheta by the forward sensitivity rollout (round 1) instead of its adjoint form
-_SENS_ROLLOUT = bool(os.environ.get("DILQR_SENS_ROLLOUT"))
 
 
 def _ptr(t):
@@ -124,12 +121,6 @@ class Workspace:
 
 
 _ws_cache = {}
-_lockstep_cap = {}
-_group_cap = {}
-LOCKSTEP_AUTO = True
-GROUP_SWEEP = "auto"          # "auto" | "always" | "never"
-GROUP_SWEEP_BOXED = True      # auto: box-constrained multi-input batches use it even when the
-                              # register-resident lockstep kernel would fit
 
 
 def _require_cuda(t, name):
@@ -241,36 +232,13 @@ def _make_problem(x_init, C_, c_, dyn, n_state, n_ctrl, T, u_lower, u_upper, u_z
     if u_zero_I is not None:
         zi = dev(u_zero_I.expand(T, B, n_ctrl), "u_zero_I", torch.uint8)
         s.u_zero_I = _ptr(zi)
-    if not L.dilqr_supported(s.dtype, n_state, n_ctrl, dyn.kind):
+    # the library chooses how the iterations resolve pnqp's batch-global decisions
+    rc = L.dilqr_mpc_plan(C.byref(s))
+    if rc == -2:
         raise _lib.DilqrLibraryError(
             "no kernel compiled for dtype=%s n_state=%d n_ctrl=%d dynamics=%d "
             "(add it to DILQR_CONFIGS in csrc/api.cu)" % (dtype, n_state, n_ctrl, dyn.kind))
-    # multi-input box-constrained problems have long, unstable pnqp traces: resolve the
-    # batch-global decisions with grid barriers when the whole batch fits on the device
-    key = (s.dtype, n_state, n_ctrl, dyn.kind)
-    boxed_multi = s.bounds_kind != _lib.BOUNDS_NONE and not solo and n_ctrl > 1
-    cap = 0
-    if boxed_multi and LOCKSTEP_AUTO:
-        cap = _lockstep_cap.get(key)
-        if cap is None:
-            cap = L.dilqr_lockstep_capacity(*key)
-            _lockstep_cap[key] = cap
-        if B <= cap:
-            s.lockstep = 1
-    # Thread-group sweep (csrc/group_kernels.cuh): shapes too large for one thread per
-    # problem (their matrices would spill to local memory), and box-constrained multi-input
-    # batches -- its barriers need no problem to be resident, so it is exact at any size
-    if GROUP_SWEEP != "never":
-        gs = _group_cap.get(key)
-        if gs is None:
-            gs = (L.dilqr_group_sweep_capacity(*key), L.dilqr_shape_staged(*key))
-            _group_cap[key] = gs
-        gcap, staged = gs
-        want = GROUP_SWEEP == "always" or staged == 0 or (
-            boxed_multi and (B > cap or GROUP_SWEEP_BOXED))
-        if want and 0 < B <= gcap:
-            s.group_sweep = 1
-            s.lockstep = 0
+    _lib.check(rc, "dilqr_mpc_plan")
     need = L.dilqr_workspace_bytes(C.byref(s))
     # one workspace per (device, stream): solves on different streams never share scratch;
     # it only ever grows (the layout comes from the problem struct, not the buffer size)
@@ -435,8 +403,8 @@ def solve_mpc(x_init, C_, c_, dyn, n_state, n_ctrl, T, u_lower=None, u_upper=Non
         raise ValueError("solo=2 needs lqr_iter <= %d" % MAX_PIPELINED_ITERS)
     if n_loops > 1 and n_loops <= MAX_PIPELINED_ITERS and (
             (pipelined and verbose <= 0) or int(solo) == 2):
-        if int(solo) == 2 or s.lockstep:
-            deferred = None          # their host logic needs the statuses right away
+        if int(solo) == 2:
+            deferred = None          # its host logic needs the statuses right away
         _solve_pipelined(L, s, ws, info, n_loops, eps_cmp, not_improved_lim, verbose, deferred)
         n_loops = 0
     for i in range(n_loops):
@@ -819,14 +787,10 @@ def dilqr_backward(dl_dx, dl_du, x_init, C_, c_, x, u, dxmod, n_state, n_ctrl, u
     dtheta = torch.empty(B, nth, dtype=dtype, device=dev)
     if fused:
         dtau = prep["ws"][prep["dtau_off"]:]
-        if _SENS_ROLLOUT:   # A/B knob: the forward sensitivity rollout of round 1
-            _lib.call("dilqr_sens_theta_blocked", _DT[dtype], kind, theta, T, B, _ptr(x), _ptr(u),
-                      C.c_void_p(prep["Kk"]), _ptr(lam), _ptr(dtau), _ptr(df), _ptr(dtheta),
-                      _stream())
-        else:               # adjoint form: reverse sweep, second-order tables via the packed Lam
-            _lib.call("dilqr_sens_theta_adjoint", _DT[dtype], kind, theta, T, B, _ptr(x), _ptr(u),
-                      C.c_void_p(prep["Kk"]), _ptr(lam), _ptr(dtau), _ptr(df), _ptr(Lam),
-                      _ptr(dtheta), _stream())
+        # adjoint form: reverse sweep, second-order tables via the packed Lam
+        _lib.call("dilqr_sens_theta_adjoint", _DT[dtype], kind, theta, T, B, _ptr(x), _ptr(u),
+                  C.c_void_p(prep["Kk"]), _ptr(lam), _ptr(dtau), _ptr(df), _ptr(Lam),
+                  _ptr(dtheta), _stream())
     else:
         _lib.call("dilqr_sens_theta", _DT[dtype], kind, theta, T, B, _ptr(x), _ptr(u),
                   _ptr(prep["K"]), _ptr(lam), _ptr(dxa), _ptr(dua), _ptr(df), _ptr(dtheta), _stream())

@@ -1,8 +1,8 @@
-#include <cstdlib>
 // api.cu -- extern "C" entry points of libdilqr (see include/dilqr.h).
 // Compiled once per scalar type (-DDILQR_SCALAR_F64=0/1) into separate objects;
 // dispatch.cu routes on DilqrSolve::dtype.
 #include <cuda_runtime.h>
+#include <atomic>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -211,7 +211,7 @@ static IterParams<Scalar> make_params(const DilqrSolve* s, int role = 1) {
   p.gains_only = s->gains_only;
   p.C_bcast = s->C_bcast;
   p.c_bcast = s->c_bcast;
-  p.lockstep = s->lockstep || s->group_sweep;   // either way the votes ARE the pnqp trace
+  p.votes_are_trace = s->group_sweep;   // the group sweep decides at barriers: nothing to replay
   p.gsQ = reinterpret_cast<S*>(ws + w.gsQ);
   p.gsG = reinterpret_cast<S*>(ws + w.gsG);
   p.gs_barrier = reinterpret_cast<unsigned int*>(ws + w.gs_barrier);
@@ -268,15 +268,9 @@ struct Geometry {
     int w = (int)((112 * 1024) / per);  // <= ~112 KB / block so two blocks fit one SM
     if (w > 4) w = 4;
     if (w < 1) w = 1;
-    static const int forced = getenv("DILQR_WPB") ? atoi(getenv("DILQR_WPB")) : 0;  // tuning knob
-    if (forced >= 1 && forced <= w) w = forced;
     return w;
   }
-  static size_t smem(int wpb) {
-    // DILQR_SMEM_PAD: extra dynamic shared memory per block (occupancy experiments)
-    static const size_t pad = getenv("DILQR_SMEM_PAD") ? (size_t)atol(getenv("DILQR_SMEM_PAD")) : 0;
-    return STAGED ? IK::smem_per_warp() * wpb + pad : 0;
-  }
+  static size_t smem(int wpb) { return STAGED ? IK::smem_per_warp() * wpb : 0; }
 };
 
 template <int NS, int NC, int DYN>
@@ -302,12 +296,11 @@ static int launch_begin(const DilqrSolve* s, cudaStream_t st) {
   }
   (void)w;
   {  // 1: begin packs the upper triangle of C for the sweeps (ilqr_kernels.cuh), 0: dense
-    static const bool off = getenv("DILQR_NO_PACK") != nullptr;   // tuning / A-B knob
-    const bool pack = !p.C_bcast && !(p.gains_only && p.x_cur) && !off;
+    const bool pack = !p.C_bcast && !(p.gains_only && p.x_cur);
     cudaMemsetAsync(p.cpk_state, 0, sizeof(uint32_t), st);
     if (pack) cudaMemsetAsync(p.cpk_state, 1, 1, st);   // little-endian: word value 1
     // 3: broadcast C, symmetry of the shared block(s) to be verified by begin
-    if (p.C_bcast && !(p.gains_only && p.x_cur) && !off) cudaMemsetAsync(p.cpk_state, 3, 1, st);
+    if (p.C_bcast && !(p.gains_only && p.x_cur)) cudaMemsetAsync(p.cpk_state, 3, 1, st);
     // ticket counter of the one-launch commit (returns to zero after every commit)
     cudaMemsetAsync(static_cast<char*>(s->workspace) + w.commit_ticket, 0, sizeof(uint32_t), st);
   }
@@ -323,26 +316,46 @@ constexpr bool group_sweep_v() {
   return (DYN == DYN_LINDX || DYN == DYN_ROCKET) && (!staged_v<S, NS, NC, DYN>() || NC > 1);
 }
 
+// Largest batch the group sweep holds on the current device (0: no group sweep for the shape):
+// one phase-B thread per problem, every block co-resident.  Queried once per (device, shape);
+// the query also raises the kernel's dynamic shared-memory limit on that device, which every
+// later launch there relies on.
 template <int NS, int NC, int DYN>
-static int group_sweep_blocks(int* max_blocks) {
+static int group_sweep_capacity() {
   using S = Scalar;
   if constexpr (!group_sweep_v<S, NS, NC, DYN>()) {
-    *max_blocks = 0;
     return 0;
   } else {
+    constexpr int kMaxDevices = 64;
+    static std::atomic<int> cached[kMaxDevices];   // capacity + 1; 0: not queried yet
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess) return 0;
+    if (dev < kMaxDevices && cached[dev].load() > 0) return cached[dev].load() - 1;
     using GS = GroupSweep<S, NS, NC, DYN>;
     auto kern = group_sweep_kernel<S, NS, NC, DYN>;
     const size_t smem = GS::smem_bytes();
     if (smem > 48 * 1024)
       cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    int per_sm = 0, dev = 0, sms = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return 0;
+    int per_sm = 0, sms = 0;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, GS::kThreads, smem) != cudaSuccess)
       return 0;
-    *max_blocks = per_sm * sms;
-    return per_sm * sms * GS::kThreads;     // one phase-B thread per problem
+    const int cap = per_sm * sms * GS::kThreads;
+    if (dev < kMaxDevices) cached[dev].store(cap + 1);
+    return cap;
   }
+}
+
+// dilqr_mpc_plan: the group sweep for shapes too large for one thread per problem and for
+// box-constrained multi-input batches, as long as the batch fits the device; trace replay
+// otherwise.  The compile-time tests come first, so most shapes never query the device.
+template <int NS, int NC, int DYN>
+static int plan(DilqrSolve* s) {
+  using S = Scalar;
+  const bool boxed_multi = s->bounds_kind != DILQR_BOUNDS_NONE && s->solo == 0 && NC > 1;
+  s->group_sweep = group_sweep_v<S, NS, NC, DYN>() && (!staged_v<S, NS, NC, DYN>() || boxed_multi) &&
+                   s->n_batch > 0 && s->n_batch <= group_sweep_capacity<NS, NC, DYN>();
+  return DILQR_OK;
 }
 
 template <int NS, int NC, int DYN>
@@ -352,9 +365,9 @@ static int launch_group_sweep(const DilqrSolve* s, IterParams<Scalar>& p, cudaSt
     return DILQR_EUNSUPPORTED;
   } else {
     using GS = GroupSweep<S, NS, NC, DYN>;
-    int max_blocks = 0;
-    const int cap = group_sweep_blocks<NS, NC, DYN>(&max_blocks);
+    const int cap = group_sweep_capacity<NS, NC, DYN>();
     if (p.B > cap) return DILQR_ELOCKSTEP;
+    const int max_blocks = cap / GS::kThreads;
     const int need_b = (p.B + GS::kThreads - 1) / GS::kThreads;       // phase B: thread per problem
     const int want_ac = (p.B + GS::GPB - 1) / GS::GPB;               // phase AC: group per problem
     int blocks = want_ac < max_blocks ? want_ac : max_blocks;
@@ -380,82 +393,37 @@ static int launch_iterate(const DilqrSolve* s, cudaStream_t st) {
   using S = Scalar;
   using G = Geometry<S, NS, NC, DYN>;
   IterParams<S> p = make_params(s);
+  const int wpb = G::warps_per_block();
+  const int warps = (p.B + kWarp - 1) / kWarp;
+  const int blocks = (warps + wpb - 1) / wpb;
+  const size_t smem = G::smem(wpb);
+  g_iterate_launches = 0;
   if (s->group_sweep) {
     // Riccati / pnqp sweep by thread groups, all problems in step; then the line-search
     // rollout (one thread per problem: its state is small) as a second launch
     int rc = launch_group_sweep<NS, NC, DYN>(s, p, st);
     if (rc != DILQR_OK) return rc;
+    g_iterate_launches = 1;
     if (p.gains_only) return DILQR_OK;
     if constexpr (group_sweep_v<S, NS, NC, DYN>()) {
-      const int wpb = G::warps_per_block();
-      const int warps = (p.B + kWarp - 1) / kWarp;
-      const size_t smem = G::smem(wpb);
-      auto fwd = ilqr_iter_kernel<S, NS, NC, DYN, G::STAGED, false, 2>;
+      auto fwd = ilqr_iter_kernel<S, NS, NC, DYN, G::STAGED, true>;
       if (smem > 48 * 1024)
         cudaFuncSetAttribute(fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      p.lockstep = 0;
-      fwd<<<(warps + wpb - 1) / wpb, wpb * kWarp, smem, st>>>(p);
+      fwd<<<blocks, wpb * kWarp, smem, st>>>(p);
+      g_iterate_launches = 2;
     }
     return cudaGetLastError() == cudaSuccess ? DILQR_OK : DILQR_ECUDA;
   }
-  const int wpb = G::warps_per_block();
-  const int warps = (p.B + kWarp - 1) / kWarp;
-  const int blocks = (warps + wpb - 1) / wpb;
-  const size_t smem = G::smem(wpb);
   if (p.bounds_kind && !p.solo)
     cudaMemsetAsync(p.votes, 0, (size_t)p.T * kPnqpMaxIter * sizeof(uint32_t), st);
-  if constexpr (NC > 1) {
-    if (p.lockstep && p.bounds_kind && !p.solo) {
-      // cooperative launch, one warp per block so that every warp of the grid owns
-      // problems (all warps must reach every grid barrier); needs the whole batch
-      // resident -- dilqr_lockstep_capacity() tells the caller whether it fits.
-      auto kern = ilqr_iter_kernel<S, NS, NC, DYN, G::STAGED, true>;
-      const size_t smem1 = G::smem(1);
-      if (smem1 > 48 * 1024)
-        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1);
-      void* args[] = {(void*)&p};
-      cudaError_t e = cudaLaunchCooperativeKernel((const void*)kern, dim3(warps), dim3(kWarp), args,
-                                                  smem1, st);
-      if (e != cudaSuccess) {
-        cudaGetLastError();
-        return DILQR_ELOCKSTEP;
-      }
-      return DILQR_OK;
-    }
-  }
-  if (s->lockstep && NC == 1 && p.bounds_kind && !p.solo) return DILQR_ELOCKSTEP;
-  p.lockstep = 0;
   g_iterate_launches = 1;
-  // Split iteration, an experiment kept behind DILQR_SPLIT=1 (measured, DESIGN section 9): the
-  // sweep needs ~240 registers in FP64 (8 warps/SM, two rounds of resident warps at B = 65536),
-  // the line-search rollout only 128 -- as its own launch (one thread per problem, operands
-  // straight from the blocked workspace through L2 prefetches, 16 warps/SM) the whole batch is
-  // one wave.  It is SLOWER (0.51 vs 0.45 ms per iteration in FP64, 0.32 vs 0.28 in FP32): with
-  // every warp in the rollout at once that launch is HBM-bound (1.2 GB, >= 0.19 ms), while the
-  // fused kernel hides the rollout's traffic behind the sweeps of the other warps.
-  if constexpr (G::STAGED && DYN != DYN_LINDX && DYN != DYN_NN && NS + NC <= 6) {
-    static const int knob = getenv("DILQR_SPLIT") ? atoi(getenv("DILQR_SPLIT")) : -1;
-    const bool split = knob > 0;
-    if (split) {
-      auto sweep = ilqr_iter_kernel<S, NS, NC, DYN, G::STAGED, false, 1>;
-      if (smem > 48 * 1024)
-        cudaFuncSetAttribute(sweep, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      sweep<<<blocks, wpb * kWarp, smem, st>>>(p);
-      if (!p.gains_only) {
-        auto roll = ilqr_iter_kernel<S, NS, NC, DYN, false, false, 2>;
-        roll<<<(warps + 3) / 4, 4 * kWarp, 0, st>>>(p);
-        g_iterate_launches = 2;
-      }
-      return cudaGetLastError() == cudaSuccess ? DILQR_OK : DILQR_ECUDA;
-    }
-  }
-  auto kern = ilqr_iter_kernel<S, NS, NC, DYN, G::STAGED, false>;
+  auto kern = ilqr_iter_kernel<S, NS, NC, DYN, G::STAGED>;
   if (smem > 48 * 1024)
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if constexpr (sym_pair_v<S, NS, NC, DYN>()) {
     // symmetric Riccati update when the packed copy of C is valid (ilqr_kernels.cuh, kSym): the
     // flag is on the device, so both kernels of the pair are enqueued and one exits at once
-    auto ksym = ilqr_iter_kernel<S, NS, NC, DYN, G::STAGED, false, 0, true>;
+    auto ksym = ilqr_iter_kernel<S, NS, NC, DYN, G::STAGED, false, true>;
     if (smem > 48 * 1024)
       cudaFuncSetAttribute(ksym, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     p.sym_pair = 1;
@@ -478,7 +446,6 @@ static int launch_gains(const DilqrSolve* s, void* lam_blk, cudaStream_t st) {
     if (s->u_zero_I || (s->bounds_kind && !s->solo && NC > 1)) return DILQR_EUNSUPPORTED;
     IterParams<S> p = make_params(s);
     p.gains_only = 1;
-    p.lockstep = 0;
     p.lam_blk = static_cast<S*>(lam_blk);
     using IK = typename G::IK;
     size_t per = IK::smem_per_warp(true);
@@ -510,7 +477,7 @@ static int launch_gains(const DilqrSolve* s, void* lam_blk, cudaStream_t st) {
     }
     kern<<<blocks, wpb * kWarp, smem, st>>>(p);
     trace_verify_kernel<<<1, 256, 0, st>>>(p.guess, p.votes, p.T, p.bounds_kind != 0, p.solo,
-                                           s->status, 0, nullptr);
+                                           s->status);
     return cudaGetLastError() == cudaSuccess ? DILQR_OK : DILQR_ECUDA;
   }
 }
@@ -525,7 +492,7 @@ static int launch_commit(const DilqrSolve* s, cudaStream_t st) {
   aux.part = reinterpret_cast<CommitPart*>(ws + w.commit_part);
   aux.ticket = reinterpret_cast<unsigned int*>(ws + w.commit_ticket);
   aux.ctrl = s->control;
-  aux.lockstep = p.lockstep;
+  aux.votes_are_trace = p.votes_are_trace;
   aux.iteration = s->iteration;
   commit_kernel<S, NS + NC, NC><<<(p.B + 127) / 128, 128, 0, st>>>(p, aux);
   return cudaGetLastError() == cudaSuccess ? DILQR_OK : DILQR_ECUDA;
@@ -548,23 +515,6 @@ static int launch_kkt(const DilqrKkt* k, cudaStream_t st) {
 }
 
 // ------------------------------------------------------------------ dispatch
-template <int NS, int NC, int DYN>
-static int lockstep_capacity() {
-  using S = Scalar;
-  using G = Geometry<S, NS, NC, DYN>;
-  if (NC == 1) return 0;   // single-input problems replay the (always right) closed-form trace
-  auto kern = ilqr_iter_kernel<S, NS, NC, DYN, G::STAGED, true>;
-  const size_t smem1 = G::smem(1);
-  if (smem1 > 48 * 1024)
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1);
-  int per_sm = 0, dev = 0, sms = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess) return 0;
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kWarp, smem1) != cudaSuccess)
-    return 0;
-  return per_sm * sms * kWarp;
-}
-
 enum Op { OP_BEGIN, OP_ITERATE, OP_COMMIT, OP_FINISH };
 
 static int dispatch(const DilqrSolve* s, Op op, cudaStream_t st) {
@@ -582,29 +532,12 @@ static int dispatch(const DilqrSolve* s, Op op, cudaStream_t st) {
   return DILQR_EUNSUPPORTED;
 }
 
-int DILQR_SUFFIX(lockstep_capacity)(int n_state, int n_ctrl, int dynamics) {
+int DILQR_SUFFIX(mpc_plan)(DilqrSolve* s) {
 #define X(NS_, NC_, DYN_) \
-  if (n_state == NS_ && n_ctrl == NC_ && dynamics == DYN_) return lockstep_capacity<NS_, NC_, DYN_>();
+  if (s->n_state == NS_ && s->n_ctrl == NC_ && s->dynamics == DYN_) return plan<NS_, NC_, DYN_>(s);
   DILQR_CONFIGS(X)
 #undef X
-  return 0;
-}
-
-int DILQR_SUFFIX(group_sweep_capacity)(int n_state, int n_ctrl, int dynamics) {
-  int mb = 0;
-#define X(NS_, NC_, DYN_) \
-  if (n_state == NS_ && n_ctrl == NC_ && dynamics == DYN_) return group_sweep_blocks<NS_, NC_, DYN_>(&mb);
-  DILQR_CONFIGS(X)
-#undef X
-  return 0;
-}
-
-int DILQR_SUFFIX(shape_staged)(int n_state, int n_ctrl, int dynamics) {
-#define X(NS_, NC_, DYN_) \
-  if (n_state == NS_ && n_ctrl == NC_ && dynamics == DYN_) return staged_v<Scalar, NS_, NC_, DYN_>() ? 1 : 0;
-  DILQR_CONFIGS(X)
-#undef X
-  return -1;
+  return DILQR_EUNSUPPORTED;
 }
 
 int DILQR_SUFFIX(supported)(int n_state, int n_ctrl, int dynamics) {
@@ -953,33 +886,6 @@ int DILQR_SUFFIX(lam_tables)(int dynamics, const double* dp, int T, int B, const
   if (dynamics == DYN_PENDULUM) return launch_lam_tables<DYN_PENDULUM>(dp, T, B, x, u, lam_blk, Lam, st);
   if (dynamics == DYN_CARTPOLE) return launch_lam_tables<DYN_CARTPOLE>(dp, T, B, x, u, lam_blk, Lam, st);
   if (dynamics == DYN_ROCKET) return launch_lam_tables<DYN_ROCKET>(dp, T, B, x, u, lam_blk, Lam, st);
-  return DILQR_EUNSUPPORTED;
-}
-
-template <int DYN>
-static int launch_sens_blocked(const double* dp, int T, int B, const void* x, const void* u,
-                               const void* Kk, const void* lam, const void* dtau, const void* df,
-                               void* dtheta, cudaStream_t st) {
-  using S = Scalar;
-  DynParams<S> P;
-  memset(&P, 0, sizeof(P));
-  for (int i = 0; i < 8; ++i) P.p[i] = (S)dp[i];
-  const int Bp = (B + kWarp - 1) / kWarp * kWarp;
-  sens_theta_kernel<S, DYN, true><<<(Bp + 63) / 64, 64, 0, st>>>(
-      P, T, B, static_cast<const S*>(x), static_cast<const S*>(u), static_cast<const S*>(Kk),
-      static_cast<const S*>(lam), static_cast<const S*>(dtau), nullptr,
-      static_cast<const S*>(df), static_cast<S*>(dtheta));
-  return cudaGetLastError() == cudaSuccess ? DILQR_OK : DILQR_ECUDA;
-}
-
-int DILQR_SUFFIX(sens_theta_blocked)(int dynamics, const double* dp, int T, int B, const void* x,
-                                     const void* u, const void* Kk, const void* lam,
-                                     const void* dtau, const void* df, void* dtheta, void* stream) {
-  if (!dp || !x || !u || !Kk || !lam || !dtau || !df || !dtheta || T <= 1 || B <= 0)
-    return DILQR_EINVAL;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (dynamics == DYN_PENDULUM) return launch_sens_blocked<DYN_PENDULUM>(dp, T, B, x, u, Kk, lam, dtau, df, dtheta, st);
-  if (dynamics == DYN_CARTPOLE) return launch_sens_blocked<DYN_CARTPOLE>(dp, T, B, x, u, Kk, lam, dtau, df, dtheta, st);
   return DILQR_EUNSUPPORTED;
 }
 

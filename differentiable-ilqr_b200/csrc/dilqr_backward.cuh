@@ -292,11 +292,7 @@ __global__ void richardson_update_kernel(int T, int B, const S* __restrict__ g,
 //   lam    [T,B,ns]     primal costates           dx,du: adjoint solution (r = w)
 //   df     [T-1,B,ns]   = -dlam_{t+1}             dtheta [B,nth]
 // ---------------------------------------------------------------------------
-// BLK: K, lam, dtau, df come in the warp-blocked workspace layouts the fused backward keeps
-// them in (Kk[T][B/32][NC*NS+NC][32] of the gains sweep, lam[T][B/32][NS][32],
-// dtau[T][B/32][N][32] and df[T-1][B/32][NS][32] of the final adjoint pass): coalesced reads,
-// and none of them is ever gathered into the API layout.
-template <class S, int DYN, bool BLK = false>
+template <class S, int DYN>
 __global__ void __launch_bounds__(128)
 sens_theta_kernel(DynParams<S> P, int T, int B, const S* __restrict__ x,
                   const S* __restrict__ u, const S* __restrict__ K, const S* __restrict__ lam,
@@ -305,24 +301,14 @@ sens_theta_kernel(DynParams<S> P, int T, int B, const S* __restrict__ x,
   using D = Dyn<S, DYN>;
   using TB = EnvTables<S, DYN>;
   constexpr int NS = D::NS, NC = D::NC, N = D::N, NTH = TB::NTH;
-  constexpr int NK = NC * NS + NC;
-  const int bw = blockIdx.x * blockDim.x + threadIdx.x;
-  const int nW = (B + kWarp - 1) / kWarp;
-  if (BLK ? (bw >= nW * kWarp) : (bw >= B)) return;
-  const int b = bw < B ? bw : B - 1;
-  auto ldK = [&](int t, int e) -> S {
-    return BLK ? K[bidx(t, e, NK, bw, nW)] : K[((size_t)t * B + b) * (NC * NS) + e];
-  };
-  auto ldlam = [&](int t, int i) -> S {
-    return BLK ? lam[bidx(t, i, NS, bw, nW)] : lam[((size_t)t * B + b) * NS + i];
-  };
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  auto ldK = [&](int t, int e) -> S { return K[((size_t)t * B + b) * (NC * NS) + e]; };
+  auto ldlam = [&](int t, int i) -> S { return lam[((size_t)t * B + b) * NS + i]; };
   auto lddtau = [&](int t, int i) -> S {
-    if (BLK) return dx[bidx(t, i, N, bw, nW)];
     return i < NS ? dx[((size_t)t * B + b) * NS + i] : du[((size_t)t * B + b) * NC + (i - NS)];
   };
-  auto lddf = [&](int t, int i) -> S {
-    return BLK ? df[bidx(t, i, NS, bw, nW)] : df[((size_t)t * B + b) * NS + i];
-  };
+  auto lddf = [&](int t, int i) -> S { return df[((size_t)t * B + b) * NS + i]; };
   S G[NS][NTH], Gp[NS][NTH], Dprev[NS][N], Kp[NC][NS];
   S acc[NTH];
 #pragma unroll
@@ -337,13 +323,11 @@ sens_theta_kernel(DynParams<S> P, int T, int B, const S* __restrict__ x,
       const size_t nb = tb + B;
       prefetch_l1(x + nb * NS);
       prefetch_l1(u + nb * NC);
-      if (!BLK) {
-        prefetch_l1(dx + nb * NS);
-        prefetch_l1(du + nb * NC);
-        prefetch_l1(lam + nb * NS);
-        prefetch_l1(df + tb * NS);
-        if (t + 2 < T) prefetch_l1(K + ((size_t)(T - 2 - t) * B + b) * (NC * NS));
-      }
+      prefetch_l1(dx + nb * NS);
+      prefetch_l1(du + nb * NC);
+      prefetch_l1(lam + nb * NS);
+      prefetch_l1(df + tb * NS);
+      if (t + 2 < T) prefetch_l1(K + ((size_t)(T - 2 - t) * B + b) * (NC * NS));
     }
     S tau[N], dtau[N];
 #pragma unroll
@@ -457,10 +441,8 @@ sens_theta_kernel(DynParams<S> P, int T, int B, const S* __restrict__ x,
 #pragma unroll
       for (int j = 0; j < NS; ++j) Kp[a][j] = Kt[a][j];
   }
-  if (bw < B) {
 #pragma unroll
-    for (int q = 0; q < NTH; ++q) dtheta[(size_t)b * NTH + q] = acc[q];
-  }
+  for (int q = 0; q < NTH; ++q) dtheta[(size_t)b * NTH + q] = acc[q];
 }
 
 // ---------------------------------------------------------------------------

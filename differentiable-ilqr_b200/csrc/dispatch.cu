@@ -6,9 +6,7 @@ namespace dilqr {
 // shape-specialised entry points: one copy per (dtype, shape group)
 #define DECL_G(sfx)                                                                       \
   int supported_##sfx(int, int, int);                                                     \
-  int lockstep_capacity_##sfx(int, int, int);                                             \
-  int group_sweep_capacity_##sfx(int, int, int);                                          \
-  int shape_staged_##sfx(int, int, int);                                                  \
+  int mpc_plan_##sfx(DilqrSolve*);                                                        \
   int mpc_begin_##sfx(const DilqrSolve*, void*);                                          \
   int mpc_iterate_##sfx(const DilqrSolve*, void*);                                        \
   int mpc_commit_##sfx(const DilqrSolve*, void*);                                         \
@@ -36,8 +34,6 @@ namespace dilqr {
   int workspace_view_##sfx(const DilqrSolve*, DilqrWsView*);                              \
   int lam_tables_##sfx(int, const double*, int, int, const void*, const void*, const void*, \
                        void*, void*);                                                     \
-  int sens_theta_blocked_##sfx(int, const double*, int, int, const void*, const void*,    \
-                               const void*, const void*, const void*, const void*, void*, void*); \
   int sens_theta_adjoint_##sfx(int, const double*, int, int, const void*, const void*,    \
                                const void*, const void*, const void*, const void*, const void*, \
                                void*, void*);                                             \
@@ -86,37 +82,9 @@ int dilqr_supported(int dtype, int ns, int nc, int dyn) {
   return 0;
 }
 
-int dilqr_lockstep_capacity(int dtype, int ns, int nc, int dyn) {
-  if (dtype == DILQR_F32)
-    return dilqr::lockstep_capacity_f32_g0(ns, nc, dyn) + dilqr::lockstep_capacity_f32_g1(ns, nc, dyn) +
-           dilqr::lockstep_capacity_f32_g2(ns, nc, dyn) + dilqr::lockstep_capacity_f32_g3(ns, nc, dyn);
-  if (dtype == DILQR_F64)
-    return dilqr::lockstep_capacity_f64_g0(ns, nc, dyn) + dilqr::lockstep_capacity_f64_g1(ns, nc, dyn) +
-           dilqr::lockstep_capacity_f64_g2(ns, nc, dyn) + dilqr::lockstep_capacity_f64_g3(ns, nc, dyn);
-  return 0;
-}
-
-int dilqr_group_sweep_capacity(int dtype, int ns, int nc, int dyn) {
-  if (dtype == DILQR_F32)
-    return dilqr::group_sweep_capacity_f32_g0(ns, nc, dyn) + dilqr::group_sweep_capacity_f32_g1(ns, nc, dyn) +
-           dilqr::group_sweep_capacity_f32_g2(ns, nc, dyn) + dilqr::group_sweep_capacity_f32_g3(ns, nc, dyn);
-  if (dtype == DILQR_F64)
-    return dilqr::group_sweep_capacity_f64_g0(ns, nc, dyn) + dilqr::group_sweep_capacity_f64_g1(ns, nc, dyn) +
-           dilqr::group_sweep_capacity_f64_g2(ns, nc, dyn) + dilqr::group_sweep_capacity_f64_g3(ns, nc, dyn);
-  return 0;
-}
-
-int dilqr_shape_staged(int dtype, int ns, int nc, int dyn) {
-  int r = -1;
-  for (int g = 0; g < 4 && r < 0; ++g) {
-    if (dtype == DILQR_F32)
-      r = g == 0 ? dilqr::shape_staged_f32_g0(ns, nc, dyn) : g == 1 ? dilqr::shape_staged_f32_g1(ns, nc, dyn)
-        : g == 2 ? dilqr::shape_staged_f32_g2(ns, nc, dyn) : dilqr::shape_staged_f32_g3(ns, nc, dyn);
-    else if (dtype == DILQR_F64)
-      r = g == 0 ? dilqr::shape_staged_f64_g0(ns, nc, dyn) : g == 1 ? dilqr::shape_staged_f64_g1(ns, nc, dyn)
-        : g == 2 ? dilqr::shape_staged_f64_g2(ns, nc, dyn) : dilqr::shape_staged_f64_g3(ns, nc, dyn);
-  }
-  return r;
+int dilqr_mpc_plan(DilqrSolve* s) {
+  if (!s) return DILQR_EINVAL;
+  BY_DTYPE_GROUPS(s->dtype, mpc_plan, s);
 }
 
 size_t dilqr_workspace_bytes(const DilqrSolve* s) {
@@ -152,15 +120,6 @@ int dilqr_lam_tables(int dtype, int dyn, const double* dp, int T, int B, const v
                      const void* u, const void* lam_blk, void* Lam, void* st) {
   return ROUTE(dtype, dilqr::lam_tables_f32_g0(dyn, dp, T, B, x, u, lam_blk, Lam, st),
                dilqr::lam_tables_f64_g0(dyn, dp, T, B, x, u, lam_blk, Lam, st));
-}
-int dilqr_sens_theta_blocked(int dtype, int dyn, const double* dp, int T, int B, const void* x,
-                             const void* u, const void* Kk, const void* lam_blk,
-                             const void* dtau_blk, const void* df_blk, void* dtheta, void* st) {
-  return ROUTE(dtype,
-               dilqr::sens_theta_blocked_f32_g0(dyn, dp, T, B, x, u, Kk, lam_blk, dtau_blk, df_blk,
-                                                dtheta, st),
-               dilqr::sens_theta_blocked_f64_g0(dyn, dp, T, B, x, u, Kk, lam_blk, dtau_blk, df_blk,
-                                                dtheta, st));
 }
 int dilqr_sens_theta_adjoint(int dtype, int dyn, const double* dp, int T, int B, const void* x,
                              const void* u, const void* Kk, const void* lam_blk,

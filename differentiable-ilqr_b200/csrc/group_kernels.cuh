@@ -364,9 +364,9 @@ struct GroupSweep {
       bool If[NC];
       LUpp<S, NC> lu;
       S rinv = S(0);
-      pnqp_thread<S, NC, 2>(H, qu, lo, hi, have_prev, k, If, lu,
-                            p.guess + (size_t)t * kPnqpMaxIter, make_uint4(0, 0, 0, 0),
-                            p.votes + (size_t)t * kPnqpMaxIter, p.solo != 0, active, lane, &rinv, &sb);
+      pnqp_thread<S, NC, true>(H, qu, lo, hi, have_prev, k, If, lu,
+                               p.guess + (size_t)t * kPnqpMaxIter, make_uint4(0, 0, 0, 0),
+                               p.votes + (size_t)t * kPnqpMaxIter, p.solo != 0, active, lane, &rinv, &sb);
       have_prev = true;
 #pragma unroll
       for (int a = 0; a < NC; ++a) {

@@ -34,7 +34,6 @@
 // zero: the trace of the previous iLQR iteration is the next guess) the result
 // is exactly what the reference computes on the whole batch.
 #pragma once
-#include <cooperative_groups.h>
 #include "common.cuh"
 #include "dynamics.cuh"
 #include "env_tables_gen.cuh"
@@ -80,7 +79,7 @@ struct IterParams {
   int* take;          // [Bp] 1: the problem's best iterate is the CURRENT trajectory and
                       //         has not been copied to traj_best yet (lazy best tracking)
   int gains_only;     // skip the line-search rollout (only K,k are wanted)
-  int lockstep;       // cooperative launch: grid-wide barriers resolve the pnqp decisions
+  int votes_are_trace;  // the group sweep resolved the pnqp decisions at barriers: no replay
   int C_bcast, c_bcast;  // cost layout: 0 dense [T,B,..], 1 batch-broadcast [T,..], 2 [..] only
   S* cost_cur;    // [Bp]
   S* cost_new;
@@ -208,30 +207,23 @@ struct SubBarrier {
   }
 };
 
-// LOCKSTEP: 0 replay a guessed trace; 1 decide with grid-wide barriers (cooperative launch,
-// every thread of the grid takes part); 2 decide with a SubBarrier (`sb`).
-template <class S, int N, int LOCKSTEP = 0>
+// BARRIER: false replays a guessed trace; true decides with a SubBarrier (`sb`).
+template <class S, int N, bool BARRIER = false>
 DILQR_DEVICE void pnqp_thread(const S (&H)[N][N], const S (&q)[N], const S (&lo)[N],
                               const S (&hi)[N], bool have_init, S (&x)[N], bool (&If)[N],
                               LUpp<S, N>& lu, const uint32_t* __restrict__ guess, uint4 gpre,
                               uint32_t* __restrict__ votes, bool solo, bool active, int lane,
                               S* rinv_out = nullptr, SubBarrier* sb = nullptr) {
-  constexpr bool lockstep = LOCKSTEP != 0;
   // N == 1: 1 / (masked Hessian) of the last evaluated iteration, handed to the caller
   // (which needs the same quotient for K, lqr_step.py:144-146) and reused across
   // iterations while the operand is unchanged -- same value, one division instead of three.
   S h_last = S(0), r_last = S(0);
   bool have_r = false;
-  // lockstep: the kernel was launched cooperatively with the whole batch resident;
-  // every batch-global decision is an atomicOr into the vote word + a grid-wide
-  // barrier (no guessing, no re-runs) -- the better trade when the control-flow trace
-  // is long and unstable (multi-input problems with many active constraints).
+  // BARRIER: every batch-global decision is an atomicOr into the vote word + a barrier over
+  // the whole batch (no guessing, no re-runs) -- the better trade when the control-flow
+  // trace is long and unstable (multi-input problems with many active constraints).
   auto grid_decide = [&](uint32_t* word, uint32_t mine) -> uint32_t {
-    if constexpr (LOCKSTEP == 1) {
-      if (mine && lane == 0) atomicOr(word, mine);
-      cooperative_groups::this_grid().sync();
-      return *reinterpret_cast<volatile uint32_t*>(word);
-    } else if constexpr (LOCKSTEP == 2) {
+    if constexpr (BARRIER) {
       if (mine && lane == 0) atomicOr(word, mine);
       sb->sync();
       return *reinterpret_cast<volatile uint32_t*>(word);
@@ -313,7 +305,7 @@ DILQR_DEVICE void pnqp_thread(const S (&H)[N][N], const S (&q)[N], const S (&lo)
     bool any_moving;
     if (solo) {
       any_moving = J;
-    } else if (lockstep) {
+    } else if (BARRIER) {
       if (__ballot_sync(kFull, active && J)) vote |= 1u;
       any_moving = (grid_decide(&votes[it], vote) & 1u) != 0;
     } else {
@@ -321,7 +313,7 @@ DILQR_DEVICE void pnqp_thread(const S (&H)[N][N], const S (&q)[N], const S (&lo)
       any_moving = (gword_at(it) & 1u) != 0;
     }
     if (!any_moving) {  // pnqp.py:57-59
-      if (!solo && !lockstep && vote && lane == 0) vote_or(&votes[it], vote);
+      if (!solo && !BARRIER && vote && lane == 0) vote_or(&votes[it], vote);
       return;
     }
     // Armijo backtracking with a batch-global exit test (pnqp.py:61-76).
@@ -341,7 +333,7 @@ DILQR_DEVICE void pnqp_thread(const S (&H)[N][N], const S (&q)[N], const S (&lo)
     }
     S alpha = S(1);
     S mx[N];
-    const uint32_t gword = (solo || lockstep) ? 0u : gword_at(it);
+    const uint32_t gword = (solo || BARRIER) ? 0u : gword_at(it);
     for (int cnt = 0; cnt < kArmijoMax; ++cnt) {
 #pragma unroll
       for (int i = 0; i < N; ++i) mx[i] = eclamp<S>(x[i] + alpha * dx[i], lo[i], hi[i]);
@@ -366,7 +358,7 @@ DILQR_DEVICE void pnqp_thread(const S (&H)[N][N], const S (&q)[N], const S (&lo)
       bool exit_loop;
       if (solo) {
         exit_loop = !small;
-      } else if (lockstep) {
+      } else if (BARRIER) {
         const uint32_t mine = __ballot_sync(kFull, active && !small) ? (2u << cnt) : 0u;
         exit_loop = (grid_decide(&votes[it], mine) >> (1 + cnt)) & 1u;
       } else {
@@ -378,7 +370,7 @@ DILQR_DEVICE void pnqp_thread(const S (&H)[N][N], const S (&q)[N], const S (&lo)
     }
 #pragma unroll
     for (int i = 0; i < N; ++i) x[i] = mx[i];  // pnqp.py:78
-    if (!solo && !lockstep && vote && lane == 0) vote_or(&votes[it], vote);
+    if (!solo && !BARRIER && vote && lane == 0) vote_or(&votes[it], vote);
   }
   // fell through n_iter iterations: the reference returns the factors / If of the
   // last iteration together with the stepped x (pnqp.py:81-82).
@@ -410,7 +402,7 @@ constexpr bool kChainFmaOn = DILQR_CHAIN_FMA != 0;
 #endif
 constexpr bool kSymRiccatiOn = DILQR_SYM_RICCATI != 0;
 
-template <class S, int NS, int NC, int DYN, bool STAGED, bool LOCKSTEP = false, bool SYM = false>
+template <class S, int NS, int NC, int DYN, bool STAGED, bool SYM = false>
 struct IterKernel {
   static constexpr int N = NS + NC;
   static constexpr int NK = NC * NS + NC;
@@ -620,7 +612,7 @@ struct IterKernel {
     // two shuffles.  A global load per timestep -- wherever it is placed -- costs an exposed L2
     // round trip: ptxas makes an unrelated instruction next to it wait on the shared scoreboard
     // (ncu: 400 cycles per timestep, profiles/r2_iter_stalls.txt).
-    const bool use_guess = p.bounds_kind && !p.solo && !LOCKSTEP;
+    const bool use_guess = p.bounds_kind && !p.solo;
     uint2 glane = make_uint2(0, 0);
     for (int t = T - 1; t >= 0; --t) {
       const int sg = (T - 1 - t) & 1;
@@ -837,10 +829,9 @@ struct IterKernel {
           gpre.x = __shfl_sync(kFull, glane.x, t & 31);
           gpre.y = __shfl_sync(kFull, glane.y, t & 31);
         }
-        pnqp_thread<S, NC, LOCKSTEP ? 1 : 0>(H, qu, lo, hi, have_prev, k, If, lu,
-                                     p.guess + (size_t)t * kPnqpMaxIter, gpre,
-                                     p.votes + (size_t)t * kPnqpMaxIter, p.solo != 0, active, lane,
-                                     &rinv);
+        pnqp_thread<S, NC>(H, qu, lo, hi, have_prev, k, If, lu, p.guess + (size_t)t * kPnqpMaxIter,
+                           gpre, p.votes + (size_t)t * kPnqpMaxIter, p.solo != 0, active, lane,
+                           &rinv);
         have_prev = true;
 #pragma unroll
         for (int a = 0; a < NC; ++a) kprev[a] = k[a];
@@ -1045,19 +1036,16 @@ struct IterKernel {
 // one SM: a 65536-problem batch (2048 warps, 13.8 per SM) then runs as ONE wave instead of
 // two, which saves a whole per-warp latency (cartpole: 0.445 -> 0.30 ms per launch).  The
 // FP64 build needs 252 registers and 27.6 KB of stage per warp and stays at 8 warps/SM.
-template <class S, int NS, int NC, int DYN, bool STAGED, int PHASE = 0>
+template <class S, int NS, int NC, int DYN, bool STAGED>
 constexpr int iter_min_blocks() {
-  // the stand-alone rollout of the small env models (split iteration, api.cu): its state is
-  // small, 128 registers give 16 warps/SM and the whole 65536-problem batch is one wave
-  if (PHASE == 2 && !STAGED && DYN != DYN_LINDX && NS + NC <= 6) return 4;
   return (sizeof(S) == 4 && STAGED && DYN != DYN_LINDX && NS + NC <= 6) ? 4 : 1;
 }
 
-template <class S, int NS, int NC, int DYN, bool STAGED, bool LOCKSTEP = false, int PHASE = 0,
-          bool SYM = false>
-__global__ void __launch_bounds__(128, iter_min_blocks<S, NS, NC, DYN, STAGED, PHASE>())
+// ROLLOUT_ONLY: the line-search rollout alone, behind the group sweep (api.cu)
+template <class S, int NS, int NC, int DYN, bool STAGED, bool ROLLOUT_ONLY = false, bool SYM = false>
+__global__ void __launch_bounds__(128, iter_min_blocks<S, NS, NC, DYN, STAGED>())
 ilqr_iter_kernel(const __grid_constant__ IterParams<S> p) {
-  using IK = IterKernel<S, NS, NC, DYN, STAGED, LOCKSTEP, SYM>;
+  using IK = IterKernel<S, NS, NC, DYN, STAGED, SYM>;
   if (SYM ? !IK::sym_ok(p) : (p.sym_pair && IK::sym_ok(p))) return;   // the other kernel of the pair runs
   extern __shared__ __align__(128) char smem[];
   const int lane = threadIdx.x & 31;
@@ -1087,8 +1075,8 @@ ilqr_iter_kernel(const __grid_constant__ IterParams<S> p) {
   }
   // padded lanes (tail warp) read the API tensors of the warp's first problem
   const int bsafe = active ? b : b0;
-  if (PHASE != 2) IK::backward_sweep(p, st, b0, bsafe, b, active, lane);
-  if (PHASE != 1 && !p.gains_only) IK::forward_linesearch(p, st, b0, bsafe, b, active, lane);
+  if (!ROLLOUT_ONLY) IK::backward_sweep(p, st, b0, bsafe, b, active, lane);
+  if (!p.gains_only) IK::forward_linesearch(p, st, b0, bsafe, b, active, lane);
 }
 
 // ---------------------------------------------------------------------------
@@ -1101,7 +1089,7 @@ ilqr_iter_kernel(const __grid_constant__ IterParams<S> p) {
 template <class S, int NS, int NC, int DYN, bool STAGED, bool SYM = false>
 __global__ void __launch_bounds__(128)
 ilqr_gains_kernel(const __grid_constant__ IterParams<S> p) {
-  using IK = IterKernel<S, NS, NC, DYN, STAGED, false, SYM>;
+  using IK = IterKernel<S, NS, NC, DYN, STAGED, SYM>;
   if (SYM ? !IK::sym_ok(p) : (p.sym_pair && IK::sym_ok(p))) return;   // the other kernel of the pair runs
   extern __shared__ __align__(128) char smem[];
   const int lane = threadIdx.x & 31;

@@ -15,7 +15,7 @@ namespace dilqr {
 // ---------------------------------------------------------------------------
 static __global__ void trace_verify_kernel(uint32_t* __restrict__ guess, const uint32_t* __restrict__ votes,
                                     int T, int boxed, int solo, DilqrStatus* status,
-                                    int lockstep = 0, DilqrControl* ctrl = nullptr) {
+                                    DilqrControl* ctrl = nullptr) {
   if (ctrl && ctrl->halt) return;   // uniform: whole block leaves
   __shared__ int s_first;
   __shared__ unsigned s_nqp, s_unconv;
@@ -35,7 +35,7 @@ static __global__ void trace_verify_kernel(uint32_t* __restrict__ guess, const u
       const int slot = t * kPnqpMaxIter + it;
       uint32_t v = votes[slot];
       if (!(v & 1u)) v = 0;
-      if (!lockstep && guess[slot] != v) atomicMin(&s_first, i);   // lockstep: votes ARE the trace
+      if (guess[slot] != v) atomicMin(&s_first, i);
     }
     __syncthreads();
     for (int t = threadIdx.x; t < T; t += blockDim.x) {
@@ -94,7 +94,7 @@ struct CommitAux {
   CommitPart* part;         // one record per block
   unsigned int* ticket;     // zero between launches
   DilqrControl* ctrl;       // may be nullptr
-  int lockstep;             // votes ARE the trace (lockstep / group sweep): nothing to compare
+  int votes_are_trace;      // group sweep: the votes ARE the trace, nothing to compare
   int iteration;
 };
 
@@ -115,7 +115,7 @@ __global__ void __launch_bounds__(128) commit_kernel(const __grid_constant__ Ite
     s_unconv = 0;
   }
   __syncthreads();
-  if (traced && !aux.lockstep) {
+  if (traced && !aux.votes_are_trace) {
     // Normalised vote of a slot: if nobody was moving the sweep left the slot right there, so
     // Armijo bits voted under a wrong "moving" guess are void.  Processing order of the sweep
     // is t = T-1 .. 0, it = 0 .. 19.

@@ -109,12 +109,10 @@ void make_problem(Problem& P, const Tensor& x_init, const Tensor& C, const Tenso
     s.u_lower = *u_lower;
     s.u_upper = *u_upper;
   }
-  TORCH_CHECK(dilqr_supported(s.dtype, s.n_state, s.n_ctrl, s.dynamics),
-              "dilqr: no kernel compiled for n_state=", s.n_state, " n_ctrl=", s.n_ctrl,
-              " dynamics=", s.dynamics);
-  if (s.bounds_kind != DILQR_BOUNDS_NONE && !solo && s.n_ctrl > 1 &&
-      s.n_batch <= dilqr_lockstep_capacity(s.dtype, s.n_state, s.n_ctrl, s.dynamics))
-    s.lockstep = 1;
+  const int rc = dilqr_mpc_plan(&s);   // the library chooses how pnqp's decisions are resolved
+  TORCH_CHECK(rc != DILQR_EUNSUPPORTED, "dilqr: no kernel compiled for n_state=", s.n_state,
+              " n_ctrl=", s.n_ctrl, " dynamics=", s.dynamics);
+  check_rc(rc, "dilqr_mpc_plan");
   auto bytes = at::TensorOptions().dtype(at::kByte).device(x_init.device());
   P.ws = at::empty({(int64_t)dilqr_workspace_bytes(&s)}, bytes);
   P.pipe = at::zeros({64 * (1 + max_iters)}, bytes);

@@ -54,7 +54,7 @@ enum {
   DILQR_EALIGN = -3,       /* a pointer is not 16-byte aligned                      */
   DILQR_EWORKSPACE = -4,   /* workspace too small                                   */
   DILQR_ECUDA = -5,        /* kernel launch failed (cudaGetLastError != success)    */
-  DILQR_ELOCKSTEP = -6     /* lockstep requested but the batch is not co-resident   */
+  DILQR_ELOCKSTEP = -6     /* group sweep: the batch does not fit the device at once */
 };
 
 #define DILQR_PNQP_MAX_ITER 20   /* pnqp.py:5  n_iter=20 (lqr_step.py:137)           */
@@ -114,9 +114,6 @@ typedef struct DilqrSolve {
   int32_t C_bcast, c_bcast; /* cost layout (mpc.py:205-219): 0 dense C[T,B,n,n] / c[T,B,n];
                                1 batch-broadcast C[T,n,n] / c[T,n]; 2 C[n,n] / c[n] -- the
                                kernels read the single shared block, nothing is tiled   */
-  int32_t lockstep;         /* iterate: resolve the batch-global pnqp decisions with grid-wide
-                               barriers in a cooperative launch (whole batch resident, see
-                               dilqr_lockstep_capacity) instead of replaying a guessed trace */
   double  linesearch_decay; /* mpc.py:134                                           */
   double  u_lower, u_upper; /* scalar bounds (mpc.py:81-82)                         */
   double  best_cost_eps;    /* mpc.py:142                                           */
@@ -165,11 +162,11 @@ typedef struct DilqrSolve {
   int32_t keep_trace_guess;  /* dilqr_mpc_begin: 1 keeps the pnqp trace guess the previous solve in
                                 this workspace ended with (same shape; steady-state loops) instead
                                 of resetting it to the default                                    */
-  int32_t group_sweep;       /* iterate: run the Riccati / pnqp sweep with the batch-synchronous
-                                thread-group kernel (csrc/group_kernels.cuh): G lanes per problem,
-                                every batch-global pnqp decision a grid barrier -- exact on any batch
-                                up to dilqr_group_sweep_capacity() problems, no trace replay.  Must
-                                be set before dilqr_workspace_bytes (it adds a scratch record)      */
+  int32_t group_sweep;       /* written by dilqr_mpc_plan.  1: iterate runs the Riccati / pnqp sweep
+                                with the batch-synchronous thread-group kernel
+                                (csrc/group_kernels.cuh): G lanes per problem, every batch-global pnqp
+                                decision a grid barrier, no trace replay.  0: one thread per problem,
+                                replaying a guessed trace.  dilqr_workspace_bytes depends on it      */
 } DilqrSolve;
 
 const char* dilqr_version(void);
@@ -177,19 +174,13 @@ const char* dilqr_version(void);
 /* 1 if kernels for this combination are compiled in, else 0. */
 int dilqr_supported(int dtype, int n_state, int n_ctrl, int dynamics);
 
-/* Largest n_batch the lockstep (cooperative) variant of dilqr_mpc_iterate can hold
- * resident on the current device for this shape; 0 if unsupported. */
-int dilqr_lockstep_capacity(int dtype, int n_state, int n_ctrl, int dynamics);
-
-/* Largest n_batch the group sweep handles for this shape on the current device (one
- * phase-B thread per problem in a co-resident cooperative grid); 0: not compiled for it
- * (single-input shapes that fit one thread per problem keep the register-resident sweep). */
-int dilqr_group_sweep_capacity(int dtype, int n_state, int n_ctrl, int dynamics);
-
-/* 1: the shape's sweeps keep a problem in one thread's registers with TMA-staged operands;
- * 0: too large for that (its matrices would live in local memory: use the group sweep);
- * -1: shape not compiled in. */
-int dilqr_shape_staged(int dtype, int n_state, int n_ctrl, int dynamics);
+/* Choose how dilqr_mpc_iterate resolves pnqp's batch-global decisions and write it to
+ * s->group_sweep.  Reads only dtype, n_state, n_ctrl, dynamics, bounds_kind, solo and n_batch;
+ * call it before dilqr_workspace_bytes.  The group sweep runs shapes whose matrices do not fit
+ * one thread's registers, and box-constrained (solo == 0) multi-input batches, wherever the
+ * shape has it and the batch fits the current device at once; everything else replays a
+ * guessed trace.  DILQR_EUNSUPPORTED: the shape is not compiled in. */
+int dilqr_mpc_plan(DilqrSolve* s);
 
 /* Bytes of workspace the dilqr_mpc_* calls need. */
 size_t dilqr_workspace_bytes(const DilqrSolve* s);
@@ -357,11 +348,11 @@ typedef struct DilqrAdjoint {
   int32_t reserved0;
   void *red_out;
   void *df_blk;          /* final: df warp-blocked [T-1][ceil(B/32)][ns][32] for
-                            dilqr_sens_theta_blocked (instead of df)                          */
+                            dilqr_sens_theta_adjoint (instead of df)                          */
 } DilqrAdjoint;
 size_t dilqr_adjoint_workspace_bytes(const DilqrAdjoint* a);
 /* Byte offset, inside the adjoint workspace, of the adjoint solution the final pass keeps:
- * dtau warp-blocked [T][ceil(B/32)][n][32] (input of dilqr_sens_theta_blocked). */
+ * dtau warp-blocked [T][ceil(B/32)][n][32] (input of dilqr_sens_theta_adjoint). */
 size_t dilqr_adjoint_dtau_offset(const DilqrAdjoint* a);
 /* Masked Riccati sweep at tau*: gains and the r-independent blocks.  Needs only C, x, u,
  * bounds, dyn_params, resid and the workspace (not w, g, Lam or the outputs), so it can be
@@ -380,25 +371,22 @@ int dilqr_sens_theta(int dtype, int dynamics, const double* dyn_params, int T, i
                      const void* x, const void* u, const void* K, const void* lam, const void* dx,
                      const void* du, const void* df, void* dtheta, void* stream);
 
-/* Same with every solver-internal operand in the warp-blocked layout it was produced in:
- * Kk (DilqrWsView), lam_blk (dilqr_mpc_gains), dtau_blk (adjoint workspace +
- * dilqr_adjoint_dtau_offset), df_blk (DilqrAdjoint.df_blk). */
-int dilqr_sens_theta_blocked(int dtype, int dynamics, const double* dyn_params, int T, int n_batch,
-                             const void* x, const void* u, const void* Kk, const void* lam_blk,
-                             const void* dtau_blk, const void* df_blk, void* dtheta, void* stream);
-
 /* Same sum in adjoint form (one reverse sweep carrying n_state scalars per problem instead of
  * the n_state x n_theta sensitivity matrix; the second-order tables enter through
- * Lam_packed [T-1][ceil(B/32)][dilqr_lam_pack_size][32] of dilqr_lam_tables).  Pendulum and
- * cartpole.  Replaces the loop of cartpole.py:755-782 / pendulum.py:412-437 contracted with
+ * Lam_packed [T-1][ceil(B/32)][dilqr_lam_pack_size][32] of dilqr_lam_tables), with every
+ * solver-internal operand in the warp-blocked layout it was produced in: Kk (DilqrWsView),
+ * lam_blk (dilqr_mpc_gains), dtau_blk (adjoint workspace + dilqr_adjoint_dtau_offset), df_blk
+ * (DilqrAdjoint.df_blk).  Pendulum and cartpole.  Replaces the loop of cartpole.py:755-782 / pendulum.py:412-437 contracted with
  * dF, df (lqr_step_explicit.py:700-708). */
 int dilqr_sens_theta_adjoint(int dtype, int dynamics, const double* dyn_params, int T, int n_batch,
                              const void* x, const void* u, const void* Kk, const void* lam_blk,
                              const void* dtau_blk, const void* df_blk, const void* Lam_packed,
                              void* dtheta, void* stream);
 
-/* Kernels the most recent dilqr_mpc_iterate enqueued (1: fused sweep + rollout, 2: split) --
- * launch accounting of the host bindings only. */
+/* Kernels the most recent successful dilqr_mpc_iterate enqueued: 1 for the fused sweep +
+ * rollout, 2 when that kernel is enqueued as a symmetric / general pair (one exits at once),
+ * 2 for the group sweep + its rollout, 1 for the group sweep with gains_only -- launch
+ * accounting of the host bindings only. */
 int dilqr_last_iterate_launches(void);
 
 /* The cost plumbing either side of the solve in the imitation-learning loop.

@@ -241,19 +241,3 @@ def test_lqr_step_explicit_entry(dilqr, port, env, dev):
         x0.to(dev), C.to(dev), c.to(dev), None)
     assert torch.equal(a[0], b[0]) and torch.equal(a[1], b[1])
 
-
-@pytest.mark.parametrize("name,T,B,sigma", [("cartpole", 50, 70, 0.05), ("pendulum", 20, 64, 1.0)])
-def test_dtheta_adjoint_form_equals_sensitivity_rollout(dilqr, port, env, dev, name, T, B, sigma):
-    """dtheta by the reverse sweep on an n_state vector (sens_theta_adjoint_kernel) == dtheta by
-    the forward rollout of the n_state x n_theta sensitivity matrix (grad_input, cartpole.py:
-    755-782) contracted with dF, df: same sum, re-associated."""
-    solver = importlib.import_module("differentiable-ilqr_b200._solver")
-    a = _solve_and_grad(dilqr, env, dev, name, T, B, port, True, sigma=sigma)
-    old = solver._SENS_ROLLOUT
-    solver._SENS_ROLLOUT = True
-    try:
-        b = _solve_and_grad(dilqr, env, dev, name, T, B, port, True, sigma=sigma)
-    finally:
-        solver._SENS_ROLLOUT = old
-    assert torch.equal(a[3], b[3]) and torch.equal(a[4], b[4])
-    assert rel(a[2], b[2]) < 1e-12, rel(a[2], b[2])

@@ -922,12 +922,12 @@ def test_module_dynamics_golden(dilqr, dev, name):
         assert rel(got, g["d_%s_%s" % (name, key)]) < gt, key
 
 
-def test_rocket_full_size_group_sweep_properties(dilqr, env, dev):
+def test_rocket_full_size_group_sweep_properties(dilqr, env, dev, monkeypatch):
     """BASELINE config 3 (rocket T=100, B=16384, box +-20, fp64) through the thread-group
-    sweep: the one-thread-per-problem kernels (lockstep barriers) give the same solution and
+    sweep: the one-thread-per-problem kernels (trace replay) give the same solution and
     the same pnqp iteration counts on the same batch; rollouts are dynamics-consistent,
     controls respect the box, best costs never exceed the initial cost."""
-    solver = importlib.import_module("differentiable-ilqr_b200._solver")
+    L = dilqr._lib.lib()
     dtype = torch.float64
     T, B = 100, 16384
     g = torch.Generator().manual_seed(0)
@@ -940,9 +940,10 @@ def test_rocket_full_size_group_sweep_properties(dilqr, env, dev):
     C = torch.diag(q)[None, None].repeat(T, B, 1, 1)
     c = p[None, None].repeat(T, B, 1)
     outs = []
-    for mode in ("auto", "never"):
-        solver.GROUP_SWEEP = mode
-        try:
+    for replay in (False, True):
+        with monkeypatch.context() as mp:
+            if replay:       # leave DilqrSolve.group_sweep at 0: one thread per problem
+                mp.setattr(L, "dilqr_mpc_plan", lambda s: 0)
             m = dilqr.mpc_explicit.MPC(13, 3, T, u_lower=-20.0, u_upper=20.0, lqr_iter=4, verbose=-1,
                                        exit_unconverged=False, detach_unconverged=False,
                                        linesearch_decay=dx.linesearch_decay,
@@ -950,8 +951,6 @@ def test_rocket_full_size_group_sweep_properties(dilqr, env, dev):
                                        n_batch=B)
             with torch.no_grad():
                 x, u, costs = m(x0, dilqr.QuadCost(C, c), dx)
-        finally:
-            solver.GROUP_SWEEP = "auto"
         outs.append((x, u, costs, list(m.last_info.qp_iters), m.last_info.retries))
     (x, u, costs, qp, retries), (x2, u2, costs2, qp2, _) = outs
     assert retries == 0                       # barriers, not a replayed trace
@@ -963,3 +962,43 @@ def test_rocket_full_size_group_sweep_properties(dilqr, env, dev):
     tau = torch.cat((x, u), 2)
     c0 = (0.5 * (x0 * q[:13] * x0).sum(1) + (x0 * p[:13]).sum(1))       # zero controls: cost of ...
     assert torch.isfinite(costs).all() and torch.isfinite(tau).all()
+
+
+@pytest.mark.parametrize("dtype", [0, 1])
+def test_mpc_plan_chooses_the_group_sweep(dilqr, dtype):
+    """dilqr_mpc_plan: the group sweep for shapes too large for one thread per problem (rocket,
+    LinDx 8+4) and for box-constrained batch-global multi-input batches of the others (LinDx
+    4+2), as long as the batch fits the device; trace replay for everything else (cartpole,
+    network dynamics, LinDx 8+4 at B = 2^20).  Planning allocates nothing."""
+    import ctypes
+    lib = dilqr._lib
+    L = lib.lib()
+    R, X = lib.DYN_ROCKET, lib.DYN_LINDX
+    S, N = lib.BOUNDS_SCALAR, lib.BOUNDS_NONE
+    cases = [  # (n_state, n_ctrl, dynamics, bounds_kind, solo, n_batch) -> group_sweep
+        ((13, 3, R, S, 0, 16384), 1), ((13, 3, R, N, 0, 64), 1),
+        ((5, 1, lib.DYN_CARTPOLE, S, 0, 64), 0), ((4, 2, lib.DYN_NN, S, 0, 256), 0),
+        ((8, 4, X, S, 0, 64), 1), ((8, 4, X, N, 0, 64), 1), ((8, 4, X, S, 1, 64), 1),
+        ((4, 2, X, S, 0, 40), 1), ((4, 2, X, N, 0, 40), 0), ((4, 2, X, S, 1, 40), 0),
+        ((8, 4, X, S, 0, 1 << 20), 0),
+    ]
+    for (ns, nc, dyn, bk, solo, B), want in cases:
+        s = lib.DilqrSolve()
+        s.n_state, s.n_ctrl, s.T, s.n_batch, s.dtype, s.dynamics = ns, nc, 10, B, dtype, dyn
+        s.bounds_kind, s.solo, s.group_sweep = bk, solo, 1 - want
+        assert L.dilqr_mpc_plan(ctypes.byref(s)) == 0
+        assert s.group_sweep == want, (ns, nc, dyn, bk, solo, B)
+    s = lib.DilqrSolve()
+    s.n_state, s.n_ctrl, s.T, s.n_batch, s.dtype, s.dynamics = 7, 3, 10, 64, dtype, X
+    assert L.dilqr_mpc_plan(ctypes.byref(s)) == -2
+
+
+def test_group_sweep_launches_are_counted(dilqr, env, port, dev):
+    """A rocket iteration is the group sweep plus its rollout: two kernels."""
+    T, B = 10, 64
+    pdx, x0, C, c, kw = env_problem(port, "rocket", T, B, torch.float64)
+    m = dilqr.mpc_explicit.MPC(13, 3, T, lqr_iter=2, verbose=-1, exit_unconverged=False,
+                               detach_unconverged=False, **kw)
+    with torch.no_grad():
+        m(x0.to(dev), dilqr.QuadCost(C.to(dev), c.to(dev)), env.RocketDx(pdx.params.to(dev)))
+    assert dilqr._lib.lib().dilqr_last_iterate_launches() == 2

@@ -132,6 +132,32 @@ def test_op_equals_module_env(ops, dilqr, port, dev):
 
 
 @pytest.mark.gpu
+def test_op_equals_module_rocket(ops, dilqr, port, dev):
+    """The op plans its solve in the library like the Python binding, so a rocket batch (too
+    large for one thread per problem) takes the group sweep -- two kernels per iteration -- in
+    both, and the forward outputs agree bitwise.  Forward only: the op's registered backward has
+    no rocket kernels."""
+    env = importlib.import_module("differentiable-ilqr_b200.env_dx")
+    lib = importlib.import_module("differentiable-ilqr_b200._lib")
+    T, B = 20, 64
+    pdx, x0, C, c, kw = env_problem(port, "rocket", T, B, torch.float64)
+    theta = pdx.params.to(dev)
+    with torch.no_grad():
+        x, u, costs, du, qp = torch.ops.dilqr.mpc_solve(
+            x0.to(dev), C.to(dev), c.to(dev), None, None, None, theta, lib.DYN_ROCKET, T,
+            pdx.lower, pdx.upper, 4, pdx.mpc_eps, pdx.linesearch_decay, pdx.max_linesearch_iter,
+            5, 1e-4, 0)
+        assert lib.lib().dilqr_last_iterate_launches() == 2
+        m = dilqr.mpc_explicit.MPC(13, 3, T, u_lower=pdx.lower, u_upper=pdx.upper, lqr_iter=4,
+                                   eps=pdx.mpc_eps, linesearch_decay=pdx.linesearch_decay,
+                                   max_linesearch_iter=pdx.max_linesearch_iter, verbose=-1,
+                                   exit_unconverged=False, detach_unconverged=False)
+        x2, u2, costs2 = m(x0.to(dev), dilqr.QuadCost(C.to(dev), c.to(dev)), env.RocketDx(theta))
+    assert torch.equal(x, x2) and torch.equal(u, u2) and torch.equal(costs, costs2)
+    assert [v for v in qp.tolist() if v >= 0] == m.last_info.qp_iters
+
+
+@pytest.mark.gpu
 @pytest.mark.parametrize("boxed", [False, True])
 def test_op_equals_module_lindx(ops, dilqr, dev, boxed):
     lib = importlib.import_module("differentiable-ilqr_b200._lib")

@@ -1,5 +1,5 @@
 """Small end-to-end case for compute-sanitizer (memcheck): staged + tail warps +
-lockstep + factored adjoint + generic adjoint paths."""
+group sweep + trace replay + factored adjoint + generic adjoint paths."""
 import importlib, os, sys
 import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
