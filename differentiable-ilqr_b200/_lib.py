@@ -14,6 +14,7 @@ CSRC = os.path.join(_HERE, "csrc")
 
 F32, F64 = 0, 1
 DYN_LINDX, DYN_PENDULUM, DYN_CARTPOLE, DYN_ROCKET, DYN_NN = 0, 1, 2, 3, 4
+DYN_LINDX_RT = 5        # LinDx through the runtime-dimension kernels (n_state + n_ctrl <= 32)
 GAIN_PLAIN, GAIN_CHOL_REG = 0, 1
 BOUNDS_NONE, BOUNDS_SCALAR, BOUNDS_TENSOR = 0, 1, 2
 PNQP_MAX_ITER = 20
@@ -80,7 +81,7 @@ class DilqrSolve(C.Structure):
 class DilqrKkt(C.Structure):
     _fields_ = [
         ("n_state", C.c_int32), ("n_ctrl", C.c_int32), ("T", C.c_int32),
-        ("n_batch", C.c_int32), ("dtype", C.c_int32), ("reserved", C.c_int32),
+        ("n_batch", C.c_int32), ("dtype", C.c_int32), ("dynamics", C.c_int32),
         ("C", C.c_void_p), ("c", C.c_void_p), ("F", C.c_void_p),
         ("x", C.c_void_p), ("u", C.c_void_p), ("dx", C.c_void_p), ("du", C.c_void_p),
         ("r", C.c_void_p),
@@ -117,6 +118,7 @@ class DilqrWsView(C.Structure):
 SYMBOLS = {
     "dilqr_version": (C.c_char_p, []),
     "dilqr_supported": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int]),
+    "dilqr_lindx_kernels": (C.c_int, [C.c_int, C.c_int, C.c_int]),
     "dilqr_mpc_plan": (C.c_int, [C.POINTER(DilqrSolve)]),
     "dilqr_workspace_bytes": (C.c_size_t, [C.POINTER(DilqrSolve)]),
     "dilqr_mpc_begin": (C.c_int, [C.POINTER(DilqrSolve), C.c_void_p]),

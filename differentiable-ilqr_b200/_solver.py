@@ -165,6 +165,19 @@ def dense_cost(t, T, B, tail_ndim):
     return t.expand(T, B, *t.shape[2:]).contiguous()
 
 
+def lindx_kernels(dtype, n_state, n_ctrl):
+    """The dynamics id whose kernels serve a LinDx problem of this shape (the library's
+    choice: the compiled kernels where they exist, else the runtime-dimension ones)."""
+    kind = _lib.lib().dilqr_lindx_kernels(_DT[dtype], n_state, n_ctrl)
+    if kind == -2:
+        raise _lib.DilqrLibraryError(
+            "LinDx n_state=%d n_ctrl=%d is not supported: the LinDx kernels take at most 32 "
+            "variables (n_state + n_ctrl)" % (n_state, n_ctrl))
+    if kind < 0:
+        _lib.check(kind, "dilqr_lindx_kernels")
+    return kind
+
+
 def _make_problem(x_init, C_, c_, dyn, n_state, n_ctrl, T, u_lower, u_upper, u_zero_I,
                   linesearch_decay, max_linesearch_iter, best_cost_eps, gain_solve,
                   solo, delta_u=None):
@@ -177,7 +190,7 @@ def _make_problem(x_init, C_, c_, dyn, n_state, n_ctrl, T, u_lower, u_upper, u_z
     s = _lib.DilqrSolve()
     s.n_state, s.n_ctrl, s.T, s.n_batch = n_state, n_ctrl, T, B
     s.dtype = _DT[dtype]
-    s.dynamics = dyn.kind
+    s.dynamics = lindx_kernels(dtype, n_state, n_ctrl) if dyn.kind == _lib.DYN_LINDX else dyn.kind
     s.gain_solve = gain_solve
     s.solo = int(solo)   # 0 batch-global, 1 per-problem QP flags, 2 per-problem outer loop too
     s.max_linesearch_iter = max_linesearch_iter
@@ -207,7 +220,7 @@ def _make_problem(x_init, C_, c_, dyn, n_state, n_ctrl, T, u_lower, u_upper, u_z
         s.dyn_aux = _ptr(aux)
         for i, v in enumerate(dyn.ai):
             s.dyn_ai[i] = int(v)
-    if dyn.kind == _lib.DYN_LINDX:
+    if dyn.kind in (_lib.DYN_LINDX, _lib.DYN_LINDX_RT):
         Fd = dev(dyn.F, "F")
         fd = dev(dyn.f, "f") if (dyn.f is not None and dyn.f.nelement() > 0) else None
         s.F, s.f = _ptr(Fd), _ptr(fd)
@@ -468,6 +481,7 @@ def kkt_grads(C_, c_, F, x, u, dx, du, r, n_state, n_ctrl, want_df=True, want_dF
     dtype, dev = x.dtype, x.device
     k = _lib.DilqrKkt()
     k.n_state, k.n_ctrl, k.T, k.n_batch, k.dtype = n_state, n_ctrl, T, B, _DT[dtype]
+    k.dynamics = lindx_kernels(dtype, n_state, n_ctrl)
     ten = [_contig(t.detach()) for t in (C_, c_, F, x, u, dx, du, r)]
     k.C, k.c, k.F, k.x, k.u, k.dx, k.du, k.r = [_ptr(t) for t in ten]
     n = n_state + n_ctrl

@@ -13,6 +13,7 @@
 #include "dilqr_backward.cuh"
 #include "adjoint_kernels.cuh"
 #include "group_kernels.cuh"
+#include "rt_kernels.cuh"
 
 namespace dilqr {
 
@@ -236,7 +237,8 @@ static IterParams<Scalar> make_params(const DilqrSolve* s, int role = 1) {
 static int check(const DilqrSolve* s, bool need_ws) {
   if (!s || s->n_state <= 0 || s->n_ctrl <= 0 || s->T <= 0 || s->n_batch <= 0) return DILQR_EINVAL;
   if (!s->x_init || !s->C || !s->c) return DILQR_EINVAL;
-  if (s->dynamics == DILQR_DYN_LINDX && s->T > 1 && !s->F) return DILQR_EINVAL;
+  if ((s->dynamics == DILQR_DYN_LINDX || s->dynamics == DILQR_DYN_LINDX_RT) && s->T > 1 && !s->F)
+    return DILQR_EINVAL;
   if (s->dynamics == DILQR_DYN_NN &&
       (!s->dyn_aux || s->dyn_ai[0] < 1 || (s->dyn_ai[0] & 0xffff) < 1 ||
        ((s->dyn_ai[0] >> 16) > 0 && (s->dyn_ai[0] & 0xffff) > 128) ||   /* two layers: H1 <= 128 */
@@ -273,6 +275,29 @@ struct Geometry {
   static size_t smem(int wpb) { return STAGED ? IK::smem_per_warp() * wpb : 0; }
 };
 
+// Workspace state a begin kernel starts from.  `packs_C`: the kernels keep a packed copy of C
+// (ilqr_kernels.cuh); without it the packed-C state word stays 0 (no copy).
+static void begin_state(const DilqrSolve* s, const IterParams<Scalar>& p, bool packs_C,
+                        cudaStream_t st) {
+  // default pnqp trace guess: at t = T-1 nothing moves (x_init=None is the exact
+  // minimiser); at t < T-1 one Newton step then convergence (SURVEY a-5).
+  const WsLayout w = ws_layout(s, sizeof(Scalar));
+  static_assert(kPnqpMaxIter == DILQR_PNQP_MAX_ITER, "trace width");
+  if (!s->keep_trace_guess) {
+    cudaMemsetAsync(p.guess, 0, (size_t)p.T * kPnqpMaxIter * sizeof(uint32_t), st);
+    if (p.T > 1)
+      cudaMemset2DAsync(p.guess, kPnqpMaxIter * sizeof(uint32_t), 3, 1, p.T - 1, st);
+  }
+  // 1: begin packs the upper triangle of C for the sweeps (ilqr_kernels.cuh), 0: dense
+  const bool pack = packs_C && !p.C_bcast && !(p.gains_only && p.x_cur);
+  cudaMemsetAsync(p.cpk_state, 0, sizeof(uint32_t), st);
+  if (pack) cudaMemsetAsync(p.cpk_state, 1, 1, st);   // little-endian: word value 1
+  // 3: broadcast C, symmetry of the shared block(s) to be verified by begin
+  if (packs_C && p.C_bcast && !(p.gains_only && p.x_cur)) cudaMemsetAsync(p.cpk_state, 3, 1, st);
+  // ticket counter of the one-launch commit (returns to zero after every commit)
+  cudaMemsetAsync(static_cast<char*>(s->workspace) + w.commit_ticket, 0, sizeof(uint32_t), st);
+}
+
 template <int NS, int NC, int DYN>
 static int launch_begin(const DilqrSolve* s, cudaStream_t st) {
   using S = Scalar;
@@ -285,25 +310,7 @@ static int launch_begin(const DilqrSolve* s, cudaStream_t st) {
   auto kern = ilqr_begin_kernel<S, NS, NC, DYN, G::STAGED>;
   if (smem > 48 * 1024)
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  // default pnqp trace guess: at t = T-1 nothing moves (x_init=None is the exact
-  // minimiser); at t < T-1 one Newton step then convergence (SURVEY a-5).
-  const WsLayout w = ws_layout(s, sizeof(S));
-  static_assert(kPnqpMaxIter == DILQR_PNQP_MAX_ITER, "trace width");
-  if (!s->keep_trace_guess) {
-    cudaMemsetAsync(p.guess, 0, (size_t)p.T * kPnqpMaxIter * sizeof(uint32_t), st);
-    if (p.T > 1)
-      cudaMemset2DAsync(p.guess, kPnqpMaxIter * sizeof(uint32_t), 3, 1, p.T - 1, st);
-  }
-  (void)w;
-  {  // 1: begin packs the upper triangle of C for the sweeps (ilqr_kernels.cuh), 0: dense
-    const bool pack = !p.C_bcast && !(p.gains_only && p.x_cur);
-    cudaMemsetAsync(p.cpk_state, 0, sizeof(uint32_t), st);
-    if (pack) cudaMemsetAsync(p.cpk_state, 1, 1, st);   // little-endian: word value 1
-    // 3: broadcast C, symmetry of the shared block(s) to be verified by begin
-    if (p.C_bcast && !(p.gains_only && p.x_cur)) cudaMemsetAsync(p.cpk_state, 3, 1, st);
-    // ticket counter of the one-launch commit (returns to zero after every commit)
-    cudaMemsetAsync(static_cast<char*>(s->workspace) + w.commit_ticket, 0, sizeof(uint32_t), st);
-  }
+  begin_state(s, p, true, st);
   kern<<<blocks, wpb * kWarp, smem, st>>>(p);
   return cudaGetLastError() == cudaSuccess ? DILQR_OK : DILQR_ECUDA;
 }
@@ -494,6 +501,7 @@ static int launch_commit(const DilqrSolve* s, cudaStream_t st) {
   aux.ctrl = s->control;
   aux.votes_are_trace = p.votes_are_trace;
   aux.iteration = s->iteration;
+  aux.nc = s->n_ctrl;
   commit_kernel<S, NS + NC, NC><<<(p.B + 127) / 128, 128, 0, st>>>(p, aux);
   return cudaGetLastError() == cudaSuccess ? DILQR_OK : DILQR_ECUDA;
 }
@@ -503,7 +511,7 @@ static int launch_finish(const DilqrSolve* s, cudaStream_t st) {
   using S = Scalar;
   IterParams<S> p = make_params(s);
   dim3 grid((p.B + 127) / 128, p.T);
-  finish_kernel<S, NS, NC><<<grid, 128, 0, st>>>(p);
+  finish_kernel<S, NS, NC><<<grid, 128, 0, st>>>(p, s->n_state, s->n_ctrl);
   return cudaGetLastError() == cudaSuccess ? DILQR_OK : DILQR_ECUDA;
 }
 
@@ -517,7 +525,42 @@ static int launch_kkt(const DilqrKkt* k, cudaStream_t st) {
 // ------------------------------------------------------------------ dispatch
 enum Op { OP_BEGIN, OP_ITERATE, OP_COMMIT, OP_FINISH };
 
+#if DILQR_GROUP == 0
+// DILQR_DYN_LINDX_RT (rt_kernels.cuh): one warp per problem, the warp's shared-memory slice
+// sized for (n_state, n_ctrl); commit and finish are the compiled family's kernels with
+// runtime dimensions.
+static int rt_launch(const DilqrSolve* s, Op op, cudaStream_t st) {
+  using S = Scalar;
+  const int ns = s->n_state, nc = s->n_ctrl;
+  if (!rt_shape_ok(ns, nc)) return DILQR_EUNSUPPORTED;
+  if (op == OP_COMMIT) return launch_commit<0, 0>(s, st);
+  if (op == OP_FINISH) return launch_finish<0, 0>(s, st);
+  IterParams<S> p = make_params(s, op == OP_BEGIN ? 0 : 1);
+  const size_t per = RtSmem<S>::bytes(ns, nc);
+  int wpb = (int)((96 * 1024) / per);   // <= 96 KB a block: two blocks fit one SM
+  if (wpb > 4) wpb = 4;
+  if (wpb < 1) wpb = 1;
+  const int blocks = (p.B + wpb - 1) / wpb;
+  const size_t smem = per * wpb;
+  auto kern = op == OP_BEGIN ? rt_begin_kernel<S> : rt_iter_kernel<S>;
+  if (smem > 48 * 1024)
+    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (op == OP_BEGIN) {
+    begin_state(s, p, false, st);
+  } else {
+    if (p.bounds_kind && !p.solo)
+      cudaMemsetAsync(p.votes, 0, (size_t)p.T * kPnqpMaxIter * sizeof(uint32_t), st);
+    g_iterate_launches = 1;
+  }
+  kern<<<blocks, wpb * kWarp, smem, st>>>(p, ns, nc);
+  return cudaGetLastError() == cudaSuccess ? DILQR_OK : DILQR_ECUDA;
+}
+#endif
+
 static int dispatch(const DilqrSolve* s, Op op, cudaStream_t st) {
+#if DILQR_GROUP == 0
+  if (s->dynamics == DILQR_DYN_LINDX_RT) return rt_launch(s, op, st);
+#endif
 #define X(NS_, NC_, DYN_)                                                            \
   if (s->n_state == NS_ && s->n_ctrl == NC_ && s->dynamics == DYN_) {                \
     switch (op) {                                                                    \
@@ -533,6 +576,13 @@ static int dispatch(const DilqrSolve* s, Op op, cudaStream_t st) {
 }
 
 int DILQR_SUFFIX(mpc_plan)(DilqrSolve* s) {
+#if DILQR_GROUP == 0
+  if (s->dynamics == DILQR_DYN_LINDX_RT) {   // replays the pnqp trace; never asks the device
+    if (!rt_shape_ok(s->n_state, s->n_ctrl)) return DILQR_EUNSUPPORTED;
+    s->group_sweep = 0;
+    return DILQR_OK;
+  }
+#endif
 #define X(NS_, NC_, DYN_) \
   if (s->n_state == NS_ && s->n_ctrl == NC_ && s->dynamics == DYN_) return plan<NS_, NC_, DYN_>(s);
   DILQR_CONFIGS(X)
@@ -541,6 +591,9 @@ int DILQR_SUFFIX(mpc_plan)(DilqrSolve* s) {
 }
 
 int DILQR_SUFFIX(supported)(int n_state, int n_ctrl, int dynamics) {
+#if DILQR_GROUP == 0
+  if (dynamics == DILQR_DYN_LINDX_RT) return rt_shape_ok(n_state, n_ctrl) ? 1 : 0;
+#endif
 #define X(NS_, NC_, DYN_) \
   if (n_state == NS_ && n_ctrl == NC_ && dynamics == DYN_) return 1;
   DILQR_CONFIGS(X)
@@ -601,8 +654,17 @@ int DILQR_SUFFIX(mpc_gains)(const DilqrSolve* s, void* lam_blk, void* stream) {
 int DILQR_SUFFIX(kkt_grads)(const DilqrKkt* k, void* stream) {
   if (!k || !k->C || !k->c || !k->x || !k->u || !k->dx || !k->du || !k->r) return DILQR_EINVAL;
   if (k->T > 1 && !k->F) return DILQR_EINVAL;
-#define X(NS_, NC_, DYN_)                                            \
-  if (DYN_ == DYN_LINDX && k->n_state == NS_ && k->n_ctrl == NC_)    \
+#if DILQR_GROUP == 0
+  if (k->dynamics == DILQR_DYN_LINDX_RT) {
+    if (k->T <= 0 || k->n_batch <= 0) return DILQR_EINVAL;
+    if (!rt_shape_ok(k->n_state, k->n_ctrl)) return DILQR_EUNSUPPORTED;
+    rt_kkt_kernel<Scalar><<<(k->n_batch + 3) / 4, 128, 0, static_cast<cudaStream_t>(stream)>>>(*k);
+    return cudaGetLastError() == cudaSuccess ? DILQR_OK : DILQR_ECUDA;
+  }
+#endif
+#define X(NS_, NC_, DYN_)                                                                 \
+  if (DYN_ == DYN_LINDX && k->dynamics == DILQR_DYN_LINDX && k->n_state == NS_ &&          \
+      k->n_ctrl == NC_)                                                                    \
     return launch_kkt<NS_, NC_>(k, static_cast<cudaStream_t>(stream));
   DILQR_CONFIGS(X)
 #undef X

@@ -82,6 +82,13 @@ int dilqr_supported(int dtype, int ns, int nc, int dyn) {
   return 0;
 }
 
+int dilqr_lindx_kernels(int dtype, int ns, int nc) {
+  if ((dtype != DILQR_F32 && dtype != DILQR_F64) || ns <= 0 || nc <= 0) return DILQR_EINVAL;
+  if (dilqr_supported(dtype, ns, nc, DILQR_DYN_LINDX)) return DILQR_DYN_LINDX;
+  if (dilqr_supported(dtype, ns, nc, DILQR_DYN_LINDX_RT)) return DILQR_DYN_LINDX_RT;
+  return DILQR_EUNSUPPORTED;
+}
+
 int dilqr_mpc_plan(DilqrSolve* s) {
   if (!s) return DILQR_EINVAL;
   BY_DTYPE_GROUPS(s->dtype, mpc_plan, s);
@@ -138,6 +145,7 @@ size_t dilqr_adjoint_dtau_offset(const DilqrAdjoint* a) {
 }
 int dilqr_kkt_grads(const DilqrKkt* k, void* st) {
   if (!k) return DILQR_EINVAL;
+  if (k->dynamics != DILQR_DYN_LINDX && k->dynamics != DILQR_DYN_LINDX_RT) return DILQR_EINVAL;
   BY_DTYPE_GROUPS(k->dtype, kkt_grads, k, st);
 }
 int dilqr_linearize(int dtype, int dyn, const double* dp, int T, int B, const void* x,

@@ -96,11 +96,13 @@ struct CommitAux {
   DilqrControl* ctrl;       // may be nullptr
   int votes_are_trace;      // group sweep: the votes ARE the trace, nothing to compare
   int iteration;
+  int nc;                   // n_ctrl of the runtime-dimension family (commit_kernel<S, 0, 0>)
 };
 
 template <class S, int N, int NCc>
 __global__ void __launch_bounds__(128) commit_kernel(const __grid_constant__ IterParams<S> p,
                                                      const CommitAux aux) {
+  const int nc = NCc ? NCc : aux.nc;
   DilqrStatus* status = reinterpret_cast<DilqrStatus*>(p.status);
   if (p.halt && *reinterpret_cast<const volatile uint32_t*>(p.halt)) return;   // uniform
   __shared__ int s_first;
@@ -146,7 +148,7 @@ __global__ void __launch_bounds__(128) commit_kernel(const __grid_constant__ Ite
     const bool frozen = (state >> 30) & 1;
     int nni = (state >> 8) & 0x3fffff;
     S acc = S(0);
-    for (int k = 0; k < p.T * NCc; ++k) acc = acc + p.dusq[(size_t)k * p.B + b];
+    for (int k = 0; k < p.T * nc; ++k) acc = acc + p.dusq[(size_t)k * p.B + b];
     const S dn = sqrtS<S>(acc);
     const S cn = p.cost_new[b];
     bool take = false, stop = frozen;
@@ -176,7 +178,7 @@ __global__ void __launch_bounds__(128) commit_kernel(const __grid_constant__ Ite
     // full_du_norm[b]: norm of row b of the [T,nc,B] squares re-read as [B, T*nc]
     // (lqr_step.py:243-245, see the note in forward_linesearch)
     {
-      const int row = p.T * NCc;
+      const int row = p.T * nc;
       const S* src = p.dusq + (size_t)b * row;
       S acc = S(0);
       int k = 0;
@@ -332,10 +334,12 @@ __global__ void __launch_bounds__(128) commit_kernel(const __grid_constant__ Ite
 // One thread per (t, b); workspace reads are coalesced, the AoS writes are
 // contiguous per warp (consecutive b).
 // ---------------------------------------------------------------------------
-template <class S, int NS, int NC>
-__global__ void finish_kernel(const __grid_constant__ IterParams<S> p) {
-  constexpr int N = NS + NC;
-  constexpr int NK = NC * NS + NC;
+// NS_ = NC_ = 0: the runtime-dimension family (rt_kernels.cuh), shape given as ns_rt, nc_rt
+template <class S, int NS_, int NC_>
+__global__ void finish_kernel(const __grid_constant__ IterParams<S> p, int ns_rt, int nc_rt) {
+  const int NS = NS_ ? NS_ : ns_rt, NC = NC_ ? NC_ : nc_rt;
+  const int N = NS + NC;
+  const int NK = NC * NS + NC;
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   const int t = blockIdx.y;
   if (b >= p.B) return;

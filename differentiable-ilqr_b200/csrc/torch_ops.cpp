@@ -78,6 +78,12 @@ void make_problem(Problem& P, const Tensor& x_init, const Tensor& C, const Tenso
   s.T = (int)T;
   s.dtype = dtype_of(x_init);
   s.dynamics = (int)dynamics;
+  if (dynamics == DILQR_DYN_LINDX) {   // the library picks compiled or runtime-dimension kernels
+    s.dynamics = dilqr_lindx_kernels(s.dtype, s.n_state, s.n_ctrl);
+    TORCH_CHECK(s.dynamics != DILQR_EUNSUPPORTED, "dilqr: LinDx n_state=", s.n_state, " n_ctrl=",
+                s.n_ctrl, " is not supported: at most 32 variables (n_state + n_ctrl)");
+    check_rc(s.dynamics < 0 ? s.dynamics : 0, "dilqr_lindx_kernels");
+  }
   s.gain_solve = DILQR_GAIN_PLAIN;
   s.solo = (int)solo;
   s.max_linesearch_iter = (int)max_ls;
@@ -237,6 +243,7 @@ std::tuple<Tensor, Tensor, Tensor, Tensor, Tensor> lqr_kkt_backward(
   DilqrKkt k;
   std::memset(&k, 0, sizeof(k));
   k.n_state = (int)ns; k.n_ctrl = (int)nc; k.T = (int)T; k.n_batch = (int)B; k.dtype = dtype_of(x);
+  k.dynamics = s.dynamics;   // the kernels make_problem chose for this shape (dilqr_lindx_kernels)
   Tensor Fc = F.detach().contiguous(), xc = x.detach().contiguous(), uc = u.detach().contiguous();
   k.C = Cd.data_ptr(); k.c = cd.data_ptr(); k.F = Fc.data_ptr(); k.x = xc.data_ptr(); k.u = uc.data_ptr();
   k.dx = dx.data_ptr(); k.du = du.data_ptr(); k.r = r.data_ptr();

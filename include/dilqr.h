@@ -36,7 +36,13 @@ enum {
   DILQR_DYN_PENDULUM = 1, /* env_dx/pendulum.py:60-95, Jacobian 444-475             */
   DILQR_DYN_CARTPOLE = 2, /* env_dx/cartpole.py:64-97, Jacobian 790-839             */
   DILQR_DYN_ROCKET   = 3, /* env_dx/rocket.py:82-164,  Jacobian 324-426             */
-  DILQR_DYN_NN       = 4  /* dynamics.py:15-130 NNDynamics, one hidden layer (dyn_aux)  */
+  DILQR_DYN_NN       = 4, /* dynamics.py:15-130 NNDynamics, one hidden layer (dyn_aux)  */
+  DILQR_DYN_LINDX_RT = 5  /* LinDx through the runtime-dimension kernels (rt_kernels.cuh):
+                             any n_state >= 1, n_ctrl >= 1 with n_state + n_ctrl <= 32, both
+                             dtypes; same problem struct and entry points as DILQR_DYN_LINDX.
+                             Replays the pnqp trace (never the group sweep); dilqr_mpc_gains
+                             and the DiLQR backward calls do not serve it.  Select it with
+                             dilqr_lindx_kernels.                                         */
 };
 
 /* How unconstrained multi-input gains are solved (the reference copies differ). */
@@ -171,15 +177,24 @@ typedef struct DilqrSolve {
 
 const char* dilqr_version(void);
 
-/* 1 if kernels for this combination are compiled in, else 0. */
+/* 1 if kernels for this combination are compiled in, else 0.  DILQR_DYN_LINDX_RT: 1 for every
+ * shape of its range, compiled-in shapes included. */
 int dilqr_supported(int dtype, int n_state, int n_ctrl, int dynamics);
+
+/* Which kernels serve a LinDx problem of this shape: DILQR_DYN_LINDX if the shape is compiled in,
+ * else DILQR_DYN_LINDX_RT if n_state + n_ctrl <= 32, else DILQR_EUNSUPPORTED; DILQR_EINVAL for a
+ * bad dtype or a non-positive dimension.  Put the result into DilqrSolve.dynamics /
+ * DilqrKkt.dynamics. */
+int dilqr_lindx_kernels(int dtype, int n_state, int n_ctrl);
 
 /* Choose how dilqr_mpc_iterate resolves pnqp's batch-global decisions and write it to
  * s->group_sweep.  Reads only dtype, n_state, n_ctrl, dynamics, bounds_kind, solo and n_batch;
  * call it before dilqr_workspace_bytes.  The group sweep runs shapes whose matrices do not fit
  * one thread's registers, and box-constrained (solo == 0) multi-input batches, wherever the
  * shape has it and the batch fits the current device at once; everything else replays a
- * guessed trace.  DILQR_EUNSUPPORTED: the shape is not compiled in. */
+ * guessed trace.  DILQR_DYN_LINDX_RT always replays (group_sweep = 0) and never queries the
+ * device.  DILQR_EUNSUPPORTED: the shape is not compiled in (DILQR_DYN_LINDX_RT: out of its
+ * range). */
 int dilqr_mpc_plan(DilqrSolve* s);
 
 /* Bytes of workspace the dilqr_mpc_* calls need. */
@@ -267,7 +282,9 @@ int dilqr_rollout(int dtype, int dynamics, const double* dyn_params, int T,
  *   dC[T,B,n,n] dc[T,B,n] dF[T-1,B,ns,n] df[T-1,B,ns] dx_init[B,ns].
  * Any output pointer may be NULL to skip it. */
 typedef struct DilqrKkt {
-  int32_t n_state, n_ctrl, T, n_batch, dtype, reserved;
+  int32_t n_state, n_ctrl, T, n_batch, dtype;
+  int32_t dynamics;             /* DILQR_DYN_LINDX (compiled shapes) or DILQR_DYN_LINDX_RT
+                                   (dilqr_lindx_kernels); other values: DILQR_EINVAL */
   const void *C, *c, *F;        /* problem data                               */
   const void *x, *u;            /* solution  x*[T,B,ns], u*[T,B,nc]           */
   const void *dx, *du;          /* adjoint solution                           */
