@@ -15,6 +15,7 @@ CSRC = os.path.join(_HERE, "csrc")
 F32, F64 = 0, 1
 DYN_LINDX, DYN_PENDULUM, DYN_CARTPOLE, DYN_ROCKET, DYN_NN = 0, 1, 2, 3, 4
 DYN_LINDX_RT = 5        # LinDx through the runtime-dimension kernels (n_state + n_ctrl <= 32)
+DYN_NN_RT = 6           # NNDynamics through the runtime-dimension kernels (n_state + n_ctrl <= 32)
 GAIN_PLAIN, GAIN_CHOL_REG = 0, 1
 BOUNDS_NONE, BOUNDS_SCALAR, BOUNDS_TENSOR = 0, 1, 2
 PNQP_MAX_ITER = 20
@@ -119,6 +120,7 @@ SYMBOLS = {
     "dilqr_version": (C.c_char_p, []),
     "dilqr_supported": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int]),
     "dilqr_lindx_kernels": (C.c_int, [C.c_int, C.c_int, C.c_int]),
+    "dilqr_nn_kernels": (C.c_int, [C.c_int, C.c_int, C.c_int]),
     "dilqr_mpc_plan": (C.c_int, [C.POINTER(DilqrSolve)]),
     "dilqr_workspace_bytes": (C.c_size_t, [C.POINTER(DilqrSolve)]),
     "dilqr_mpc_begin": (C.c_int, [C.POINTER(DilqrSolve), C.c_void_p]),

@@ -48,7 +48,7 @@ class DynSpec:
         self.params = list(params) if params is not None else []
         self.F = F
         self.f = f
-        self.aux = aux      # DYN_NN: packed weight buffer (device tensor)
+        self.aux = aux      # DYN_NN / DYN_NN_RT: packed weight buffer (device tensor)
         self.ai = list(ai) if ai is not None else []
 
 
@@ -178,6 +178,19 @@ def lindx_kernels(dtype, n_state, n_ctrl):
     return kind
 
 
+def nn_kernels(dtype, n_state, n_ctrl):
+    """The dynamics id whose kernels serve a network (NNDynamics) problem of this shape: the
+    compiled kernels where they exist, else the runtime-dimension ones."""
+    kind = _lib.lib().dilqr_nn_kernels(_DT[dtype], n_state, n_ctrl)
+    if kind == -2:
+        raise _lib.DilqrLibraryError(
+            "NNDynamics n_state=%d n_ctrl=%d is not supported: the network kernels take at most "
+            "32 variables (n_state + n_ctrl)" % (n_state, n_ctrl))
+    if kind < 0:
+        _lib.check(kind, "dilqr_nn_kernels")
+    return kind
+
+
 def _make_problem(x_init, C_, c_, dyn, n_state, n_ctrl, T, u_lower, u_upper, u_zero_I,
                   linesearch_decay, max_linesearch_iter, best_cost_eps, gain_solve,
                   solo, delta_u=None):
@@ -190,7 +203,12 @@ def _make_problem(x_init, C_, c_, dyn, n_state, n_ctrl, T, u_lower, u_upper, u_z
     s = _lib.DilqrSolve()
     s.n_state, s.n_ctrl, s.T, s.n_batch = n_state, n_ctrl, T, B
     s.dtype = _DT[dtype]
-    s.dynamics = lindx_kernels(dtype, n_state, n_ctrl) if dyn.kind == _lib.DYN_LINDX else dyn.kind
+    if dyn.kind == _lib.DYN_LINDX:
+        s.dynamics = lindx_kernels(dtype, n_state, n_ctrl)
+    elif dyn.kind == _lib.DYN_NN:
+        s.dynamics = nn_kernels(dtype, n_state, n_ctrl)
+    else:   # an explicit id, e.g. a runtime family forced on a compiled shape
+        s.dynamics = dyn.kind
     s.gain_solve = gain_solve
     s.solo = int(solo)   # 0 batch-global, 1 per-problem QP flags, 2 per-problem outer loop too
     s.max_linesearch_iter = max_linesearch_iter
@@ -215,7 +233,7 @@ def _make_problem(x_init, C_, c_, dyn, n_state, n_ctrl, T, u_lower, u_upper, u_z
     s.c_bcast, cd = cost_layout(c_.to(dtype), T, B, 1)
     keep.extend((Cd, cd))
     s.x_init, s.C, s.c = _ptr(xi), _ptr(Cd), _ptr(cd)
-    if dyn.kind == _lib.DYN_NN:
+    if dyn.kind in (_lib.DYN_NN, _lib.DYN_NN_RT):
         aux = dev(dyn.aux, "network weights")
         s.dyn_aux = _ptr(aux)
         for i, v in enumerate(dyn.ai):

@@ -239,7 +239,7 @@ static int check(const DilqrSolve* s, bool need_ws) {
   if (!s->x_init || !s->C || !s->c) return DILQR_EINVAL;
   if ((s->dynamics == DILQR_DYN_LINDX || s->dynamics == DILQR_DYN_LINDX_RT) && s->T > 1 && !s->F)
     return DILQR_EINVAL;
-  if (s->dynamics == DILQR_DYN_NN &&
+  if ((s->dynamics == DILQR_DYN_NN || s->dynamics == DILQR_DYN_NN_RT) &&
       (!s->dyn_aux || s->dyn_ai[0] < 1 || (s->dyn_ai[0] & 0xffff) < 1 ||
        ((s->dyn_ai[0] >> 16) > 0 && (s->dyn_ai[0] & 0xffff) > 128) ||   /* two layers: H1 <= 128 */
        s->dyn_ai[1] < 0 || s->dyn_ai[1] > 1 ||
@@ -526,9 +526,13 @@ static int launch_kkt(const DilqrKkt* k, cudaStream_t st) {
 enum Op { OP_BEGIN, OP_ITERATE, OP_COMMIT, OP_FINISH };
 
 #if DILQR_GROUP == 0
-// DILQR_DYN_LINDX_RT (rt_kernels.cuh): one warp per problem, the warp's shared-memory slice
-// sized for (n_state, n_ctrl); commit and finish are the compiled family's kernels with
-// runtime dimensions.
+// DILQR_DYN_LINDX_RT / DILQR_DYN_NN_RT (rt_kernels.cuh): one warp per problem, the warp's
+// shared-memory slice sized for (n_state, n_ctrl) and, for a network, its hidden widths; commit
+// and finish are the compiled family's kernels with runtime dimensions.
+static bool rt_dynamics(int dynamics) {
+  return dynamics == DILQR_DYN_LINDX_RT || dynamics == DILQR_DYN_NN_RT;
+}
+
 static int rt_launch(const DilqrSolve* s, Op op, cudaStream_t st) {
   using S = Scalar;
   const int ns = s->n_state, nc = s->n_ctrl;
@@ -536,13 +540,15 @@ static int rt_launch(const DilqrSolve* s, Op op, cudaStream_t st) {
   if (op == OP_COMMIT) return launch_commit<0, 0>(s, st);
   if (op == OP_FINISH) return launch_finish<0, 0>(s, st);
   IterParams<S> p = make_params(s, op == OP_BEGIN ? 0 : 1);
-  const size_t per = RtSmem<S>::bytes(ns, nc);
+  const bool nn = s->dynamics == DILQR_DYN_NN_RT;
+  const size_t per = nn ? rt_nn_slice_bytes<S>(ns, nc, s->dyn_ai[0]) : RtSmem<S>::bytes(ns, nc);
   int wpb = (int)((96 * 1024) / per);   // <= 96 KB a block: two blocks fit one SM
   if (wpb > 4) wpb = 4;
   if (wpb < 1) wpb = 1;
   const int blocks = (p.B + wpb - 1) / wpb;
   const size_t smem = per * wpb;
-  auto kern = op == OP_BEGIN ? rt_begin_kernel<S> : rt_iter_kernel<S>;
+  auto kern = op == OP_BEGIN ? (nn ? rt_nn_begin_kernel<S> : rt_begin_kernel<S>)
+                             : (nn ? rt_nn_iter_kernel<S> : rt_iter_kernel<S>);
   if (smem > 48 * 1024)
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (op == OP_BEGIN) {
@@ -559,7 +565,7 @@ static int rt_launch(const DilqrSolve* s, Op op, cudaStream_t st) {
 
 static int dispatch(const DilqrSolve* s, Op op, cudaStream_t st) {
 #if DILQR_GROUP == 0
-  if (s->dynamics == DILQR_DYN_LINDX_RT) return rt_launch(s, op, st);
+  if (rt_dynamics(s->dynamics)) return rt_launch(s, op, st);
 #endif
 #define X(NS_, NC_, DYN_)                                                            \
   if (s->n_state == NS_ && s->n_ctrl == NC_ && s->dynamics == DYN_) {                \
@@ -577,7 +583,7 @@ static int dispatch(const DilqrSolve* s, Op op, cudaStream_t st) {
 
 int DILQR_SUFFIX(mpc_plan)(DilqrSolve* s) {
 #if DILQR_GROUP == 0
-  if (s->dynamics == DILQR_DYN_LINDX_RT) {   // replays the pnqp trace; never asks the device
+  if (rt_dynamics(s->dynamics)) {   // replays the pnqp trace; never asks the device
     if (!rt_shape_ok(s->n_state, s->n_ctrl)) return DILQR_EUNSUPPORTED;
     s->group_sweep = 0;
     return DILQR_OK;
@@ -592,7 +598,7 @@ int DILQR_SUFFIX(mpc_plan)(DilqrSolve* s) {
 
 int DILQR_SUFFIX(supported)(int n_state, int n_ctrl, int dynamics) {
 #if DILQR_GROUP == 0
-  if (dynamics == DILQR_DYN_LINDX_RT) return rt_shape_ok(n_state, n_ctrl) ? 1 : 0;
+  if (rt_dynamics(dynamics)) return rt_shape_ok(n_state, n_ctrl) ? 1 : 0;
 #endif
 #define X(NS_, NC_, DYN_) \
   if (n_state == NS_ && n_ctrl == NC_ && dynamics == DYN_) return 1;

@@ -82,11 +82,20 @@ int dilqr_supported(int dtype, int ns, int nc, int dyn) {
   return 0;
 }
 
-int dilqr_lindx_kernels(int dtype, int ns, int nc) {
+// the compiled kernels of a shape where they exist, else the runtime-dimension family
+static int kernels_for(int dtype, int ns, int nc, int compiled, int runtime) {
   if ((dtype != DILQR_F32 && dtype != DILQR_F64) || ns <= 0 || nc <= 0) return DILQR_EINVAL;
-  if (dilqr_supported(dtype, ns, nc, DILQR_DYN_LINDX)) return DILQR_DYN_LINDX;
-  if (dilqr_supported(dtype, ns, nc, DILQR_DYN_LINDX_RT)) return DILQR_DYN_LINDX_RT;
+  if (dilqr_supported(dtype, ns, nc, compiled)) return compiled;
+  if (dilqr_supported(dtype, ns, nc, runtime)) return runtime;
   return DILQR_EUNSUPPORTED;
+}
+
+int dilqr_lindx_kernels(int dtype, int ns, int nc) {
+  return kernels_for(dtype, ns, nc, DILQR_DYN_LINDX, DILQR_DYN_LINDX_RT);
+}
+
+int dilqr_nn_kernels(int dtype, int ns, int nc) {
+  return kernels_for(dtype, ns, nc, DILQR_DYN_NN, DILQR_DYN_NN_RT);
 }
 
 int dilqr_mpc_plan(DilqrSolve* s) {

@@ -20,6 +20,14 @@
 // pnqp's batch-global decisions replay the guessed trace exactly like the one-thread path: each
 // problem reads the guess word of its timestep, ORs what it observed into the vote word, and
 // commit_kernel verifies and corrects the guess.  There is no group sweep for this family.
+//
+// Network dynamics (DILQR_DYN_NN_RT) are a compile-time variant of the same kernels (NN = true):
+// the sweep forms F_t as the network's Jacobian at the current trajectory instead of reading it,
+// and the rollouts evaluate the network instead of F_t th + f_t.  Every value is formed with the
+// operations and order of Dyn<S, DYN_NN> (dynamics.cuh), and the Riccati update uses the chained
+// association of the compiled env kernels (kChainFma), so the two NN families agree to
+// round-off.  The warp computes hidden units 32 at a time (one per lane) into its slice of shared
+// memory; the outputs / Jacobian entries then accumulate over the hidden units in ascending order.
 #pragma once
 #include "ilqr_kernels.cuh"
 
@@ -30,6 +38,36 @@ constexpr int kRtMaxN = 32;   // one lane per row
 __host__ __device__ inline bool rt_shape_ok(int ns, int nc) {
   return ns >= 1 && nc >= 1 && ns + nc <= kRtMaxN;
 }
+
+// Network scratch of the NN variant, after the RtSmem slice of the warp: one chunk of hidden
+// units, the central-difference input / outputs, and for two hidden layers the first layer's
+// activations z1[H1] and the n_state x H1 product G = W3 diag(d2) W2 of jacobian2.
+template <class S>
+struct RtNetSmem {
+  S *hz, *tp, *fp, *fm, *z1, *G;
+
+  __host__ __device__ size_t carve(char* base, int ns, int nc, int ai0) {
+    const int n = ns + nc, H1 = ai0 & 0xffff;
+    const bool two = (ai0 >> 16) != 0;
+    size_t off = 0;
+    auto take = [&](int cnt) {
+      S* ptr = base ? reinterpret_cast<S*>(base + off) : nullptr;
+      off += (size_t)cnt * sizeof(S);
+      return ptr;
+    };
+    hz = take(kWarp);
+    tp = take(n);
+    fp = take(ns);
+    fm = take(ns);
+    z1 = take(two ? H1 : 0);
+    G = take(two ? ns * H1 : 0);
+    return (off + 15) & ~(size_t)15;
+  }
+  __host__ __device__ static size_t bytes(int ns, int nc, int ai0) {
+    RtNetSmem w;
+    return w.carve(nullptr, ns, nc, ai0);
+  }
+};
 
 // This warp's slice of shared memory.
 template <class S>
@@ -80,6 +118,12 @@ struct RtSmem {
     return m.carve(nullptr, ns, nc);
   }
 };
+
+// One warp's slice of shared memory for the NN variant (ai0 = DynParams::ai[0]).
+template <class S>
+__host__ __device__ inline size_t rt_nn_slice_bytes(int ns, int nc, int ai0) {
+  return RtSmem<S>::bytes(ns, nc) + RtNetSmem<S>::bytes(ns, nc, ai0);
+}
 
 // ---------------------------------------------------------------------------
 // One-thread factorisations over row-major shared-memory matrices: LUpp / Chol of smallmat.cuh
@@ -328,6 +372,146 @@ DILQR_DEVICE void rt_lin_step(const IterParams<S>& p, const RtSmem<S>& m, int t,
   __syncwarp();
 }
 
+// out[0..ns) = the network at in[0..n) (Dyn<S, DYN_NN>::step / step2).  The last hidden layer
+// is computed 32 units at a time, one per lane, into w.hz; lane i < ns then accumulates output i
+// over those units in ascending order.  Two hidden layers: the first goes to w.z1 beforehand.
+template <class S>
+DILQR_DEVICE void rt_nn_step(const DynParams<S>& P, const RtNetSmem<S>& w, const S* in, S* out,
+                             int ns, int nc, int lane) {
+  using D = Dyn<S, DYN_NN>;
+  const int n = ns + nc, H1 = P.ai[0] & 0xffff, H2 = P.ai[0] >> 16, act = P.ai[1];
+  const bool two = H2 != 0;
+  const S* W1 = P.aux;
+  const S* b1 = W1 + (size_t)H1 * n;
+  const int HL = two ? H2 : H1;         // last hidden layer: HL units over KL inputs
+  const int KL = two ? H1 : n;
+  const S* WL = two ? b1 + H1 : W1;
+  const S* bL = WL + (size_t)HL * KL;
+  const S* Wo = bL + HL;                // output layer [ns][HL], bias [ns]
+  const S* bo = Wo + (size_t)ns * HL;
+  const S* src = two ? w.z1 : in;
+  if (two) {
+    for (int h = lane; h < H1; h += kWarp) {
+      S a = S(0);
+      for (int j = 0; j < n; ++j) a = fmaS<S>(__ldg(W1 + (size_t)h * n + j), in[j], a);
+      w.z1[h] = D::act(a + __ldg(b1 + h), act);
+    }
+    __syncwarp();
+  }
+  S acc = S(0);
+  for (int h0 = 0; h0 < HL; h0 += kWarp) {
+    const int h = h0 + lane;
+    if (h < HL) {
+      S a = S(0);
+      for (int j = 0; j < KL; ++j) a = fmaS<S>(__ldg(WL + (size_t)h * KL + j), src[j], a);
+      w.hz[lane] = D::act(a + __ldg(bL + h), act);
+    }
+    __syncwarp();
+    if (lane < ns) {
+      const int cnt = min(kWarp, HL - h0);
+      for (int q = 0; q < cnt; ++q)
+        acc = fmaS<S>(__ldg(Wo + (size_t)lane * HL + h0 + q), w.hz[q], acc);
+    }
+    __syncwarp();
+  }
+  if (lane < ns) {
+    S v = acc + __ldg(bo + lane);
+    if (P.ai[2]) v = v + in[lane];
+    out[lane] = v;
+  }
+  __syncwarp();
+}
+
+// F[ns][n] = d net / d tau at tau (Dyn<S, DYN_NN>::jacobian / jacobian2 / jacobian_fd).  Lane j
+// < n owns column j; every entry accumulates over the hidden units in ascending order with the
+// rounded products W1[h][j] * d_h of the compiled family.
+template <class S>
+DILQR_DEVICE void rt_nn_jacobian(const DynParams<S>& P, const RtNetSmem<S>& w, const S* tau, S* F,
+                                 int ns, int nc, int lane) {
+  using D = Dyn<S, DYN_NN>;
+  const int n = ns + nc;
+  if (P.ai[3] == 1) {   // central differences, eps = 1e-4: 2n network evaluations
+    const S eps = S(1e-4), two_eps = S(2. * 1e-4);
+    if (lane < n) w.tp[lane] = tau[lane];
+    __syncwarp();
+    for (int j = 0; j < n; ++j) {
+      if (lane == 0) w.tp[j] = tau[j] + eps;
+      __syncwarp();
+      rt_nn_step<S>(P, w, w.tp, w.fp, ns, nc, lane);
+      if (lane == 0) w.tp[j] = tau[j] - eps;
+      __syncwarp();
+      rt_nn_step<S>(P, w, w.tp, w.fm, ns, nc, lane);
+      if (lane == 0) w.tp[j] = tau[j];
+      if (lane < ns) F[lane * n + j] = (w.fp[lane] - w.fm[lane]) / two_eps;
+      __syncwarp();
+    }
+    return;
+  }
+  const int H1 = P.ai[0] & 0xffff, H2 = P.ai[0] >> 16, act = P.ai[1];
+  const S* W1 = P.aux;
+  const S* b1 = W1 + (size_t)H1 * n;
+  auto dact = [act](S z) { return act == 1 ? (z <= S(0) ? S(0) : S(1)) : z * (S(1) - z); };
+  for (int e = lane; e < ns * n; e += kWarp) F[e] = S(0);
+  if (H2 == 0) {
+    const S* W2 = b1 + H1;
+    for (int h0 = 0; h0 < H1; h0 += kWarp) {
+      const int h = h0 + lane;
+      if (h < H1) {
+        S a = S(0);
+        for (int j = 0; j < n; ++j) a = fmaS<S>(__ldg(W1 + (size_t)h * n + j), tau[j], a);
+        w.hz[lane] = dact(D::act(a + __ldg(b1 + h), act));
+      }
+      __syncwarp();
+      if (lane < n) {
+        const int j = lane, cnt = min(kWarp, H1 - h0);
+        for (int q = 0; q < cnt; ++q) {
+          const S wj = __ldg(W1 + (size_t)(h0 + q) * n + j) * w.hz[q];
+          for (int i = 0; i < ns; ++i)
+            F[i * n + j] = fmaS<S>(__ldg(W2 + (size_t)i * H1 + h0 + q), wj, F[i * n + j]);
+        }
+      }
+      __syncwarp();
+    }
+  } else {   // G = W3 (diag(d2) W2), then F = G (diag(d1) W1)
+    const S* W2 = b1 + H1;
+    const S* b2 = W2 + (size_t)H2 * H1;
+    const S* W3 = b2 + H2;
+    for (int h = lane; h < H1; h += kWarp) {
+      S a = S(0);
+      for (int j = 0; j < n; ++j) a = fmaS<S>(__ldg(W1 + (size_t)h * n + j), tau[j], a);
+      w.z1[h] = D::act(a + __ldg(b1 + h), act);
+      for (int i = 0; i < ns; ++i) w.G[i * H1 + h] = S(0);
+    }
+    __syncwarp();
+    for (int k0 = 0; k0 < H2; k0 += kWarp) {
+      const int k = k0 + lane;
+      if (k < H2) {
+        S a = S(0);
+        for (int h = 0; h < H1; ++h) a = fmaS<S>(__ldg(W2 + (size_t)k * H1 + h), w.z1[h], a);
+        w.hz[lane] = dact(D::act(a + __ldg(b2 + k), act));
+      }
+      __syncwarp();
+      const int cnt = min(kWarp, H2 - k0);
+      for (int h = lane; h < H1; h += kWarp)   // column h of G on one lane
+        for (int q = 0; q < cnt; ++q) {
+          const S wv = __ldg(W2 + (size_t)(k0 + q) * H1 + h) * w.hz[q];
+          for (int i = 0; i < ns; ++i)
+            w.G[i * H1 + h] = fmaS<S>(__ldg(W3 + (size_t)i * H2 + k0 + q), wv, w.G[i * H1 + h]);
+        }
+      __syncwarp();
+    }
+    if (lane < n) {
+      const int j = lane;
+      for (int h = 0; h < H1; ++h) {
+        const S wj = __ldg(W1 + (size_t)h * n + j) * dact(w.z1[h]);
+        for (int i = 0; i < ns; ++i) F[i * n + j] = fmaS<S>(w.G[i * H1 + h], wj, F[i * n + j]);
+      }
+    }
+  }
+  if (P.ai[2] && lane < ns) F[lane * n + lane] = F[lane * n + lane] + S(1);
+  __syncwarp();
+}
+
 template <class S>
 DILQR_DEVICE void rt_bounds(const IterParams<S>& p, int t, int b, int nc, int a, S* lo, S* hi) {
   if (p.bounds_kind == 2) {
@@ -341,11 +525,13 @@ DILQR_DEVICE void rt_bounds(const IterParams<S>& p, int t, int b, int nc, int a,
 
 // ---------------------------------------------------------------------------
 // Phase A: c_back + Riccati backward sweep with gains and pnqp (lqr_step.py:52-160,289-295),
-// the order of operations of IterKernel::backward_sweep for LinDx.
+// the order of operations of IterKernel::backward_sweep for LinDx (NN: for DYN_NN, whose
+// Riccati update uses the chained association kChainFma).
 // ---------------------------------------------------------------------------
-template <class S>
-DILQR_DEVICE void rt_backward_sweep(const IterParams<S>& p, const RtSmem<S>& m, int ns, int nc,
-                                    int b, int lane) {
+template <class S, bool NN>
+DILQR_DEVICE void rt_backward_sweep(const IterParams<S>& p, const RtSmem<S>& m,
+                                    const RtNetSmem<S>& w, int ns, int nc, int b, int lane) {
+  constexpr bool kChain = NN && kChainFmaOn;
   const int n = ns + nc, NK = nc * ns + nc, T = p.T;
   // lazy best-iterate tracking (mpc.py:272-285), see IterParams::take
   const bool flush = (p.take[b] & 1) != 0;
@@ -354,7 +540,7 @@ DILQR_DEVICE void rt_backward_sweep(const IterParams<S>& p, const RtSmem<S>& m, 
     const S* Cg = cost_src<S>(p.C, p.C_bcast, t, p.B, b, n * n);
     const S* cg = cost_src<S>(p.c, p.c_bcast, t, p.B, b, n);
     for (int e = lane; e < n * n; e += kWarp) m.Q[e] = __ldg(Cg + e);
-    if (t < T - 1) {
+    if (!NN && t < T - 1) {
       const S* Fg = p.F + ((size_t)t * p.B + b) * (ns * n);
       for (int e = lane; e < ns * n; e += kWarp) m.F[e] = __ldg(Fg + e);
     }
@@ -364,11 +550,14 @@ DILQR_DEVICE void rt_backward_sweep(const IterParams<S>& p, const RtSmem<S>& m, 
       if (flush) p.traj_best[bidx(t, lane, n, b, p.nW)] = tv;
     }
     __syncwarp();
+    if constexpr (NN) {   // F_t = the network's Jacobian at tau_t (mpc_explicit.py:516-546)
+      if (t < T - 1) rt_nn_jacobian<S>(p.dyn, w, m.tau, m.F, ns, nc, lane);
+    }
     if (lane < n) {
       const int i = lane;
-      S acc = S(0);  // c_back = C tau + c   (lqr_step.py:294)
+      S acc = kChain ? __ldg(cg + i) : S(0);  // c_back = C tau + c   (lqr_step.py:294)
       for (int j = 0; j < n; ++j) acc = fmaS<S>(m.Q[i * n + j], m.tau[j], acc);
-      m.q[i] = acc + __ldg(cg + i);
+      m.q[i] = kChain ? acc : acc + __ldg(cg + i);
       if (t < T - 1) {  // Q = C + (F' V) F ; q = c~ + F' v     (lqr_step.py:66-70)
         for (int k = 0; k < ns; ++k) {
           S a2 = S(0);
@@ -376,13 +565,13 @@ DILQR_DEVICE void rt_backward_sweep(const IterParams<S>& p, const RtSmem<S>& m, 
           m.M[i * ns + k] = a2;
         }
         for (int j = 0; j < n; ++j) {
-          S a2 = S(0);
+          S a2 = kChain ? m.Q[i * n + j] : S(0);
           for (int k = 0; k < ns; ++k) a2 = fmaS<S>(m.M[i * ns + k], m.F[k * n + j], a2);
-          m.Q[i * n + j] = m.Q[i * n + j] + a2;
+          m.Q[i * n + j] = kChain ? a2 : m.Q[i * n + j] + a2;
         }
-        S a3 = S(0);
+        S a3 = kChain ? m.q[i] : S(0);
         for (int l = 0; l < ns; ++l) a3 = fmaS<S>(m.F[l * n + i], m.v[l], a3);
-        m.q[i] = m.q[i] + a3;
+        m.q[i] = kChain ? a3 : m.q[i] + a3;
       }
     }
     __syncwarp();
@@ -484,22 +673,37 @@ DILQR_DEVICE void rt_backward_sweep(const IterParams<S>& p, const RtSmem<S>& m, 
         for (int c2 = 0; c2 < nc; ++c2) acc = fmaS<S>(m.K[c2 * ns + i], Qu[c2 * n + ns + a], acc);
         m.KQ[i * nc + a] = acc;
       }
-      for (int j = 0; j < ns; ++j) {
+      if constexpr (kChain) {
+        for (int j = 0; j < ns; ++j) {
+          S acc = m.Q[i * n + j];
+          for (int a = 0; a < nc; ++a) acc = fmaS<S>(m.Q[i * n + ns + a], m.K[a * ns + j], acc);
+          for (int a = 0; a < nc; ++a) acc = fmaS<S>(m.K[a * ns + i], Qu[a * n + j], acc);
+          for (int a = 0; a < nc; ++a) acc = fmaS<S>(m.KQ[i * nc + a], m.K[a * ns + j], acc);
+          m.V[i * ns + j] = acc;
+        }
+        S acc = m.q[i];
+        for (int a = 0; a < nc; ++a) acc = fmaS<S>(m.Q[i * n + ns + a], m.k[a], acc);
+        for (int a = 0; a < nc; ++a) acc = fmaS<S>(m.K[a * ns + i], m.q[ns + a], acc);
+        for (int a = 0; a < nc; ++a) acc = fmaS<S>(m.KQ[i * nc + a], m.k[a], acc);
+        m.v[i] = acc;
+      } else {
+        for (int j = 0; j < ns; ++j) {
+          S t1 = S(0), t2 = S(0), t3 = S(0);
+          for (int a = 0; a < nc; ++a) {
+            t1 = fmaS<S>(m.Q[i * n + ns + a], m.K[a * ns + j], t1);
+            t2 = fmaS<S>(m.K[a * ns + i], Qu[a * n + j], t2);
+            t3 = fmaS<S>(m.KQ[i * nc + a], m.K[a * ns + j], t3);
+          }
+          m.V[i * ns + j] = ((m.Q[i * n + j] + t1) + t2) + t3;
+        }
         S t1 = S(0), t2 = S(0), t3 = S(0);
         for (int a = 0; a < nc; ++a) {
-          t1 = fmaS<S>(m.Q[i * n + ns + a], m.K[a * ns + j], t1);
-          t2 = fmaS<S>(m.K[a * ns + i], Qu[a * n + j], t2);
-          t3 = fmaS<S>(m.KQ[i * nc + a], m.K[a * ns + j], t3);
+          t1 = fmaS<S>(m.Q[i * n + ns + a], m.k[a], t1);
+          t2 = fmaS<S>(m.K[a * ns + i], m.q[ns + a], t2);
+          t3 = fmaS<S>(m.KQ[i * nc + a], m.k[a], t3);
         }
-        m.V[i * ns + j] = ((m.Q[i * n + j] + t1) + t2) + t3;
+        m.v[i] = ((m.q[i] + t1) + t2) + t3;
       }
-      S t1 = S(0), t2 = S(0), t3 = S(0);
-      for (int a = 0; a < nc; ++a) {
-        t1 = fmaS<S>(m.Q[i * n + ns + a], m.k[a], t1);
-        t2 = fmaS<S>(m.K[a * ns + i], m.q[ns + a], t2);
-        t3 = fmaS<S>(m.KQ[i * nc + a], m.k[a], t3);
-      }
-      m.v[i] = ((m.q[i] + t1) + t2) + t3;
     }
     __syncwarp();
   }
@@ -509,9 +713,9 @@ DILQR_DEVICE void rt_backward_sweep(const IterParams<S>& p, const RtSmem<S>& m, 
 // Phase B: rollout with the affine control law + line search (lqr_step.py:164-261), the
 // bookkeeping of IterKernel::forward_linesearch for one problem.
 // ---------------------------------------------------------------------------
-template <class S>
-DILQR_DEVICE void rt_forward_linesearch(const IterParams<S>& p, const RtSmem<S>& m, int ns, int nc,
-                                        int b, int lane) {
+template <class S, bool NN>
+DILQR_DEVICE void rt_forward_linesearch(const IterParams<S>& p, const RtSmem<S>& m,
+                                        const RtNetSmem<S>& w, int ns, int nc, int b, int lane) {
   const int n = ns + nc, NK = nc * ns + nc, T = p.T;
   const S old_cost = p.cost_cur[b];
   S alpha = S(1);
@@ -554,7 +758,10 @@ DILQR_DEVICE void rt_forward_linesearch(const IterParams<S>& p, const RtSmem<S>&
       if (lane < n) p.traj_new[bidx(t, lane, n, b, p.nW)] = m.th[lane];
       cost = cost + rt_stage_cost<S>(m, cost_src<S>(p.C, p.C_bcast, t, p.B, b, n * n),
                                      cost_src<S>(p.c, p.c_bcast, t, p.B, b, n), n, lane);
-      if (t < T - 1) rt_lin_step<S>(p, m, t, b, ns, nc, lane);
+      if (t < T - 1) {
+        if constexpr (NN) rt_nn_step<S>(p.dyn, w, m.th, m.xh, ns, nc, lane);
+        else rt_lin_step<S>(p, m, t, b, ns, nc, lane);
+      }
     }
     if (lane == 0) {
       res_cost = cost;
@@ -571,39 +778,46 @@ DILQR_DEVICE void rt_forward_linesearch(const IterParams<S>& p, const RtSmem<S>&
   }
 }
 
-// One warp per problem; the warp's slice of dynamic shared memory is RtSmem<S>::bytes(ns, nc).
-template <class S>
+// One warp per problem; the warp's slice of dynamic shared memory is RtSmem<S>::bytes(ns, nc),
+// followed for the NN variant by its RtNetSmem (rt_nn_slice_bytes).
+template <class S, bool NN>
 DILQR_DEVICE bool rt_warp_setup(const IterParams<S>& p, int ns, int nc, char* smem, RtSmem<S>& m,
-                                int& b, int& lane) {
+                                RtNetSmem<S>& w, int& b, int& lane) {
   lane = threadIdx.x & 31;
   const int warp = threadIdx.x >> 5;
   b = blockIdx.x * (blockDim.x >> 5) + warp;
   if (b >= p.B) return false;
-  m.carve(smem + warp * RtSmem<S>::bytes(ns, nc), ns, nc);
+  if constexpr (NN) {
+    char* base = smem + warp * rt_nn_slice_bytes<S>(ns, nc, p.dyn.ai[0]);
+    m.carve(base, ns, nc);
+    w.carve(base + RtSmem<S>::bytes(ns, nc), ns, nc, p.dyn.ai[0]);
+  } else {
+    m.carve(smem + warp * RtSmem<S>::bytes(ns, nc), ns, nc);
+  }
   return true;
 }
 
-template <class S>
-__global__ void rt_iter_kernel(const __grid_constant__ IterParams<S> p,
-                                                      int ns, int nc) {
+template <class S, bool NN>
+DILQR_DEVICE void rt_iter(const IterParams<S>& p, int ns, int nc) {
   extern __shared__ __align__(128) char smem[];
   if (p.halt && *reinterpret_cast<const volatile uint32_t*>(p.halt)) return;  // pipelined loop stopped
   RtSmem<S> m;
+  RtNetSmem<S> w;
   int b, lane;
-  if (!rt_warp_setup<S>(p, ns, nc, smem, m, b, lane)) return;
-  rt_backward_sweep<S>(p, m, ns, nc, b, lane);
-  if (!p.gains_only) rt_forward_linesearch<S>(p, m, ns, nc, b, lane);
+  if (!rt_warp_setup<S, NN>(p, ns, nc, smem, m, w, b, lane)) return;
+  rt_backward_sweep<S, NN>(p, m, w, ns, nc, b, lane);
+  if (!p.gains_only) rt_forward_linesearch<S, NN>(p, m, w, ns, nc, b, lane);
 }
 
 // begin: nominal rollout of u_init (util.get_traj) + its cost (util.get_cost), or the given
 // trajectory x_cur (standalone LQRStep), into the current-trajectory buffer.
-template <class S>
-__global__ void rt_begin_kernel(const __grid_constant__ IterParams<S> p,
-                                                       int ns, int nc) {
+template <class S, bool NN>
+DILQR_DEVICE void rt_begin(const IterParams<S>& p, int ns, int nc) {
   extern __shared__ __align__(128) char smem[];
   RtSmem<S> m;
+  RtNetSmem<S> w;
   int b, lane;
-  if (!rt_warp_setup<S>(p, ns, nc, smem, m, b, lane)) return;
+  if (!rt_warp_setup<S, NN>(p, ns, nc, smem, m, w, b, lane)) return;
   const int n = ns + nc, T = p.T;
   const bool want_cost = !(p.gains_only && p.x_cur);
   if (lane < ns) m.xh[lane] = __ldg(p.x_init + (size_t)b * ns + lane);
@@ -617,13 +831,34 @@ __global__ void rt_begin_kernel(const __grid_constant__ IterParams<S> p,
     if (want_cost)
       cost = cost + rt_stage_cost<S>(m, cost_src<S>(p.C, p.C_bcast, t, p.B, b, n * n),
                                      cost_src<S>(p.c, p.c_bcast, t, p.B, b, n), n, lane);
-    if (want_cost && t < T - 1 && !p.x_cur) rt_lin_step<S>(p, m, t, b, ns, nc, lane);
+    if (want_cost && t < T - 1 && !p.x_cur) {
+      if constexpr (NN) rt_nn_step<S>(p.dyn, w, m.th, m.xh, ns, nc, lane);
+      else rt_lin_step<S>(p, m, t, b, ns, nc, lane);
+    }
     __syncwarp();
   }
   if (lane == 0) {
     p.cost_cur[b] = cost;
     p.take[b] = 0;
   }
+}
+
+// LinDx (DILQR_DYN_LINDX_RT) and network (DILQR_DYN_NN_RT) instantiations
+template <class S>
+__global__ void rt_iter_kernel(const __grid_constant__ IterParams<S> p, int ns, int nc) {
+  rt_iter<S, false>(p, ns, nc);
+}
+template <class S>
+__global__ void rt_nn_iter_kernel(const __grid_constant__ IterParams<S> p, int ns, int nc) {
+  rt_iter<S, true>(p, ns, nc);
+}
+template <class S>
+__global__ void rt_begin_kernel(const __grid_constant__ IterParams<S> p, int ns, int nc) {
+  rt_begin<S, false>(p, ns, nc);
+}
+template <class S>
+__global__ void rt_nn_begin_kernel(const __grid_constant__ IterParams<S> p, int ns, int nc) {
+  rt_begin<S, true>(p, ns, nc);
 }
 
 // ---------------------------------------------------------------------------

@@ -1,8 +1,10 @@
 """Dynamics containers of the upstream mpc.pytorch API kept by the reference
 (dynamics.py): ``NNDynamics``, ``AffineDynamics`` and ``CtrlPassthroughDynamics``.
 
-``NNDynamics`` (one hidden layer) runs inside the fused iteration kernels as the
-device dynamics ``DILQR_DYN_NN`` (csrc/dynamics.cuh): ``MPC.forward`` packs the weights
+``NNDynamics`` with one or two hidden layers (sigmoid or relu; at most 128 units in the first
+of two layers) runs inside the iteration kernels as device dynamics, for any shape with
+``n_state + n_ctrl <= 32``: ``DILQR_DYN_NN`` (csrc/dynamics.cuh) on the compiled shapes,
+``DILQR_DYN_NN_RT`` (csrc/rt_kernels.cuh) on every other one.  ``MPC.forward`` packs the weights
 once per call; the KKT gradients ``dF, df`` of the solve reach the weights through
 ``grad_input`` evaluated (with autograd) at the solution, which is what the reference
 does in ``linearize_dynamics(diff=True)`` (mpc.py:490-523).
@@ -82,7 +84,8 @@ class NNDynamics(nn.Module):
 
     # -- device side ---------------------------------------------------------
     def _dilqr_pack(self, dtype, device):
-        """(weight buffer, ints) for DILQR_DYN_NN: weight[out][in], bias[out] per layer."""
+        """(weight buffer, ints) for DILQR_DYN_NN / DILQR_DYN_NN_RT: weight[out][in], bias[out]
+        per layer."""
         if len(self.fcs) not in (2, 3):
             raise NotImplementedError("device NNDynamics: one or two hidden layers; got %d"
                                       % (len(self.fcs) - 1))

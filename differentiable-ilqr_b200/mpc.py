@@ -467,9 +467,11 @@ class MPC(nn.Module):
 
     def _forward_network(self, x_init, C, c, dx, n_batch):
         """Module dynamics ``dynamics.NNDynamics`` (mpc.py:248-337 with
-        grad_method=ANALYTIC): the iLQR solve runs in the fused kernels with the network
-        as device dynamics; the gradient is the KKT adjoint at the solution with F, f from
-        ``linearize_dynamics(diff=True)`` (mpc.py:490-523)."""
+        grad_method=ANALYTIC): the iLQR solve runs in the kernels with the network as device
+        dynamics -- the compiled ones for their shapes, the runtime-dimension ones for any
+        other shape up to 32 variables (``_solver.nn_kernels``); the gradient is the KKT
+        adjoint at the solution with F, f from ``linearize_dynamics(diff=True)``
+        (mpc.py:490-523), a LinDx problem of the same shape."""
         if self.grad_method not in (GradMethods.ANALYTIC, GradMethods.AUTO_DIFF,
                                     GradMethods.FINITE_DIFF):
             raise NotImplementedError("Module dynamics: grad_method %s" % self.grad_method)

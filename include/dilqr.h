@@ -36,13 +36,21 @@ enum {
   DILQR_DYN_PENDULUM = 1, /* env_dx/pendulum.py:60-95, Jacobian 444-475             */
   DILQR_DYN_CARTPOLE = 2, /* env_dx/cartpole.py:64-97, Jacobian 790-839             */
   DILQR_DYN_ROCKET   = 3, /* env_dx/rocket.py:82-164,  Jacobian 324-426             */
-  DILQR_DYN_NN       = 4, /* dynamics.py:15-130 NNDynamics, one hidden layer (dyn_aux)  */
-  DILQR_DYN_LINDX_RT = 5  /* LinDx through the runtime-dimension kernels (rt_kernels.cuh):
+  DILQR_DYN_NN       = 4, /* dynamics.py:15-130 NNDynamics, one or two hidden layers
+                             (dyn_aux, dyn_ai); compiled shapes only                   */
+  DILQR_DYN_LINDX_RT = 5, /* LinDx through the runtime-dimension kernels (rt_kernels.cuh):
                              any n_state >= 1, n_ctrl >= 1 with n_state + n_ctrl <= 32, both
                              dtypes; same problem struct and entry points as DILQR_DYN_LINDX.
                              Replays the pnqp trace (never the group sweep); dilqr_mpc_gains
                              and the DiLQR backward calls do not serve it.  Select it with
                              dilqr_lindx_kernels.                                         */
+  DILQR_DYN_NN_RT    = 6  /* NNDynamics through the runtime-dimension kernels: any n_state >= 1,
+                             n_ctrl >= 1 with n_state + n_ctrl <= 32, both dtypes; the same
+                             network limits, DilqrSolve fields (dyn_aux, dyn_ai) and entry points
+                             as DILQR_DYN_NN.  Replays the pnqp trace (never the group sweep);
+                             dilqr_mpc_gains does not serve it and dilqr_kkt_grads rejects it (the
+                             gradient of a network solve is a LinDx KKT problem at the solution).
+                             Select it with dilqr_nn_kernels.                                   */
 };
 
 /* How unconstrained multi-input gains are solved (the reference copies differ). */
@@ -149,7 +157,8 @@ typedef struct DilqrSolve {
   /* scratch */
   void*  workspace;
   size_t workspace_bytes;
-  /* DILQR_DYN_NN only: the network of dynamics.NNDynamics(hidden_sizes=[H] or [H1,H2]) */
+  /* DILQR_DYN_NN / DILQR_DYN_NN_RT only: the network of dynamics.NNDynamics(hidden_sizes=[H] or
+     [H1,H2]) */
   const void* dyn_aux;      /* device, packed in the call's dtype, layer by layer:
                                weight[out][in] then bias[out] (fc0, fc1[, fc2])        */
   int32_t dyn_ai[4];        /* {H1 | H2 << 16 (H2 = 0: one hidden layer; two layers need
@@ -177,8 +186,8 @@ typedef struct DilqrSolve {
 
 const char* dilqr_version(void);
 
-/* 1 if kernels for this combination are compiled in, else 0.  DILQR_DYN_LINDX_RT: 1 for every
- * shape of its range, compiled-in shapes included. */
+/* 1 if kernels for this combination are compiled in, else 0.  DILQR_DYN_LINDX_RT and
+ * DILQR_DYN_NN_RT: 1 for every shape of their range, compiled-in shapes included. */
 int dilqr_supported(int dtype, int n_state, int n_ctrl, int dynamics);
 
 /* Which kernels serve a LinDx problem of this shape: DILQR_DYN_LINDX if the shape is compiled in,
@@ -187,14 +196,19 @@ int dilqr_supported(int dtype, int n_state, int n_ctrl, int dynamics);
  * DilqrKkt.dynamics. */
 int dilqr_lindx_kernels(int dtype, int n_state, int n_ctrl);
 
+/* The same choice for a network (NNDynamics) problem: DILQR_DYN_NN if the shape is compiled in,
+ * else DILQR_DYN_NN_RT if n_state + n_ctrl <= 32, else DILQR_EUNSUPPORTED; DILQR_EINVAL for a bad
+ * dtype or a non-positive dimension.  Put the result into DilqrSolve.dynamics. */
+int dilqr_nn_kernels(int dtype, int n_state, int n_ctrl);
+
 /* Choose how dilqr_mpc_iterate resolves pnqp's batch-global decisions and write it to
  * s->group_sweep.  Reads only dtype, n_state, n_ctrl, dynamics, bounds_kind, solo and n_batch;
  * call it before dilqr_workspace_bytes.  The group sweep runs shapes whose matrices do not fit
  * one thread's registers, and box-constrained (solo == 0) multi-input batches, wherever the
  * shape has it and the batch fits the current device at once; everything else replays a
- * guessed trace.  DILQR_DYN_LINDX_RT always replays (group_sweep = 0) and never queries the
- * device.  DILQR_EUNSUPPORTED: the shape is not compiled in (DILQR_DYN_LINDX_RT: out of its
- * range). */
+ * guessed trace.  DILQR_DYN_LINDX_RT and DILQR_DYN_NN_RT always replay (group_sweep = 0) and
+ * never query the device.  DILQR_EUNSUPPORTED: the shape is not compiled in (the runtime ids: out
+ * of their range). */
 int dilqr_mpc_plan(DilqrSolve* s);
 
 /* Bytes of workspace the dilqr_mpc_* calls need. */
