@@ -19,6 +19,8 @@ DYN_NN_RT = 6           # NNDynamics through the runtime-dimension kernels (n_st
 GAIN_PLAIN, GAIN_CHOL_REG = 0, 1
 BOUNDS_NONE, BOUNDS_SCALAR, BOUNDS_TENSOR = 0, 1, 2
 PNQP_MAX_ITER = 20
+PNQP_COMPILED, PNQP_RT = 0, 1   # dilqr_pnqp_kernels: dilqr_pnqp / dilqr_pnqp_rt serves the call
+PNQP_RT_MAX_N, PNQP_RT_MAX_ITER = 256, 1024
 
 ERRORS = {0: "ok", -1: "invalid argument", -2: "unsupported (dtype, n_state, n_ctrl, dynamics)",
           -3: "pointer not 16-byte aligned", -4: "workspace too small",
@@ -144,6 +146,8 @@ SYMBOLS = {
                                    C.c_void_p, C.POINTER(C.c_void_p), C.c_void_p]),
     "dilqr_pnqp": (C.c_int, [C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 10 + [C.c_int]
                    + [C.c_void_p] * 2),
+    "dilqr_pnqp_kernels": (C.c_int, [C.c_int] * 3),
+    "dilqr_pnqp_rt": (C.c_int, [C.c_int] * 4 + [C.c_void_p] * 10 + [C.c_int] + [C.c_void_p] * 2),
     "dilqr_costate_tables": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_double), C.c_int, C.c_int]
                              + [C.c_void_p] * 6 + [C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "dilqr_lam_pack_size": (C.c_int, [C.c_int]),
@@ -207,7 +211,7 @@ KERNELS_PER_CALL = {
     "dilqr_sens_theta_adjoint": 1, "dilqr_kkt_grads": 1, "dilqr_linearize": 1, "dilqr_rollout": 1,
     "dilqr_costate_tables": 1, "dilqr_richardson_update": 1, "dilqr_sens_theta": 1,
     "dilqr_adjoint_factor": 1, "dilqr_adjoint_pass": 1, "dilqr_adjoint_final": 1,
-    "dilqr_pnqp": 2, "dilqr_env_tables": 1, "dilqr_tile_cost": 2, "dilqr_tile_cost_grad": 2,
+    "dilqr_pnqp": 2, "dilqr_pnqp_rt": 2, "dilqr_env_tables": 1, "dilqr_tile_cost": 2, "dilqr_tile_cost_grad": 2,
 }
 launch_count = 0     # running total of kernels launched through this binding
 profile = None       # set to a dict {name: [(start_event, end_event), ...]} to time calls

@@ -14,6 +14,9 @@
 #include "adjoint_kernels.cuh"
 #include "group_kernels.cuh"
 #include "rt_kernels.cuh"
+#if !defined(DILQR_GROUP) || DILQR_GROUP == 0
+#include "pnqp_rt.cuh"
+#endif
 
 namespace dilqr {
 
@@ -756,6 +759,35 @@ int DILQR_SUFFIX(pnqp)(int n, int B, const void* H, const void* q, const void* l
     case 8: return launch_pnqp<8>(B, H, q, lo, hi, x0, x, lu, piv, If, trace, solo, status, st);
     default: return DILQR_EUNSUPPORTED;
   }
+}
+
+// n and the iteration budget at run time (pnqp_rt.cuh): one warp per problem, the warp's
+// shared-memory slice sized for n.
+int DILQR_SUFFIX(pnqp_rt)(int n, int n_iter, int B, const void* H, const void* q, const void* lo,
+                          const void* hi, const void* x0, void* x, void* lu, int32_t* piv, void* If,
+                          uint32_t* trace, int solo, DilqrStatus* status, void* stream) {
+  if (!H || !q || !lo || !hi || !x || !lu || !piv || !If || !trace || !status || B <= 0 ||
+      n <= 0 || n_iter <= 0)
+    return DILQR_EINVAL;
+  if (!pnqp_rt_ok(n, n_iter)) return DILQR_EUNSUPPORTED;
+  if (reinterpret_cast<uintptr_t>(trace) % sizeof(uint32_t)) return DILQR_EALIGN;
+  using S = Scalar;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  uint32_t* guess = trace;
+  uint32_t* votes = trace + n_iter;
+  const size_t per = PnqpRtSmem<S>::bytes(n);
+  int wpb = (int)((96 * 1024) / per);   // <= 96 KB a block: two blocks fit one SM
+  if (wpb > 4) wpb = 4;
+  const size_t smem = per * wpb;
+  if (smem > 48 * 1024)
+    cudaFuncSetAttribute(pnqp_rt_kernel<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaMemsetAsync(votes, 0, (size_t)n_iter * sizeof(uint32_t), st);
+  pnqp_rt_kernel<S><<<(B + wpb - 1) / wpb, wpb * kWarp, smem, st>>>(
+      B, n, n_iter, static_cast<const S*>(H), static_cast<const S*>(q), static_cast<const S*>(lo),
+      static_cast<const S*>(hi), static_cast<const S*>(x0), static_cast<S*>(x), static_cast<S*>(lu),
+      piv, static_cast<S*>(If), guess, votes, solo);
+  pnqp_rt_verify_kernel<<<1, 32, 0, st>>>(guess, votes, n_iter, solo, status);
+  return cudaGetLastError() == cudaSuccess ? DILQR_OK : DILQR_ECUDA;
 }
 
 // ------------------------------------------------- factored adjoint solves

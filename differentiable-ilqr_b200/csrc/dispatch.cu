@@ -29,6 +29,9 @@ namespace dilqr {
   int env_tables_##sfx(int, const double*, int, const void*, const void*, void* const*, void*); \
   int pnqp_##sfx(int, int, const void*, const void*, const void*, const void*, const void*, \
                  void*, void*, int32_t*, void*, uint32_t*, int, DilqrStatus*, void*);     \
+  int pnqp_rt_##sfx(int, int, int, const void*, const void*, const void*, const void*,    \
+                    const void*, void*, void*, int32_t*, void*, uint32_t*, int, DilqrStatus*, \
+                    void*);                                                               \
   size_t adjoint_workspace_bytes_##sfx(const DilqrAdjoint*);                              \
   size_t adjoint_dtau_offset_##sfx(const DilqrAdjoint*);                                  \
   int workspace_view_##sfx(const DilqrSolve*, DilqrWsView*);                              \
@@ -203,6 +206,26 @@ int dilqr_pnqp(int dtype, int n, int B, const void* H, const void* q, const void
   return ROUTE(dtype,
                dilqr::pnqp_f32_g0(n, B, H, q, lower, upper, x_init, x, lu, pivots, If, trace, solo, status, st),
                dilqr::pnqp_f64_g0(n, B, H, q, lower, upper, x_init, x, lu, pivots, If, trace, solo, status, st));
+}
+
+int dilqr_pnqp_kernels(int dtype, int n, int n_iter) {
+  if ((dtype != DILQR_F32 && dtype != DILQR_F64) || n <= 0 || n_iter <= 0) return DILQR_EINVAL;
+  // the sizes DILQR_SUFFIX(pnqp) (api.cu) instantiates, at their fixed budget
+  const bool compiled = n == 1 || n == 2 || n == 3 || n == 4 || n == 6 || n == 8;
+  if (compiled && n_iter == DILQR_PNQP_MAX_ITER) return DILQR_PNQP_COMPILED;
+  if (n <= DILQR_PNQP_RT_MAX_N && n_iter <= DILQR_PNQP_RT_MAX_ITER) return DILQR_PNQP_RT;
+  return DILQR_EUNSUPPORTED;
+}
+
+int dilqr_pnqp_rt(int dtype, int n, int n_iter, int B, const void* H, const void* q,
+                  const void* lower, const void* upper, const void* x_init, void* x, void* lu,
+                  int32_t* pivots, void* If, uint32_t* trace, int solo, DilqrStatus* status,
+                  void* st) {
+  return ROUTE(dtype,
+               dilqr::pnqp_rt_f32_g0(n, n_iter, B, H, q, lower, upper, x_init, x, lu, pivots, If,
+                                     trace, solo, status, st),
+               dilqr::pnqp_rt_f64_g0(n, n_iter, B, H, q, lower, upper, x_init, x, lu, pivots, If,
+                                     trace, solo, status, st));
 }
 
 size_t dilqr_adjoint_workspace_bytes(const DilqrAdjoint* a) {

@@ -11,15 +11,20 @@ namespace dilqr {
 // Verify the replayed pnqp control-flow trace (one block).  votes == guess up
 // to the first wrong guess; on mismatch the votes become the next guess.
 // Also derives n_total_qp_iter = sum_t (1 + n_qp_iter_t)  (lqr_step.py:140) and
-// resets the reduction fields of the status block.
+// resets the reduction fields of the status block.  W words per timestep (the
+// pnqp iteration budget n_iter): W_CT when > 0, else W_RT.  trace_verify_kernel
+// passes W_CT = kPnqpMaxIter and compiles to the code it had before the runtime
+// budget existed.
 // ---------------------------------------------------------------------------
-static __global__ void trace_verify_kernel(uint32_t* __restrict__ guess, const uint32_t* __restrict__ votes,
-                                    int T, int boxed, int solo, DilqrStatus* status,
-                                    DilqrControl* ctrl = nullptr) {
+template <int W_CT>
+DILQR_DEVICE void trace_verify_block(uint32_t* __restrict__ guess, const uint32_t* __restrict__ votes,
+                                     int T, int W_RT, int boxed, int solo, DilqrStatus* status,
+                                     DilqrControl* ctrl) {
+  const int W = W_CT > 0 ? W_CT : W_RT;
   if (ctrl && ctrl->halt) return;   // uniform: whole block leaves
   __shared__ int s_first;
   __shared__ unsigned s_nqp, s_unconv;
-  const int n = T * kPnqpMaxIter;
+  const int n = T * W;
   if (threadIdx.x == 0) {
     s_first = n;
     s_nqp = 0;
@@ -31,8 +36,8 @@ static __global__ void trace_verify_kernel(uint32_t* __restrict__ guess, const u
     // right there, so Armijo bits voted under a wrong "moving" guess are void.
     // Processing order of the sweep is t = T-1 .. 0, it = 0 .. 19.
     for (int i = threadIdx.x; i < n; i += blockDim.x) {
-      const int t = T - 1 - i / kPnqpMaxIter, it = i % kPnqpMaxIter;
-      const int slot = t * kPnqpMaxIter + it;
+      const int t = T - 1 - i / W, it = i % W;
+      const int slot = t * W + it;
       uint32_t v = votes[slot];
       if (!(v & 1u)) v = 0;
       if (guess[slot] != v) atomicMin(&s_first, i);
@@ -40,10 +45,10 @@ static __global__ void trace_verify_kernel(uint32_t* __restrict__ guess, const u
     __syncthreads();
     for (int t = threadIdx.x; t < T; t += blockDim.x) {
       int it = 0;
-      while (it < kPnqpMaxIter && (votes[t * kPnqpMaxIter + it] & 1u)) ++it;
-      if (it == kPnqpMaxIter) {
+      while (it < W && (votes[t * W + it] & 1u)) ++it;
+      if (it == W) {
         atomicAdd(&s_unconv, 1u);
-        it = kPnqpMaxIter - 1;   // pnqp.py:82 returns i = n_iter-1
+        it = W - 1;   // pnqp.py:82 returns i = n_iter-1
       }
       atomicAdd(&s_nqp, 1u + (unsigned)it);
     }
@@ -72,6 +77,12 @@ static __global__ void trace_verify_kernel(uint32_t* __restrict__ guess, const u
     status->mean_best_cost = 0.0;
     if (ctrl && s_first < n) ctrl->halt = 2u;
   }
+}
+
+static __global__ void trace_verify_kernel(uint32_t* __restrict__ guess, const uint32_t* __restrict__ votes,
+                                    int T, int boxed, int solo, DilqrStatus* status,
+                                    DilqrControl* ctrl = nullptr) {
+  trace_verify_block<kPnqpMaxIter>(guess, votes, T, 0, boxed, solo, status, ctrl);
 }
 
 // ---------------------------------------------------------------------------

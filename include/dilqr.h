@@ -273,10 +273,34 @@ int dilqr_mpc_gains(const DilqrSolve* s, void* lam_blk, void* stream);
  * 20 vote words).  After the call status->trace_match tells whether the replayed
  * batch-global control flow was right; if 0, call again (the guess was corrected).
  * status->n_total_qp_iter - 1 is the returned iteration count `i`,
- * status->pnqp_unconverged != 0 the "[WARNING] pnqp warning" case (pnqp.py:81). */
+ * status->pnqp_unconverged != 0 the "[WARNING] pnqp warning" case (pnqp.py:81).
+ * Compiled for n in {1,2,3,4,6,8} and n_iter = DILQR_PNQP_MAX_ITER (else DILQR_EUNSUPPORTED);
+ * every other size up to 256 and budget up to 1024 is served by dilqr_pnqp_rt below. */
 int dilqr_pnqp(int dtype, int n, int n_batch, const void* H, const void* q, const void* lower,
                const void* upper, const void* x_init, void* x, void* lu, int32_t* pivots,
                void* If, uint32_t* trace, int solo, DilqrStatus* status, void* stream);
+
+/* Which kernels serve a standalone pnqp of size n with budget n_iter: DILQR_PNQP_COMPILED
+ * (dilqr_pnqp) for n in {1,2,3,4,6,8} with n_iter == DILQR_PNQP_MAX_ITER, else DILQR_PNQP_RT
+ * (dilqr_pnqp_rt) for n <= DILQR_PNQP_RT_MAX_N and n_iter <= DILQR_PNQP_RT_MAX_ITER, else
+ * DILQR_EUNSUPPORTED; DILQR_EINVAL for a bad dtype or n <= 0 or n_iter <= 0. */
+enum { DILQR_PNQP_COMPILED = 0, DILQR_PNQP_RT = 1 };
+#define DILQR_PNQP_RT_MAX_N 256
+#define DILQR_PNQP_RT_MAX_ITER 1024
+int dilqr_pnqp_kernels(int dtype, int n, int n_iter);
+
+/* dilqr_pnqp with n and the iteration budget n_iter at run time (csrc/pnqp_rt.cuh, one warp per
+ * problem): any 1 <= n <= DILQR_PNQP_RT_MAX_N, 1 <= n_iter <= DILQR_PNQP_RT_MAX_ITER, both dtypes,
+ * the compiled sizes included (where it returns bitwise what dilqr_pnqp returns).  Same
+ * arguments, outputs and status fields as dilqr_pnqp, except that `trace` holds 2 * n_iter
+ * words (n_iter guess words, zero-initialised by the caller before the first call, then n_iter
+ * vote words) and needs only 4-byte alignment.  DILQR_EINVAL for a null pointer, n_batch <= 0,
+ * n <= 0 or n_iter <= 0, DILQR_EUNSUPPORTED beyond the limits, DILQR_EALIGN for a misaligned
+ * `trace`; nothing is enqueued then. */
+int dilqr_pnqp_rt(int dtype, int n, int n_iter, int n_batch, const void* H, const void* q,
+                  const void* lower, const void* upper, const void* x_init, void* x, void* lu,
+                  int32_t* pivots, void* If, uint32_t* trace, int solo, DilqrStatus* status,
+                  void* stream);
 
 /* ---- analytic linearisation (mpc_explicit.py:516-546) --------------------
  * x[T,B,ns], u[T,B,nc] -> F[T-1,B,ns,n], f[T-1,B,ns] (f may be NULL). */
