@@ -579,15 +579,20 @@ def dilqr_prepare(x_init, C_, c_, x, u, dxmod, n_state, n_ctrl, u_lower=None, u_
     if not scalar_bounds or kind == _lib.DYN_ROCKET:
         factored = False      # factored adjoint kernels: pendulum / cartpole only
     # cost layout: dense [T,B,..] or broadcast (C[n,n] / C[T,n,n]); the generic path
-    # (LinDx kernels + kkt_grads) wants dense tensors
+    # (LinDx kernels + kkt_grads) wants dense tensors.  C_sum / c_sum: the axes the
+    # densification of a C[n,n] / C[T,n,n] added, over which the backward sums the dense
+    # gradient so that it comes back in the shape handed in (as the factored path's does)
     C_in, c_in = C_, c_
     Cb, C_ = cost_layout(C_in.to(dtype), T, B, 2)
     cb, c_ = cost_layout(c_in.to(dtype), T, B, 1)
+    C_sum = c_sum = ()
     if not factored and (Cb or cb):
         C_, c_ = dense_cost(C_in.to(dtype), T, B, 2), dense_cost(c_in.to(dtype), T, B, 1)
+        C_sum = {2: (0, 1), 3: (1,)}.get(C_in.dim(), ())
+        c_sum = {1: (0, 1), 2: (1,)}.get(c_in.dim(), ())
         Cb = cb = 0
     prep = dict(theta=theta, kind=kind, factored=factored, Cb=Cb, cb=cb, C_=C_, c_=c_, x=x, u=u,
-                x_init=x_init, C_in=C_in, c_in=c_in, fused=False)
+                x_init=x_init, C_in=C_in, c_in=c_in, C_sum=C_sum, c_sum=c_sum, fused=False)
     nW = (B + 31) // 32
     fused = (FUSED_BACKWARD and factored and solve_info is not None and n_ctrl == 1
              and getattr(solve_info, "_problem", None) is not None)
@@ -864,8 +869,11 @@ def dilqr_backward(dl_dx, dl_du, x_init, C_, c_, x, u, dxmod, n_state, n_ctrl, u
         dC = dC.sum(1 if Cb == 1 else 0)
     if cb:
         dc = dc.sum(1 if cb == 1 else 0)
+    if prep["C_sum"]:    # generic path on a densified C[n,n] / C[T,n,n]
+        dC = dC.sum(prep["C_sum"])
+    if prep["c_sum"]:
+        dc = dc.sum(prep["c_sum"])
     if tile_reduce:      # the tiling's adjoint on the dense gradients (generic path)
-        dC = dC.reshape(T, B, n, n) if not Cb else dC
         return (dC.diagonal(dim1=-2, dim2=-1).reshape(-1, n).sum(0),
                 dc.reshape(-1, n).sum(0), dtheta)
     return dC, dc, dtheta
