@@ -666,9 +666,16 @@ __global__ void __launch_bounds__(64) adjoint_pass_kernel(const __grid_constant_
     st.issue_bound(stage, t, 0xfu | (first ? rmask : (1u << 7)));
   };
   constexpr bool reduce = REDUCE;
+  // a bulk store needs a 16-byte aligned destination: the slab of step t starts t * B rows in,
+  // so the row stride B * N (N * N) scalars must be a 16-byte multiple too (FP32, N = 6 and an
+  // odd B is not)
   const bool bulk_out = !reduce && (nvalid == kWarp) &&
                         ((((size_t)N * N * sizeof(S) * kWarp) & 15) == 0) &&
                         ((((size_t)N * sizeof(S) * kWarp) & 15) == 0) &&
+                        ((((size_t)p.B * N * N * sizeof(S)) & 15) == 0) &&
+                        ((((size_t)p.B * N * sizeof(S)) & 15) == 0) &&
+                        ((reinterpret_cast<uintptr_t>(p.dC) & 15) == 0) &&
+                        ((reinterpret_cast<uintptr_t>(p.dc) & 15) == 0) &&
                         (p.C_bcast == 0 || p.c_bcast == 0);
   const int gwarp = b0 / kWarp;
   auto warp_sum = [&](S v) -> S {

@@ -84,8 +84,11 @@ costate_tables_kernel(DynParams<S> P, int T, int B, const S* __restrict__ C,
                                cost_src<S>(c, c_bcast, t, B, b0, N), x + o * NS, u + o * NC};
     st.issue(stage, src, CS::kNSeg);
   };
+  // a bulk store needs a 16-byte aligned destination: the slab of step t starts t * B rows in
   const bool bulk_out = !PACKED && (nvalid == kWarp) &&
-                        ((((size_t)N * N * sizeof(S) * kWarp) & 15) == 0);
+                        ((((size_t)N * N * sizeof(S) * kWarp) & 15) == 0) &&
+                        ((((size_t)B * N * N * sizeof(S)) & 15) == 0) &&
+                        ((reinterpret_cast<uintptr_t>(Lam_out) & 15) == 0);
   using LP = LamPack<S, DYN>;
   const int nWp = (B + kWarp - 1) / kWarp;
   S lam[NS];

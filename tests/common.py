@@ -1,10 +1,42 @@
-"""Helpers shared by the tests (problem generators, golden loader)."""
+"""Helpers shared by the tests (problem generators, golden loader, the kernel-family table)."""
+import importlib
 import os
 
 import numpy as np
 import torch
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+# ------------------------------------------------------------------ which kernels serve a solve
+# The family table of test_oracle_matrix.py (written out by hand, not taken from the library's
+# rule): tests assert the family each of their solves ran, so a change of plan fails them.
+LINDX_COMPILED = {(2, 1), (2, 2), (3, 1), (4, 1), (4, 2), (4, 4), (5, 1), (6, 2), (8, 1), (8, 2),
+                  (8, 4), (13, 3), (16, 1), (16, 2), (16, 4)}
+NN_COMPILED = {(3, 1), (4, 2), (5, 1)}
+# compiled LinDx shapes whose Riccati stage (C, c, F, f slabs of a warp, double-buffered) does
+# not fit the 56 KB per-warp budget: every solve of these runs the group sweep
+UNSTAGED = {torch.float64: {(6, 2), (8, 1), (8, 2), (8, 4), (13, 3), (16, 1), (16, 2), (16, 4)},
+            torch.float32: {(8, 4), (13, 3), (16, 1), (16, 2), (16, 4)}}
+
+
+def expected_family(ns, nc, dtype, box_global, nn=False):
+    """The family of a LinDx (or, with ``nn``, NNDynamics) solve whose batch fits the group
+    sweep's capacity."""
+    if nn:
+        return "nn" if (ns, nc) in NN_COMPILED else "nn_rt"
+    if (ns, nc) not in LINDX_COMPILED:
+        return "runtime"
+    if (ns, nc) in UNSTAGED[dtype] or (nc > 1 and box_global):
+        return "group"
+    return "thread"
+
+
+def family(info):
+    """The family a solve ran, from its SolveInfo: runtime, nn, nn_rt, group or thread."""
+    lib = importlib.import_module("differentiable-ilqr_b200._lib")
+    p = info._problem[0]
+    return {lib.DYN_LINDX_RT: "runtime", lib.DYN_NN: "nn", lib.DYN_NN_RT: "nn_rt"}.get(
+        p.dynamics, "group" if p.group_sweep else "thread")
 
 
 def golden(name):

@@ -4,9 +4,9 @@ FP64 and FP32, and results that do not depend on what ran earlier in the shared 
 Which kernels serve a call is not visible in it: `dilqr_lindx_kernels` / `dilqr_nn_kernels`
 and `dilqr_mpc_plan` choose from the shape, the dtype, the bounds, `solo` and the batch.  Every
 GPU case here asserts the family each of its solves ran (`info._problem[0].dynamics` and
-`.group_sweep`, see `family`), so a change of plan fails the test instead of quietly moving
-the coverage elsewhere.  The expected family comes from `expected_family`, a table written out
-by hand, not from the library's rule.
+`.group_sweep`, see `common.family`), so a change of plan fails the test instead of quietly
+moving the coverage elsewhere.  The expected family comes from `common.expected_family`, a
+table written out by hand, not from the library's rule.
 
 Families:
   thread   one thread per problem (csrc/ilqr_kernels.cuh): compiled shapes whose per-warp
@@ -60,7 +60,8 @@ import math
 import pytest
 import torch
 
-from common import env_problem, lindx_problem, rel
+from common import (LINDX_COMPILED, NN_COMPILED, env_problem, expected_family, family,
+                    lindx_problem, rel)
 
 F64, F32 = torch.float64, torch.float32
 STEP_TOL = {F64: 3e-9, F32: 3e-4}
@@ -71,33 +72,6 @@ BOX = 0.5                            # the scalar box [-BOX, BOX]
 
 def _lib():
     return importlib.import_module("differentiable-ilqr_b200._lib")
-
-
-# ------------------------------------------------------------------ which kernels serve a solve
-LINDX_COMPILED = {(2, 1), (2, 2), (3, 1), (4, 1), (4, 2), (4, 4), (5, 1), (6, 2), (8, 1), (8, 2),
-                  (8, 4), (13, 3), (16, 1), (16, 2), (16, 4)}
-NN_COMPILED = {(3, 1), (4, 2), (5, 1)}
-# compiled LinDx shapes whose Riccati stage (C, c, F, f slabs of a warp, double-buffered) does
-# not fit the 56 KB per-warp budget: every solve of these runs the group sweep
-UNSTAGED = {F64: {(6, 2), (8, 1), (8, 2), (8, 4), (13, 3), (16, 1), (16, 2), (16, 4)},
-            F32: {(8, 4), (13, 3), (16, 1), (16, 2), (16, 4)}}
-
-
-def expected_family(ns, nc, dtype, box_global, nn=False):
-    if nn:
-        return "nn" if (ns, nc) in NN_COMPILED else "nn_rt"
-    if (ns, nc) not in LINDX_COMPILED:
-        return "runtime"
-    if (ns, nc) in UNSTAGED[dtype] or (nc > 1 and box_global):
-        return "group"
-    return "thread"
-
-
-def family(info):
-    lib = _lib()
-    p = info._problem[0]
-    return {lib.DYN_LINDX_RT: "runtime", lib.DYN_NN: "nn", lib.DYN_NN_RT: "nn_rt"}.get(
-        p.dynamics, "group" if p.group_sweep else "thread")
 
 
 # ------------------------------------------------------------------ problems
