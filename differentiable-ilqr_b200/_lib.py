@@ -110,6 +110,17 @@ class DilqrAdjoint(C.Structure):
     ]
 
 
+class DilqrKrylov(C.Structure):
+    _fields_ = [
+        ("n_state", C.c_int32), ("n_ctrl", C.c_int32), ("T", C.c_int32), ("n_batch", C.c_int32),
+        ("dtype", C.c_int32), ("restart", C.c_int32), ("max_iter", C.c_int32), ("step", C.c_int32),
+        ("op_negate", C.c_int32), ("reserved0", C.c_int32), ("tol", C.c_double),
+        ("gx", C.c_void_p), ("gu", C.c_void_p), ("w", C.c_void_p), ("op_in", C.c_void_p),
+        ("op_out", C.c_void_p), ("iters", C.c_void_p), ("resid", C.c_void_p),
+        ("control", C.c_void_p), ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t),
+    ]
+
+
 class DilqrWsView(C.Structure):
     _fields_ = [
         ("Kk", C.c_void_p), ("Cpk", C.c_void_p), ("cpk_state", C.c_void_p),
@@ -158,6 +169,12 @@ SYMBOLS = {
     "dilqr_adjoint_factor": (C.c_int, [C.POINTER(DilqrAdjoint), C.c_void_p]),
     "dilqr_adjoint_pass": (C.c_int, [C.POINTER(DilqrAdjoint), C.c_void_p]),
     "dilqr_adjoint_final": (C.c_int, [C.POINTER(DilqrAdjoint), C.c_void_p]),
+    "dilqr_krylov_workspace_bytes": (C.c_size_t, [C.POINTER(DilqrKrylov)]),
+    "dilqr_krylov_cycle_steps": (C.c_int, [C.POINTER(DilqrKrylov), C.c_int]),
+    "dilqr_krylov_start": (C.c_int, [C.POINTER(DilqrKrylov), C.c_void_p]),
+    "dilqr_krylov_arnoldi": (C.c_int, [C.POINTER(DilqrKrylov), C.c_void_p]),
+    "dilqr_krylov_update": (C.c_int, [C.POINTER(DilqrKrylov), C.c_void_p]),
+    "dilqr_krylov_restart": (C.c_int, [C.POINTER(DilqrKrylov), C.c_void_p]),
     "dilqr_tile_cost": (C.c_int, [C.c_int] * 4 + [C.c_void_p] * 5),
     "dilqr_tile_cost_grad_workspace_bytes": (C.c_size_t, [C.c_int]),
     "dilqr_tile_cost_grad": (C.c_int, [C.c_int] * 4 + [C.c_void_p] * 5 + [C.c_size_t, C.c_void_p]),
@@ -212,6 +229,8 @@ KERNELS_PER_CALL = {
     "dilqr_costate_tables": 1, "dilqr_richardson_update": 1, "dilqr_sens_theta": 1,
     "dilqr_adjoint_factor": 1, "dilqr_adjoint_pass": 1, "dilqr_adjoint_final": 1,
     "dilqr_pnqp": 2, "dilqr_pnqp_rt": 2, "dilqr_env_tables": 1, "dilqr_tile_cost": 2, "dilqr_tile_cost_grad": 2,
+    "dilqr_krylov_start": 1, "dilqr_krylov_arnoldi": 1, "dilqr_krylov_update": 1,
+    "dilqr_krylov_restart": 1,
 }
 launch_count = 0     # running total of kernels launched through this binding
 profile = None       # set to a dict {name: [(start_event, end_event), ...]} to time calls

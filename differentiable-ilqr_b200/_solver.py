@@ -687,11 +687,121 @@ def _read_status_raw(ws):
 
 RICHARDSON_WARN = 1e-6     # relative residual above which a fixed-pass solve warns
 
+# GMRES for the adjoint system (solver="gmres"): relative residual |g - A'w| / |g| per problem at
+# which a problem is frozen, by dtype, and the default budget of Arnoldi steps per problem,
+# GMRES_ITER_PER_DIM * T * n: full GMRES reaches the exact solution within T * n steps in exact
+# arithmetic, and the factor leaves room for restarted cycles (restart < T * n) and rounding.
+GMRES_TOL = {torch.float64: 1e-12, torch.float32: 1e-5}
+GMRES_ITER_PER_DIM = 2
+
+
+class GmresResult:
+    """Per-problem outcome of ``_gmres``: iterations (int32 [B]) and final relative residual
+    (float64 [B]) on the host once resolved, the operator applications enqueued, and the
+    solution w [T,B,n] (device)."""
+
+    def __init__(self, tol, max_iter, restart):
+        self.tol, self.max_iter, self.restart = tol, max_iter, restart
+        self.iters = self.resid = self.w = None
+        self.op_calls = 0
+
+    @property
+    def unconverged(self):
+        return int((~(self.resid <= self.tol)).sum())
+
+    @property
+    def worst(self):
+        return float(self.resid.max()) if self.resid.numel() else 0.0
+
+    def fill(self, raw, B):
+        self.resid = torch.frombuffer(bytearray(raw[:8 * B]), dtype=torch.float64)
+        self.iters = torch.frombuffer(bytearray(raw[8 * B:12 * B]), dtype=torch.int32)
+
+    def warn(self):
+        bad = self.unconverged
+        if bad:
+            import warnings
+            warnings.warn("DiLQR backward: GMRES left %d of %d problems above the relative residual "
+                          "%.1e within %d iterations (worst %.2e); their gradient is approximate -- "
+                          "raise gmres_max_iter or gmres_restart"
+                          % (bad, self.resid.numel(), self.tol, self.max_iter, self.worst))
+
+
+def _gmres(op, op_in, op_out, negate, gx, gu, T, B, n_state, n_ctrl, restart, tol, max_iter,
+           deferred=None):
+    """Restarted GMRES(restart) for A'w = g per problem (include/dilqr.h, DilqrKrylov): returns
+    (w[T,B,n], GmresResult).  ``op()`` applies M': reads op_in, writes op_out.  Immediate mode
+    reads the count of problems still iterating once per cycle and stops when it is 0;
+    ``deferred`` enqueues the whole budget with no host read (frozen problems do not change,
+    so both give the same bits) and reads the per-problem status when the caller resolves it."""
+    L = _lib.lib()
+    dtype, dev = gu.dtype, gu.device
+    n = n_state + n_ctrl
+    k = _lib.DilqrKrylov()
+    k.n_state, k.n_ctrl, k.T, k.n_batch, k.dtype = n_state, n_ctrl, T, B, _DT[dtype]
+    k.restart = max(1, min(int(restart), T * n))
+    k.max_iter = int(max_iter)
+    k.op_negate = 1 if negate else 0
+    k.tol = float(tol)
+    w = torch.empty(T, B, n, dtype=dtype, device=dev)
+    status = torch.empty(12 * B, dtype=torch.uint8, device=dev)   # resid f64 [B] | iters i32 [B]
+    ctl = torch.zeros(2, dtype=torch.int32, device=dev)
+    k.gx, k.gu, k.w = _ptr(gx), _ptr(gu), _ptr(w)
+    k.op_in, k.op_out = _ptr(op_in), _ptr(op_out)
+    k.resid = C.c_void_p(status.data_ptr())
+    k.iters = C.c_void_p(status.data_ptr() + 8 * B)
+    k.control = _ptr(ctl)
+    need = L.dilqr_krylov_workspace_bytes(C.byref(k))
+    if need == 0:
+        raise _lib.DilqrLibraryError("GMRES: invalid sizes (restart %d, max_iter %d)"
+                                     % (k.restart, k.max_iter))
+    ws = torch.empty(need, dtype=torch.uint8, device=dev)
+    k.workspace, k.workspace_bytes = _ptr(ws), need
+    res = GmresResult(k.tol, k.max_iter, k.restart)
+    res.w = w
+    st = _stream()
+
+    def apply():
+        op()
+        res.op_calls += 1
+
+    _lib.call("dilqr_krylov_start", C.byref(k), st)
+    cycle = 0
+    steps = L.dilqr_krylov_cycle_steps(C.byref(k), 0)
+    if steps > 0:
+        apply()
+    while steps > 0:
+        if deferred is None and int(ctl[0]) == 0:     # every problem frozen
+            break
+        for j in range(steps):
+            k.step = j
+            _lib.call("dilqr_krylov_arnoldi", C.byref(k), st)
+            if j < steps - 1:
+                apply()
+        _lib.call("dilqr_krylov_update", C.byref(k), st)
+        apply()
+        _lib.call("dilqr_krylov_restart", C.byref(k), st)
+        cycle += 1
+        steps = L.dilqr_krylov_cycle_steps(C.byref(k), cycle)
+        if steps > 0:
+            apply()
+    if deferred is not None:
+        def check(raw, res=res, B=B):
+            res.fill(raw, B)
+            res.warn()
+            return None
+        deferred.add(status, check)
+    else:
+        res.fill(status.cpu().numpy().tobytes(), B)
+        res.warn()
+    return w, res
+
 
 @_on_device_of("x_init", 2)
 def dilqr_backward(dl_dx, dl_du, x_init, C_, c_, x, u, dxmod, n_state, n_ctrl, u_lower=None,
                    u_upper=None, n_passes=8, tol=None, back_eps=1e-7, solo=False, stats=None,
-                   theta_host=None, factored=True, prep=None, tile_reduce=False, deferred=None):
+                   theta_host=None, factored=True, prep=None, tile_reduce=False, deferred=None,
+                   solver="richardson", gmres_restart=64, gmres_tol=None, gmres_max_iter=None):
     """DiLQR implicit gradient (lqr_step_explicit.py:652-712 + fix_point_equ
     458-598) in matrix-free form (SURVEY Appendix C; derivation in
     csrc/dilqr_backward.cuh).  Returns (dC, dc, dtheta[B, n_theta]); with
@@ -713,7 +823,22 @@ def dilqr_backward(dl_dx, dl_du, x_init, C_, c_, x, u, dxmod, n_state, n_ctrl, u
     recomputed with the generic line-searching kernels (``factored=False``).
 
     ``prep``: the gradient-independent part (``dilqr_prepare``) if the forward pass
-    already enqueued it."""
+    already enqueued it.
+
+    ``solver="gmres"`` solves A'w = g by restarted GMRES(``gmres_restart``, clipped to T n)
+    per problem instead (``_gmres``), to the relative residual ``gmres_tol`` (None:
+    ``GMRES_TOL`` of the dtype) within ``gmres_max_iter`` Arnoldi steps (None:
+    ``GMRES_ITER_PER_DIM`` T n); ``n_passes`` / ``tol`` are then unused.  It returns the
+    reference's dense solution where Richardson iteration diverges (rho(M) >= 1), at a
+    data-dependent number of adjoint solves and (restart + 1) T B n scalars of basis.  A
+    problem that misses the tolerance raises a warning.  When the reference's line search
+    would shorten an adjoint step the adjoint map is not linear and no Krylov method applies:
+    that raises ``DilqrLibraryError``."""
+    if solver not in ("richardson", "gmres"):
+        raise ValueError("solver must be 'richardson' or 'gmres', got %r" % (solver,))
+    gmres = solver == "gmres"
+    gm_opts = dict(solver=solver, gmres_restart=gmres_restart, gmres_tol=gmres_tol,
+                   gmres_max_iter=gmres_max_iter)
     if prep is None:
         prep = dilqr_prepare(x_init, C_, c_, x, u, dxmod, n_state, n_ctrl, u_lower, u_upper,
                              solo, theta_host, factored)
@@ -731,7 +856,7 @@ def dilqr_backward(dl_dx, dl_du, x_init, C_, c_, x, u, dxmod, n_state, n_ctrl, u
                              solo, theta_host, factored)
         return dilqr_backward(dl_dx, dl_du, x_init, C_, c_, x, u, dxmod, n_state, n_ctrl,
                               u_lower, u_upper, n_passes, tol, back_eps, solo, stats, theta_host,
-                              factored, prep, tile_reduce, deferred)
+                              factored, prep, tile_reduce, deferred, **gm_opts)
     if dl_du is None:
         dl_du = torch.zeros(T, B, n_ctrl, dtype=dtype, device=dev)
     gu = _aligned(dl_du.contiguous())
@@ -755,7 +880,27 @@ def dilqr_backward(dl_dx, dl_du, x_init, C_, c_, x, u, dxmod, n_state, n_ctrl, u
         r = resid.cpu()
         return float(r[0]) / (float(r[1]) + 1e-300)
 
-    if factored:
+    krylov = None
+    if gmres:
+        gm_tol = GMRES_TOL[dtype] if gmres_tol is None else float(gmres_tol)
+        gm_iter = GMRES_ITER_PER_DIM * T * n if gmres_max_iter is None else int(gmres_max_iter)
+    if factored and gmres:
+        a = prep["a"]
+        st = _stream()
+        # M'v: one adjoint pass with g = 0, in place on the operator buffer
+        opbuf = torch.empty(T, B, n, dtype=dtype, device=dev)
+        zu = torch.zeros(T, B, n_ctrl, dtype=dtype, device=dev)
+
+        def op():
+            a.gx, a.gu, a.w = None, _ptr(zu), _ptr(opbuf)
+            a.first_pass, a.want_resid = 0, 0
+            _lib.call("dilqr_adjoint_pass", C.byref(a), st)
+
+        w, krylov = _gmres(op, opbuf, opbuf, False, gx, gu, T, B, n_state, n_ctrl, gmres_restart,
+                           gm_tol, gm_iter, deferred)
+        a.gx, a.gu, a.w = _ptr(gx), _ptr(gu), _ptr(w)
+        a.first_pass = 0
+    elif factored:
         a = prep["a"]
         w = torch.empty(T, B, n, dtype=dtype, device=dev) if n_passes > 0 else None
         a.gx, a.gu, a.w = _ptr(gx), _ptr(gu), _ptr(w)
@@ -773,6 +918,7 @@ def dilqr_backward(dl_dx, dl_du, x_init, C_, c_, x, u, dxmod, n_state, n_ctrl, u
                 if rel <= tol:
                     break
         a.first_pass = 1 if passes == 0 else 0
+    if factored:
         if fused:
             df = torch.empty(T - 1, nwarp, n_state, 32, dtype=dtype, device=dev)
             a.df_blk, a.df, a.dx_out, a.du_out = _ptr(df), None, None, None
@@ -808,7 +954,26 @@ def dilqr_backward(dl_dx, dl_du, x_init, C_, c_, x, u, dxmod, n_state, n_ctrl, u
                              eps=back_eps, gain_solve=_lib.GAIN_CHOL_REG, verbose=-1,
                              sync=False)[:2]
 
-        for _ in range(n_passes):
+        if gmres:
+            # M'v: the adjoint solve on cost (C, -v), then w <- 0 - Lam dtau
+            vneg = torch.empty(T, B, n, dtype=dtype, device=dev)
+            mv = torch.empty(T, B, n, dtype=dtype, device=dev)
+            g0 = torch.zeros(T, B, n, dtype=dtype, device=dev)
+            scratch = torch.empty(T, B, n, dtype=dtype, device=dev)
+            res0 = torch.zeros(3, dtype=torch.float64, device=dev)
+
+            def op():
+                dxo, duo = solve_mpc(zero, C_d, vneg, lin, n_state, n_ctrl, T, u_zero_I=I,
+                                     lqr_iter=1, eps=back_eps, gain_solve=_lib.GAIN_CHOL_REG,
+                                     verbose=-1, sync=False)[:2]
+                _lib.call("dilqr_richardson_update", _DT[dtype], n_state, n_ctrl, T, B, _ptr(g0),
+                          _ptr(Lam), _ptr(dxo), _ptr(duo), _ptr(mv), _ptr(scratch), _ptr(res0),
+                          _stream())
+
+            w, krylov = _gmres(op, vneg, mv, True, gx, gu, T, B, n_state, n_ctrl, gmres_restart,
+                               gm_tol, gm_iter, deferred)
+            negw = -w
+        for _ in range(0 if gmres else n_passes):
             dxa, dua = adjoint()
             _lib.call("dilqr_richardson_update", _DT[dtype], n_state, n_ctrl, T, B, _ptr(g),
                       _ptr(Lam), _ptr(dxa), _ptr(dua), _ptr(w), _ptr(negw), _ptr(resid), _stream())
@@ -838,6 +1003,10 @@ def dilqr_backward(dl_dx, dl_du, x_init, C_, c_, x, u, dxmod, n_state, n_ctrl, u
             r = dmax / (wmax + 1e-300)
             if stats is not None and passes and stats.get("resid") is None:
                 stats["resid"] = r
+            if n_rej and gmres:
+                return ("the reference's line search would shorten an adjoint step (a non-convex "
+                        "adjoint QP): the adjoint map is not linear, so GMRES cannot solve the "
+                        "system the reference assembles -- use solver='richardson'")
             if n_rej:
                 return "the reference's line search would reject an adjoint step"
             if passes and tol is None and r > RICHARDSON_WARN:
@@ -850,7 +1019,10 @@ def dilqr_backward(dl_dx, dl_du, x_init, C_, c_, x, u, dxmod, n_state, n_ctrl, u
             deferred.add(resid.view(torch.uint8), check)
         else:
             # one sync at the end: did the reference's line search reject any adjoint step?
-            if check(bytes(resid.view(torch.uint8).cpu().numpy().tobytes())):
+            why = check(bytes(resid.view(torch.uint8).cpu().numpy().tobytes()))
+            if why and gmres:
+                raise _lib.DilqrLibraryError("DiLQR backward: " + why)
+            if why:
                 return dilqr_backward(dl_dx, dl_du, x_init, prep["C_in"], prep["c_in"], x, u, dxmod,
                                       n_state, n_ctrl, u_lower, u_upper, n_passes, tol, back_eps,
                                       solo, stats, theta_host=theta_host, factored=False,
@@ -862,6 +1034,11 @@ def dilqr_backward(dl_dx, dl_du, x_init, C_, c_, x, u, dxmod, n_state, n_ctrl, u
             stats["resid"] = rel
         stats["factored"] = factored
         stats["fused"] = fused
+        stats["solver"] = solver
+        if krylov is not None:
+            # the per-problem status: filled now (immediate) or when the step is resolved
+            stats["gmres"] = krylov
+            stats["passes"] = krylov.op_calls
     if reduce_in_kernel:
         r = red.sum(0)
         return r[:n], r[n:], dtheta

@@ -12,6 +12,7 @@
 #include "misc_kernels.cuh"
 #include "dilqr_backward.cuh"
 #include "adjoint_kernels.cuh"
+#include "krylov_kernels.cuh"
 #include "group_kernels.cuh"
 #include "rt_kernels.cuh"
 #if !defined(DILQR_GROUP) || DILQR_GROUP == 0
@@ -1066,6 +1067,100 @@ int DILQR_SUFFIX(env_tables)(int dynamics, const double* dp, int n, const void* 
   if (dynamics == DYN_CARTPOLE) return launch_tables<DYN_CARTPOLE>(dp, n, x, u, out, st);
   if (dynamics == DYN_ROCKET) return launch_tables<DYN_ROCKET>(dp, n, x, u, out, st);
   return DILQR_EUNSUPPORTED;
+}
+
+// ------------------------------------------------- GMRES for the adjoint system
+struct KrylovLayout {
+  size_t V, H, Y, R, gam, cs, sn, gnorm, klen, flags, total;
+};
+
+static bool krylov_dims_ok(const DilqrKrylov* k) {
+  if (!k || k->T < 1 || k->n_batch <= 0 || k->n_state <= 0 || k->n_ctrl <= 0) return false;
+  const long long L = (long long)k->T * (k->n_state + k->n_ctrl);
+  return k->restart >= 1 && k->restart <= L && k->max_iter >= 1;
+}
+
+static KrylovLayout krylov_layout(const DilqrKrylov* k) {
+  KrylovLayout w;
+  const size_t B = (size_t)k->n_batch, m = (size_t)k->restart;
+  const size_t vec = (size_t)k->T * B * (k->n_state + k->n_ctrl) * sizeof(Scalar);
+  size_t off = 0;
+  auto take = [&](size_t bytes) {
+    size_t o = off;
+    off = align_up(off + bytes, 256);
+    return o;
+  };
+  w.V = take((m + 1) * vec);
+  w.H = take((m + 1) * B * sizeof(double));
+  w.Y = take((m + 1) * B * sizeof(double));
+  w.R = take(m * (m + 1) / 2 * B * sizeof(double));
+  w.gam = take((m + 1) * B * sizeof(double));
+  w.cs = take(m * B * sizeof(double));
+  w.sn = take(m * B * sizeof(double));
+  w.gnorm = take(B * sizeof(double));
+  w.klen = take(B * sizeof(int));
+  w.flags = take(B * sizeof(int));
+  w.total = off;
+  return w;
+}
+
+size_t DILQR_SUFFIX(krylov_workspace_bytes)(const DilqrKrylov* k) {
+  return krylov_dims_ok(k) ? krylov_layout(k).total : 0;
+}
+
+int DILQR_SUFFIX(krylov_run)(const DilqrKrylov* k, int what, void* stream) {
+  using S = Scalar;
+  if (!krylov_dims_ok(k) || !k->gu || !k->w || !k->op_in || !k->op_out || !k->iters || !k->resid ||
+      !k->control || !k->workspace || !(k->tol >= 0.0))
+    return DILQR_EINVAL;
+  if (what == 1 && (k->step < 0 || k->step >= k->restart)) return DILQR_EINVAL;
+  const KrylovLayout L = krylov_layout(k);
+  if (k->workspace_bytes < L.total) return DILQR_EWORKSPACE;
+  char* ws = static_cast<char*>(k->workspace);
+  KrylovParams<S> p;
+  memset(&p, 0, sizeof(p));
+  p.T = k->T;
+  p.B = k->n_batch;
+  p.n = k->n_state + k->n_ctrl;
+  p.ns = k->n_state;
+  p.m = k->restart;
+  p.j = k->step;
+  p.tol = k->tol;
+  p.negate = k->op_negate ? 1 : 0;
+  p.gx = static_cast<const S*>(k->gx);
+  p.gu = static_cast<const S*>(k->gu);
+  p.w = static_cast<S*>(k->w);
+  p.opin = static_cast<S*>(k->op_in);
+  p.opout = static_cast<const S*>(k->op_out);
+  p.V = reinterpret_cast<S*>(ws + L.V);
+  p.H = reinterpret_cast<double*>(ws + L.H);
+  p.Y = reinterpret_cast<double*>(ws + L.Y);
+  p.R = reinterpret_cast<double*>(ws + L.R);
+  p.gam = reinterpret_cast<double*>(ws + L.gam);
+  p.cs = reinterpret_cast<double*>(ws + L.cs);
+  p.sn = reinterpret_cast<double*>(ws + L.sn);
+  p.gnorm = reinterpret_cast<double*>(ws + L.gnorm);
+  p.klen = reinterpret_cast<int*>(ws + L.klen);
+  p.flags = reinterpret_cast<int*>(ws + L.flags);
+  p.iters = k->iters;
+  p.resid = k->resid;
+  p.ctl = k->control;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int grid = (p.B + 127) / 128;
+  if (what == 0) {
+    cudaMemsetAsync(p.ctl, 0, sizeof(unsigned), st);
+    krylov_start_kernel<S><<<grid, 128, 0, st>>>(p);
+  } else if (what == 1) {
+    krylov_arnoldi_kernel<S><<<grid, 128, 0, st>>>(p);
+  } else if (what == 2) {
+    krylov_update_kernel<S><<<grid, 128, 0, st>>>(p);
+  } else {
+    // count the problems still iterating into ctl[1], then publish it as ctl[0]
+    cudaMemsetAsync(p.ctl + 1, 0, sizeof(unsigned), st);
+    krylov_restart_kernel<S><<<grid, 128, 0, st>>>(p);
+    cudaMemcpyAsync(p.ctl, p.ctl + 1, sizeof(unsigned), cudaMemcpyDeviceToDevice, st);
+  }
+  return cudaGetLastError() == cudaSuccess ? DILQR_OK : DILQR_ECUDA;
 }
 
 #endif  // DILQR_GROUP == 0

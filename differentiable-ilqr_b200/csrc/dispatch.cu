@@ -40,7 +40,9 @@ namespace dilqr {
   int sens_theta_adjoint_##sfx(int, const double*, int, int, const void*, const void*,    \
                                const void*, const void*, const void*, const void*, const void*, \
                                void*, void*);                                             \
-  int adjoint_run_##sfx(const DilqrAdjoint*, int, void*);
+  int adjoint_run_##sfx(const DilqrAdjoint*, int, void*);                                \
+  size_t krylov_workspace_bytes_##sfx(const DilqrKrylov*);                                \
+  int krylov_run_##sfx(const DilqrKrylov*, int, void*);
 DECL_G(f32_g0) DECL_G(f32_g1) DECL_G(f32_g2) DECL_G(f32_g3)
 DECL_G(f64_g0) DECL_G(f64_g1) DECL_G(f64_g2) DECL_G(f64_g3)
 DECL_0(f32_g0) DECL_0(f64_g0)
@@ -244,6 +246,33 @@ int dilqr_adjoint_pass(const DilqrAdjoint* a, void* st) {
 int dilqr_adjoint_final(const DilqrAdjoint* a, void* st) {
   if (!a) return DILQR_EINVAL;
   return ROUTE(a->dtype, dilqr::adjoint_run_f32_g0(a, 2, st), dilqr::adjoint_run_f64_g0(a, 2, st));
+}
+
+size_t dilqr_krylov_workspace_bytes(const DilqrKrylov* k) {
+  if (!k) return 0;
+  return k->dtype == DILQR_F32 ? dilqr::krylov_workspace_bytes_f32_g0(k)
+       : k->dtype == DILQR_F64 ? dilqr::krylov_workspace_bytes_f64_g0(k) : 0;
+}
+int dilqr_krylov_cycle_steps(const DilqrKrylov* k, int cycle) {
+  if (!k || k->restart < 1 || k->max_iter < 1 || cycle < 0) return DILQR_EINVAL;
+  const long long left = (long long)k->max_iter - (long long)cycle * k->restart;
+  return left <= 0 ? 0 : (int)(left < k->restart ? left : k->restart);
+}
+int dilqr_krylov_start(const DilqrKrylov* k, void* st) {
+  if (!k) return DILQR_EINVAL;
+  return ROUTE(k->dtype, dilqr::krylov_run_f32_g0(k, 0, st), dilqr::krylov_run_f64_g0(k, 0, st));
+}
+int dilqr_krylov_arnoldi(const DilqrKrylov* k, void* st) {
+  if (!k) return DILQR_EINVAL;
+  return ROUTE(k->dtype, dilqr::krylov_run_f32_g0(k, 1, st), dilqr::krylov_run_f64_g0(k, 1, st));
+}
+int dilqr_krylov_update(const DilqrKrylov* k, void* st) {
+  if (!k) return DILQR_EINVAL;
+  return ROUTE(k->dtype, dilqr::krylov_run_f32_g0(k, 2, st), dilqr::krylov_run_f64_g0(k, 2, st));
+}
+int dilqr_krylov_restart(const DilqrKrylov* k, void* st) {
+  if (!k) return DILQR_EINVAL;
+  return ROUTE(k->dtype, dilqr::krylov_run_f32_g0(k, 3, st), dilqr::krylov_run_f64_g0(k, 3, st));
 }
 
 }  // extern "C"

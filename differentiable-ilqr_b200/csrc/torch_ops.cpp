@@ -14,6 +14,7 @@
 #include <c10/cuda/CUDAStream.h>
 #include <torch/library.h>
 
+#include <algorithm>
 #include <cstring>
 #include <tuple>
 #include <vector>
@@ -264,7 +265,11 @@ std::tuple<Tensor, Tensor, Tensor> dilqr_backward(
     const optional<Tensor>& gx, const Tensor& gu, const Tensor& x_init, const Tensor& C,
     const Tensor& c, const Tensor& x, const Tensor& u, const Tensor& theta, int64_t dynamics,
     optional<double> u_lower, optional<double> u_upper, int64_t n_passes, int64_t max_ls,
-    double decay) {
+    double decay, c10::string_view adjoint_solver, int64_t gmres_restart,
+    optional<double> gmres_tol, optional<int64_t> gmres_max_iter) {
+  const bool gmres = adjoint_solver == "gmres";
+  TORCH_CHECK(gmres || adjoint_solver == "richardson",
+              "dilqr::dilqr_backward: adjoint_solver must be 'richardson' or 'gmres'");
   c10::cuda::CUDAGuard guard(x.device());
   cudaStream_t st = c10::cuda::getCurrentCUDAStream();
   TORCH_CHECK(dynamics == DILQR_DYN_PENDULUM || dynamics == DILQR_DYN_CARTPOLE,
@@ -335,11 +340,66 @@ std::tuple<Tensor, Tensor, Tensor> dilqr_backward(
   a.workspace = aws.data_ptr();
   a.workspace_bytes = (size_t)aws.numel();
   check_rc(dilqr_adjoint_factor(&a, st), "dilqr_adjoint_factor");
-  for (int64_t i = 0; i < n_passes; ++i) {
-    a.first_pass = i == 0;
-    check_rc(dilqr_adjoint_pass(&a, st), "dilqr_adjoint_pass");
+  if (gmres) {
+    // restarted GMRES on A'w = g; M'v is one adjoint pass with g = 0, in place on opbuf
+    Tensor opbuf = at::empty({T, B, n}, opt), zu = at::zeros({T, B, nc}, opt);
+    Tensor status = at::empty({12 * B}, opt.dtype(at::kByte));   // resid f64 [B] | iters i32 [B]
+    Tensor ctl = at::zeros({2}, opt.dtype(at::kInt));
+    DilqrKrylov k;
+    std::memset(&k, 0, sizeof(k));
+    k.n_state = (int)ns; k.n_ctrl = (int)nc; k.T = (int)T; k.n_batch = (int)B; k.dtype = dt;
+    k.restart = (int)std::max<int64_t>(1, std::min<int64_t>(gmres_restart, T * n));
+    k.max_iter = (int)(gmres_max_iter.has_value() ? *gmres_max_iter : 2 * T * n);
+    k.tol = gmres_tol.has_value() ? *gmres_tol : (dt == DILQR_F64 ? 1e-12 : 1e-5);
+    k.gx = a.gx; k.gu = a.gu; k.w = w.data_ptr();
+    k.op_in = opbuf.data_ptr(); k.op_out = opbuf.data_ptr();
+    char* sb = static_cast<char*>(status.data_ptr());
+    k.resid = reinterpret_cast<double*>(sb);
+    k.iters = reinterpret_cast<int32_t*>(sb + 8 * B);
+    k.control = reinterpret_cast<uint32_t*>(ctl.data_ptr());
+    const size_t need = dilqr_krylov_workspace_bytes(&k);
+    TORCH_CHECK(need > 0, "dilqr::dilqr_backward: invalid GMRES sizes");
+    Tensor kws = at::empty({(int64_t)need}, opt.dtype(at::kByte));
+    k.workspace = kws.data_ptr(); k.workspace_bytes = need;
+    DilqrAdjoint op = a;
+    op.gx = nullptr; op.gu = zu.data_ptr(); op.w = opbuf.data_ptr();
+    op.first_pass = 0; op.want_resid = 0;
+    auto apply = [&]() { check_rc(dilqr_adjoint_pass(&op, st), "dilqr_adjoint_pass"); };
+    check_rc(dilqr_krylov_start(&k, st), "dilqr_krylov_start");
+    int steps = dilqr_krylov_cycle_steps(&k, 0);
+    check_rc(steps < 0 ? steps : 0, "dilqr_krylov_cycle_steps");
+    if (steps > 0) apply();
+    for (int cycle = 0; steps > 0;) {
+      if (ctl[0].item<int>() == 0) break;     // every problem frozen (one host read per cycle)
+      for (int j = 0; j < steps; ++j) {
+        k.step = j;
+        check_rc(dilqr_krylov_arnoldi(&k, st), "dilqr_krylov_arnoldi");
+        if (j < steps - 1) apply();
+      }
+      check_rc(dilqr_krylov_update(&k, st), "dilqr_krylov_update");
+      apply();
+      check_rc(dilqr_krylov_restart(&k, st), "dilqr_krylov_restart");
+      steps = dilqr_krylov_cycle_steps(&k, ++cycle);
+      if (steps > 0) apply();
+    }
+    Tensor rh = status.narrow(0, 0, 8 * B).view(at::kDouble).cpu();
+    const double* r = rh.data_ptr<double>();
+    int64_t bad = 0;
+    double worst = 0.0;
+    for (int64_t b = 0; b < B; ++b) {
+      if (!(r[b] <= k.tol)) ++bad;
+      worst = std::max(worst, r[b]);
+    }
+    if (bad)
+      TORCH_WARN("dilqr::dilqr_backward: GMRES left ", bad, " of ", B, " problems above the relative "
+                 "residual ", k.tol, " within ", k.max_iter, " iterations (worst ", worst, ")");
+  } else {
+    for (int64_t i = 0; i < n_passes; ++i) {
+      a.first_pass = i == 0;
+      check_rc(dilqr_adjoint_pass(&a, st), "dilqr_adjoint_pass");
+    }
   }
-  a.first_pass = n_passes == 0;
+  a.first_pass = !gmres && n_passes == 0;
   const std::vector<int64_t> shC = Cb == 0 ? std::vector<int64_t>{T, B, n, n}
                                  : Cb == 1 ? std::vector<int64_t>{T, nW, n, n} : std::vector<int64_t>{nW, n, n};
   const std::vector<int64_t> shc = cb == 0 ? std::vector<int64_t>{T, B, n}
@@ -358,6 +418,9 @@ std::tuple<Tensor, Tensor, Tensor> dilqr_backward(
   Tensor rh = resid.cpu();
   int64_t n_rej;
   std::memcpy(&n_rej, rh.data_ptr<double>() + 2, sizeof(n_rej));
+  TORCH_CHECK(n_rej == 0 || !gmres, "dilqr::dilqr_backward: the reference's line search would shorten "
+              "an adjoint step for ", n_rej, " problem(s) (non-convex adjoint QP): the adjoint map is "
+              "not linear, so GMRES cannot solve the system the reference assembles");
   TORCH_CHECK(n_rej == 0, "dilqr::dilqr_backward: the reference's line search would reject an adjoint "
                           "step for ", n_rej, " problem(s) (non-convex model); use the Python "
                           "mpc_explicit.MPC, which falls back to the line-searching kernels");
@@ -375,7 +438,8 @@ TORCH_LIBRARY(dilqr, m) {
         "int solo) -> (Tensor, Tensor, Tensor, Tensor, Tensor)");
   m.def("dilqr_backward(Tensor? gx, Tensor gu, Tensor x_init, Tensor C, Tensor c, Tensor x, Tensor u, "
         "Tensor theta, int dynamics, float? u_lower, float? u_upper, int n_passes, "
-        "int max_linesearch_iter, float linesearch_decay) -> (Tensor, Tensor, Tensor)");
+        "int max_linesearch_iter, float linesearch_decay, str adjoint_solver=\"richardson\", "
+        "int gmres_restart=64, float? gmres_tol=None, int? gmres_max_iter=None) -> (Tensor, Tensor, Tensor)");
   m.def("lqr_kkt_backward(Tensor? gx, Tensor gu, Tensor x_init, Tensor C, Tensor c, Tensor F, Tensor x, "
         "Tensor u, float? u_lower, float? u_upper) -> (Tensor, Tensor, Tensor, Tensor, Tensor)");
 }

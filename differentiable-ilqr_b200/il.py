@@ -64,7 +64,10 @@ def tile_cost(q, p, T, B):
 
 class ImitationStep:
     def __init__(self, dx_cls, T, lqr_iter, dtype, device, n_richardson=4, richardson_tol=None,
-                 group=None, tile=True, detach_unconverged=False):
+                 group=None, tile=True, detach_unconverged=False, adjoint_solver="richardson",
+                 gmres_restart=64, gmres_tol=None, gmres_max_iter=None):
+        # adjoint_solver / gmres_*: the solver of the backward's adjoint system, as in
+        # mpc_explicit.MPC (the GMRES status is read in the step's one deferred host sync)
         # tile=True: materialise Q,p as [T,B,n,n] / [T,B,n] exactly like il_env.py:159-162;
         # tile=False: hand MPC the [n,n] / [n] tensors (mpc.py:205-219 broadcasts them)
         self.tile = tile
@@ -78,11 +81,15 @@ class ImitationStep:
             verbose=-1, exit_unconverged=False, detach_unconverged=detach_unconverged,
             linesearch_decay=proto.linesearch_decay,
             max_linesearch_iter=proto.max_linesearch_iter, eps=proto.mpc_eps,
-            richardson_passes=n_richardson, richardson_tol=richardson_tol)
+            richardson_passes=n_richardson, richardson_tol=richardson_tol,
+            adjoint_solver=adjoint_solver, gmres_restart=gmres_restart, gmres_tol=gmres_tol,
+            gmres_max_iter=gmres_max_iter)
         self.group = group
         self.retries = 0
         self.redone = 0           # steps repeated because a deferred check failed
-        self.backward_name = "DiLQR implicit (%d Richardson passes)" % n_richardson
+        self.backward_name = ("DiLQR implicit (%d Richardson passes)" % n_richardson
+                              if adjoint_solver == "richardson" else
+                              "DiLQR implicit (GMRES(%d))" % gmres_restart)
         self.d2h_bytes = 0
         self.defer = True         # one host sync per step (see _solver.Deferred)
         self._out_host = None
@@ -212,7 +219,8 @@ class ImitationLearner:
 
     def __init__(self, dx_cls, theta_init, T, lqr_iter=100, dtype=torch.float64,
                  device=None, lr=1e-2, alpha=0.5, richardson_passes=30, richardson_tol=1e-10,
-                 group=None, learn_dx=True, learn_cost=False):
+                 group=None, learn_dx=True, learn_cost=False, adjoint_solver="richardson",
+                 gmres_restart=64, gmres_tol=None, gmres_max_iter=None):
         self.dx_cls, self.T = dx_cls, T
         self.dtype, self.device, self.group = dtype, device, group
         self.learn_dx, self.learn_cost = learn_dx, learn_cost
@@ -231,7 +239,9 @@ class ImitationLearner:
             verbose=-1, exit_unconverged=False, detach_unconverged=True,
             linesearch_decay=proto.linesearch_decay,
             max_linesearch_iter=proto.max_linesearch_iter, eps=proto.mpc_eps,
-            richardson_passes=richardson_passes, richardson_tol=richardson_tol)
+            richardson_passes=richardson_passes, richardson_tol=richardson_tol,
+            adjoint_solver=adjoint_solver, gmres_restart=gmres_restart, gmres_tol=gmres_tol,
+            gmres_max_iter=gmres_max_iter)
         self.warm = None
 
     def cost(self):

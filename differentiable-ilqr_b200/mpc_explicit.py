@@ -84,7 +84,8 @@ class _MPCExplicitFn(Function):
             mod.n_ctrl, mod.u_lower, mod.u_upper, n_passes=mod.richardson_passes,
             tol=mod.richardson_tol, back_eps=mod.back_eps, solo=mod.solo, stats=stats,
             theta_host=ctx.theta_host, prep=ctx.prep, tile_reduce=ctx.tiled,
-            deferred=ctx.deferred)
+            deferred=ctx.deferred, solver=mod.adjoint_solver, gmres_restart=mod.gmres_restart,
+            gmres_tol=mod.gmres_tol, gmres_max_iter=mod.gmres_max_iter)
         ctx.prep = None
         mod.last_backward = stats
         # dC / dc come back in the layout of the cost tensors handed in (dense, or already
@@ -99,12 +100,21 @@ class _MPCExplicitFn(Function):
 
 
 class MPC(_BaseMPC):
-    """Arguments as the reference (mpc_explicit.py:122-143) plus two knobs of the
-    matrix-free fixed-point solve: ``richardson_passes`` (max adjoint-LQR passes)
-    and ``richardson_tol`` (relative stop tolerance; None = fixed pass count)."""
+    """Arguments as the reference (mpc_explicit.py:122-143) plus the solver of the
+    matrix-free fixed-point system A'w = g of the backward:
+
+    - ``adjoint_solver="richardson"`` (default): ``richardson_passes`` (max adjoint-LQR
+      passes) and ``richardson_tol`` (relative stop tolerance; None = fixed pass count).
+      Converges only where the iteration matrix M = I - A has rho(M) < 1 (a converged
+      iLQR fixed point).
+    - ``adjoint_solver="gmres"``: restarted GMRES per problem, the reference's dense solve
+      wherever A is nonsingular; ``gmres_restart`` basis vectors per cycle (clipped to T n),
+      ``gmres_tol`` relative residual (None: 1e-12 in FP64, 1e-5 in FP32), ``gmres_max_iter``
+      Arnoldi steps (None: 2 T n).  See ``_solver.dilqr_backward``."""
 
     def __init__(self, *args, richardson_passes=30, richardson_tol=1e-14,
-                 prepare_in_forward=True, **kw):
+                 prepare_in_forward=True, adjoint_solver="richardson", gmres_restart=64,
+                 gmres_tol=None, gmres_max_iter=None, **kw):
         super().__init__(*args, **kw)
         self.prepare_in_forward = prepare_in_forward
         # defer_checks: postpone every validation read of a step (pnqp trace, stop-rule
@@ -115,6 +125,13 @@ class MPC(_BaseMPC):
         self.deferred = None
         self.richardson_passes = richardson_passes
         self.richardson_tol = richardson_tol
+        if adjoint_solver not in ("richardson", "gmres"):
+            raise ValueError("adjoint_solver must be 'richardson' or 'gmres', got %r"
+                             % (adjoint_solver,))
+        self.adjoint_solver = adjoint_solver
+        self.gmres_restart = gmres_restart
+        self.gmres_tol = gmres_tol
+        self.gmres_max_iter = gmres_max_iter
         self.last_backward = None
 
     def forward(self, x_init, cost, dx):

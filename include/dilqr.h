@@ -418,6 +418,55 @@ int dilqr_adjoint_pass(const DilqrAdjoint* a, void* stream);
 /* Adjoint solve with r = w, then costates and dC, dc, df (lqr_step.py:346-402). */
 int dilqr_adjoint_final(const DilqrAdjoint* a, void* stream);
 
+/* ---- GMRES for the adjoint system A' w = g of the DiLQR backward ------------------------
+ * Restarted GMRES(restart), independent per problem (csrc/krylov_kernels.cuh), for the
+ * system the reference solves densely (fix_point_equ, lqr_step_explicit.py:458-598).  The
+ * operator is A'v = v - M'v; the caller applies M' between the calls below, reading op_in and
+ * writing op_out (which may be the same buffer):
+ *   factored path: dilqr_adjoint_pass with w = op_in = op_out, gx = NULL, gu = zeros,
+ *                  first_pass = 0 (op_negate = 0);
+ *   generic path:  the adjoint LQR solve on cost (C, op_in) (op_negate = 1: op_in = -v),
+ *                  then dilqr_richardson_update with g = zeros and w = op_out.
+ * Sequence: start, op, then per cycle c while steps = dilqr_krylov_cycle_steps(k, c) > 0:
+ *   arnoldi(0), op, arnoldi(1), op, ..., arnoldi(steps - 1), update, op, restart, op.
+ * A problem whose relative residual |g - A'w| / |g|
+ * reaches tol is frozen (w, iters, resid stop changing); control[0] counts the problems still
+ * iterating after the latest start / restart, and every Krylov kernel exits at once when it
+ * is 0, so the host may stop after any restart that leaves it 0 or enqueue the whole budget
+ * without reading it -- both give the same bits.  g_b = 0 gives w_b = 0 exactly. */
+typedef struct DilqrKrylov {
+  int32_t n_state, n_ctrl, T, n_batch, dtype;
+  int32_t restart;       /* basis vectors per cycle, 1 <= restart <= T * (n_state + n_ctrl)  */
+  int32_t max_iter;      /* Arnoldi steps per problem over all cycles (>= 1)                 */
+  int32_t step;          /* dilqr_krylov_arnoldi: index of the step within its cycle        */
+  int32_t op_negate;     /* 1: op_in receives -v (generic adjoint solve), 0: +v             */
+  int32_t reserved0;
+  double  tol;           /* relative residual at which a problem is frozen                  */
+  const void *gx, *gu;   /* right-hand side g as [T,B,ns] (NULL: zero) and [T,B,nc]          */
+  void *w;               /* [T,B,n] solution                                               */
+  void *op_in;           /* [T,B,n] operator input, written by the Krylov calls            */
+  const void *op_out;    /* [T,B,n] M' op_in as the operator left it                        */
+  int32_t *iters;        /* [B] Arnoldi steps taken per problem                             */
+  double *resid;         /* [B] relative residual of w at the latest start / restart        */
+  uint32_t *control;     /* device, 2 words: [0] problems iterating, [1] scratch           */
+  void *workspace;       /* basis (restart + 1) x T*B*n scalars + per-problem FP64 data    */
+  size_t workspace_bytes;
+} DilqrKrylov;
+size_t dilqr_krylov_workspace_bytes(const DilqrKrylov* k);
+/* Arnoldi steps of cycle `cycle` under the budget: min(restart, max_iter - cycle * restart),
+ * 0 once the budget is spent; DILQR_EINVAL for bad sizes. */
+int dilqr_krylov_cycle_steps(const DilqrKrylov* k, int cycle);
+/* w = 0, iters = 0, v_0 = g / |g| into op_in; control[0] = problems with g != 0. */
+int dilqr_krylov_start(const DilqrKrylov* k, void* stream);
+/* Arnoldi step k->step: reads v_step and op_out = M'v_step, orthogonalises (CGS2), updates the
+ * Givens rotations and the residual estimate, writes v_{step+1} into the basis and op_in. */
+int dilqr_krylov_arnoldi(const DilqrKrylov* k, void* stream);
+/* End of a cycle, first half: w += V y from the triangle of the cycle; op_in = w. */
+int dilqr_krylov_update(const DilqrKrylov* k, void* stream);
+/* End of a cycle, second half: with op_out = M'w, the true residual r = g - A'w; freezes a
+ * problem at |r| / |g| <= tol, else restarts it from v_0 = r / |r|; updates control[0]. */
+int dilqr_krylov_restart(const DilqrKrylov* k, void* stream);
+
 /* dtheta[B,n_theta] = sum_t <dF_w, dD_t/dtheta> + <df_w, dd_t/dtheta> with the
  * closed-loop sensitivity rollout grad_input (cartpole.py:717-788, pendulum.py:
  * 383-443) contracted on the fly.  K[T,B,nc,ns]: gains of the final LQR pass in
